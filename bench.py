@@ -1,7 +1,7 @@
 """
 Benchmark of the Timbre-Trap hot path on B200 (contract: see the round prompt / DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--blocks 256]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--blocks 256] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2], the configuration the audio-s/s metric is quoted on): transcribe + reconstruct of a
@@ -239,6 +239,24 @@ def synthetic_targets(n_items, n_frames, seed):
     return torch.from_numpy(gt)
 
 
+DUMP_ELEMENTS = 12 << 20      # float32 values --dump-outputs writes in all (48 MiB), shared equally by the outputs
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes each tensor of `outputs` (name -> tensor) as out_dir/<name>.npy in float32.  One that fits its share of DUMP_ELEMENTS is
+    written whole, in its own shape; a larger one as a 1-D array of its elements at sorted flat indices drawn without replacement by a
+    generator of fixed seed from its element count alone, so two runs with the same arguments write the same positions."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_ELEMENTS // len(outputs)
+    for name, t in outputs.items():
+        t = t.detach()
+        if t.numel() > share:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), share, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, f'{name}.npy'), t.float().cpu().numpy())
+
+
 def run_ours(args, rank, world, local_rank):
     import torch.distributed as dist
     from timbre_trap_b200 import _lib
@@ -283,13 +301,17 @@ def run_ours(args, rank, world, local_rank):
     _lib.lib().tt_launch_count(1)
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     a.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - 1):
         step_resident()
+    last = step_resident()                      # held past the loop only: the earlier steps' outputs are freed as before
     b.record()
     barrier()
     launches = int(_lib.lib().tt_launch_count(1))
     ms_total = max_over_ranks(a.elapsed_time(b))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(activations=last[0], audio=last[1]))
+    del last
     ms_step = ms_total / args.steps
     value = world * n_blocks * SECS / (ms_step * 1e-3)
     # whole-step arithmetic against the SUSTAINED bf16 peak: 3 chunks per block, encoder once + decoder twice per chunk
@@ -523,7 +545,14 @@ def main():
     ap.add_argument('--no-train', action='store_true', help='skip the loss-step leg (BASELINE.json configs[3])')
     ap.add_argument('--no-hour', action='store_true', help='skip the sharded one-hour-clip leg (BASELINE.json configs[4])')
     ap.add_argument('--no-eager', action='store_true', help='skip the eager-PyTorch GPU anchor')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the activations and audio of the last device-resident step as DIR/<name>.npy '
+                         '(float32; larger outputs as a fixed, seeded sample, 48 MiB in all) on rank 0')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))
