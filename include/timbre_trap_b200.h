@@ -248,20 +248,7 @@ int tt_transcription_loss(const float* estimate, const float* target, int B, int
                           float* out, float* scratch, void* stream);
 
 /*
- * ---- backward half of the loss step (experiments/train.py:470-496), first native version -----------------------------
- * Generic direct-convolution gradient kernels on fp32 NCHW tensors (B, C, H, T) for a REGULAR convolution
- *   y[b,co,ho,t] = bias[co] + sum W[co,ci,kh,kw] x[b,ci, ho*sh + kh*dh - ph, t + kw*dw - pw]     (stride / dilation in T are 1 / dw)
- * The transposed layers use them with the roles swapped (convT forward = bwd_data, convT backward-data = fwd, convT weight
- * gradient = bwd_weight with x := dy, dz := x); hout_override gives the row count of the dz-side tensor when output_padding
- * makes it differ from the regular formula.  bwd_weight ACCUMULATES into dw / db.
- */
-int tt_conv_fwd_f32(const float* x, const float* w, const float* bias, float* y, int B, int Cin, int Hin, int T, int Cout,
-                    int KH, int KW, int sh, int dh, int dw, int ph, int pw, int act_elu, void* stream);
-int tt_conv_bwd_data_f32(const float* dz, const float* w, float* dx, int B, int Cin, int Hin, int T, int Cout,
-                         int KH, int KW, int sh, int dh, int dw, int ph, int pw, int hout_override, void* stream);
-int tt_conv_bwd_weight_f32(const float* x, const float* dz, float* dw, float* db, int B, int Cin, int Hin, int T, int Cout,
-                           int KH, int KW, int sh, int dh, int dw_, int ph, int pw, int hout_override, void* stream);
-/*
+ * ---- backward half of the loss step (experiments/train.py:470-496) ---------------------------------------------------
  * Tensor-core weight gradients of the residual blocks' 'same' convolutions, straight from the inference layouts: x, dz C8 planar bf16
  * (B, C/8, H, T, 8) with the PADDED channel counts Cin / Cout (8, 16 or 32); dw (cout_real, cin_real, k, k) fp32 and db (cout_real)
  * fp32 (db may be NULL) are ACCUMULATED into.  k = 3 (dilation 1..3, zero padding = dilation) or k = 1.  The GEMM's K axis is the
@@ -294,10 +281,6 @@ int tt_res_out_bwd_bf16(const void* gy, const void* y, const void* x, void* dz, 
 /* packed 4-channel (B, H, T, 4) <-> C8 planar with one channel group (B, 1, H, T, 8), n_pixels = B * H * T */
 int tt_p4_to_c8(const void* p4, void* c8, int64_t n_pixels, void* stream);
 int tt_c8_to_p4(const void* c8, void* p4, int64_t n_pixels, void* stream);
-/* db[c] += sum over (b, h, t) of dz (B, C, hw): the bias gradient of the transposed layers */
-int tt_channel_sum(const float* dz, float* db, int B, int C, int64_t hw, void* stream);
-/* dz = dy * ELU'(z), through the activated output a: ELU'(z) = 1 if a > 0 else a + 1 */
-int tt_elu_bwd(const float* dy, const float* a, float* dz, int64_t n, void* stream);
 /* gradients of tt_sum_sq_diff (both arguments; either output may be NULL), tt_transcription_loss (estimate), tanh|c| */
 int tt_sum_sq_diff_bwd(const float* a, const float* b, const float* gout, double scale, float* ga, float* gb, int64_t n, void* stream);
 int tt_transcription_loss_bwd(const float* estimate, const float* target, const float* gout, int B, int F, int T,

@@ -1,5 +1,4 @@
-"""Device time of the weight-gradient entry points at the loss step's shapes (batch 8 x 9 s): python scripts/time_wgrad.py
-(TT_WGRAD_LEGACY=1 selects the one-MMA-per-tap kernels)."""
+"""Device time of the weight-gradient entry points at the loss step's shapes (batch 8 x 9 s): python scripts/time_wgrad.py"""
 import os
 import sys
 

@@ -1,5 +1,5 @@
 """
-GPU parity of the backward half of the loss step (experiments/train.py:470-496): the generic gradient kernels against torch
+GPU parity of the backward half of the loss step (experiments/train.py:470-496): the weight-gradient kernels against torch
 autograd, the whole step's parameter gradients against the CPU oracle's autograd (fp32), and clip + AdamW against torch.optim.
 Tolerance on gradients: the forward runs in bf16 and activation gradients travel in bf16 between layers (the reference trains
 under fp16 autocast), so per-parameter gradients are compared at rel-L2 <= 1e-1 (the small bias vectors are the noisiest) and the global gradient at 3e-2.
@@ -16,52 +16,6 @@ from tests.helpers import tonal_clip
 pytestmark = pytest.mark.gpu
 
 SMALL = dict(sample_rate=8000, n_octaves=6, bins_per_octave=12, secs_per_block=0.5)
-
-
-@pytest.mark.parametrize('Cin,Cout,KH,KW,sh,d,ph,pw,H', [(3, 5, 3, 3, 1, 2, 2, 2, 11), (4, 8, 4, 1, 2, 1, 0, 0, 14), (6, 2, 1, 1, 1, 1, 0, 0, 5),
-                                                          (8, 16, 7, 1, 1, 1, 0, 0, 7), (2, 4, 3, 3, 1, 1, 1, 1, 9), (5, 3, 3, 3, 1, 3, 3, 3, 13)])
-def test_generic_conv_kernels_match_autograd(Cin, Cout, KH, KW, sh, d, ph, pw, H):
-    from timbre_trap_b200.framework import train as TR
-    g = torch.Generator().manual_seed(KH * 100 + Cin)
-    B, T = 2, 37
-    x = torch.randn((B, Cin, H, T), generator=g, requires_grad=True)
-    w = torch.randn((Cout, Cin, KH, KW), generator=g, requires_grad=True)
-    b = torch.randn((Cout,), generator=g, requires_grad=True)
-    y = F.elu(F.conv2d(x, w, b, stride=(sh, 1), padding=(ph, pw), dilation=(d if KH > 1 else 1, d if KW > 1 else 1)))
-    gy = torch.randn(y.shape, generator=g)
-    y.backward(gy)
-    geom = TR._geom(KH, KW, sh=sh, dh=d if KH > 1 else 1, dw=d if KW > 1 else 1, ph=ph, pw=pw)
-    xc, wc, bc = x.detach().cuda(), w.detach().cuda(), b.detach().cuda()
-    yk = TR._conv_fwd(xc, wc, bc, geom, True)
-    assert torch.allclose(yk.cpu(), y.detach(), atol=1e-4, rtol=1e-4)
-    dz = TR._elu_bwd(gy.cuda(), yk)
-    dx = TR._conv_bwd_data(dz, wc, xc.shape, geom)
-    dw, db = TR._conv_bwd_weight(xc, dz, wc.shape, geom, True)
-    assert torch.allclose(dx.cpu(), x.grad, atol=2e-4, rtol=1e-3)
-    assert torch.allclose(dw.cpu(), w.grad, atol=2e-3, rtol=1e-3)
-    assert torch.allclose(db.cpu(), b.grad, atol=2e-3, rtol=1e-3)
-
-
-@pytest.mark.parametrize('Cin,Cout,KH,sh,op,H', [(6, 4, 4, 2, 1, 9), (8, 3, 4, 2, 0, 6), (5, 7, 6, 1, 0, 1)])
-def test_transposed_roles(Cin, Cout, KH, sh, op, H):
-    """convT forward / backward through the regular-conv kernels with the roles swapped (DecoderBlock.tconv, Decoder.convin)."""
-    from timbre_trap_b200.framework import train as TR
-    g = torch.Generator().manual_seed(KH + Cin)
-    B, T = 2, 21
-    x = torch.randn((B, Cin, H, T), generator=g, requires_grad=True)
-    w = torch.randn((Cin, Cout, KH, 1), generator=g, requires_grad=True)
-    y = F.conv_transpose2d(x, w, None, stride=(sh, 1), output_padding=(op, 0))
-    gy = torch.randn(y.shape, generator=g)
-    y.backward(gy)
-    geom = TR._geom(KH, 1, sh=sh)
-    wc, gyc, xc = w.detach().cuda(), gy.cuda(), x.detach().cuda()
-    yk = TR._conv_bwd_data(xc, wc, (B, Cout, y.shape[2], T), geom)          # convT forward = bwd_data
-    assert torch.allclose(yk.cpu(), y.detach(), atol=1e-4, rtol=1e-4)
-    gx = TR._conv_fwd(gyc, wc, None, geom, False)                            # convT backward-data = regular forward
-    assert gx.shape == x.shape and torch.allclose(gx.cpu(), x.grad, atol=2e-4, rtol=1e-3)
-    dw, _ = TR._conv_bwd_weight(gyc, xc, wc.shape, geom, False)
-    assert torch.allclose(dw.cpu(), w.grad, atol=2e-3, rtol=1e-3)
-    assert torch.allclose(TR._channel_sum(gyc).cpu(), gy.sum(dim=(0, 2, 3)), atol=1e-3, rtol=1e-4)
 
 
 def _setup(skip=False, latent=None):
@@ -96,7 +50,8 @@ def _oracle_grads(R, sd, c, audio, gt):
     return {k: v.grad for k, v in sd.items()}, losses, float(total.detach())
 
 
-@pytest.mark.parametrize('skip,latent', [(False, None), (True, None), (False, 40)])     # 40 latent channels: padded to 64 in the kernels
+# 40 latent channels: padded to 64 in the kernels; 200: padded to 256, the latent weight gradients in two slices of 128 channels
+@pytest.mark.parametrize('skip,latent', [(False, None), (True, None), (False, 40), (False, 200)])
 def test_step_gradients_match_oracle_autograd(skip, latent):
     from timbre_trap_b200.framework.train import TrainStep
     R, model, sd, c, audio, gt = _setup(skip, latent)
@@ -205,7 +160,7 @@ def test_tensor_core_weight_gradient_strided_and_transposed(Cf, Cc, Hc, T, op, B
     assert float((dbt.cpu() - bt.grad).abs().max()) <= 2e-4 * float(bt.grad.abs().max()) + 2e-3
 
 
-@pytest.mark.parametrize('Ct,Cf,H,T,B', [(64, 128, 31, 256, 2), (32, 32, 5, 200, 3), (64, 100, 31, 128, 1)])
+@pytest.mark.parametrize('Ct,Cf,H,T,B', [(64, 128, 31, 256, 2), (32, 32, 5, 200, 3), (64, 100, 31, 128, 1), (64, 200, 31, 128, 1)])
 def test_tensor_core_weight_gradient_tall_kernel_layers(Ct, Cf, H, T, B):
     """tt_conv_wgrad_lat against torch autograd: Encoder.convlat (Conv2d (Cf, Ct, H, 1) over the full height) and Decoder.convin
     (ConvTranspose2d (Cf + 1, Ct, H, 1) with the indicator channel: its weight row and the bias are row sums of the output gradient)."""

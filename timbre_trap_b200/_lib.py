@@ -56,9 +56,6 @@ SIGNATURES = {
     'tt_loss_scratch_floats': (c_int, []),
     'tt_sum_sq_diff': (c_int, [c_void_p, c_void_p, c_int64, ctypes.c_double, c_void_p, c_void_p, c_void_p]),
     'tt_transcription_loss': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
-    'tt_conv_fwd_f32': (c_int, [c_void_p] * 4 + [c_int] * 13 + [c_void_p]),
-    'tt_conv_bwd_data_f32': (c_int, [c_void_p] * 3 + [c_int] * 13 + [c_void_p]),
-    'tt_conv_bwd_weight_f32': (c_int, [c_void_p] * 4 + [c_int] * 13 + [c_void_p]),
     'tt_wgrad_scratch_floats': (c_int64, [c_int, c_int, c_int]),
     'tt_conv_wgrad_same': (c_int, [c_void_p] * 4 + [c_int] * 9 + [c_void_p, c_void_p]),
     'tt_conv_wgrad_updown': (c_int, [c_void_p] * 4 + [c_int] * 9 + [c_void_p, c_void_p]),
@@ -68,8 +65,6 @@ SIGNATURES = {
     'tt_res_out_bwd_bf16': (c_int, [c_void_p] * 4 + [c_int64, c_void_p]),
     'tt_p4_to_c8': (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
     'tt_c8_to_p4': (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
-    'tt_channel_sum': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int64, c_void_p]),
-    'tt_elu_bwd': (c_int, [c_void_p] * 3 + [c_int64, c_void_p]),
     'tt_sum_sq_diff_bwd': (c_int, [c_void_p] * 3 + [ctypes.c_double] + [c_void_p] * 2 + [c_int64, c_void_p]),
     'tt_transcription_loss_bwd': (c_int, [c_void_p] * 3 + [c_int] * 4 + [c_void_p, c_void_p]),
     'tt_activations_bwd': (c_int, [c_void_p] * 3 + [c_int64, c_void_p]),

@@ -1,12 +1,7 @@
 // Backward half of the loss step (reference: experiments/train.py:470-496 = autograd through timbre_trap/framework/modules.py
-// and objectives.py, clip_grad_norm_, AdamW): direct-convolution gradient kernels on CUDA cores over fp32 NCHW tensors (B, C, H, T),
-// correct for every layer shape of the model, register-tiled where the problem is large; tensor-core versions are the next step
-// (the residual blocks already take their data gradients on the tensor cores, framework/train.py).
-//
-// All three conv kernels are written for a REGULAR convolution
-//     y[b,co,ho,t] = bias[co] + sum_{ci,kh,kw} W[co,ci,kh,kw] * x[b,ci, ho*sh + kh*dh - ph, t + kw*dw - pw]
-// and the transposed layers (DecoderBlock.tconv, Decoder.convin) use them with the roles swapped:
-//     convT forward      = bwd_data(dz := x, W)          convT backward-data = fwd(dy, W)          convT weight grad = bwd_weight(x := dy, dz := x)
+// and objectives.py, clip_grad_norm_, AdamW): the gradients of the losses with respect to their inputs, and clip + AdamW over the
+// flat parameter / gradient buckets.  The layers' weight gradients are in wgrad_tc.cu; their data gradients run through the
+// forward kernels (framework/train.py).
 #include <math.h>
 
 #include <algorithm>
@@ -15,315 +10,6 @@
 #include "tt_common.cuh"
 
 namespace tt {
-
-struct ConvGeom {
-    int B, Cin, Hin, T, Cout, Hout;
-    int KH, KW, sh, dh, dw, ph, pw;
-};
-
-__device__ __forceinline__ float elu_act(float v) { return v > 0.f ? v : expm1f(v); }
-
-// y = act(conv(x, W) + bias); one thread per output element, t fastest (coalesced)
-__global__ void __launch_bounds__(256) conv_fwd_f32_kernel(const float* __restrict__ x, const float* __restrict__ w,
-                                                           const float* __restrict__ bias, float* __restrict__ y, ConvGeom g, int act) {
-    const long long n = (long long)g.B * g.Cout * g.Hout * g.T;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const int t = (int)(i % g.T);
-        long long r = i / g.T;
-        const int ho = (int)(r % g.Hout); r /= g.Hout;
-        const int co = (int)(r % g.Cout);
-        const int b = (int)(r / g.Cout);
-        float acc = bias ? bias[co] : 0.f;
-        for (int ci = 0; ci < g.Cin; ++ci) {
-            const float* xp = x + ((size_t)b * g.Cin + ci) * g.Hin * g.T;
-            const float* wp = w + ((size_t)co * g.Cin + ci) * g.KH * g.KW;
-            for (int kh = 0; kh < g.KH; ++kh) {
-                const int hi = ho * g.sh + kh * g.dh - g.ph;
-                if (hi < 0 || hi >= g.Hin) continue;
-                for (int kw = 0; kw < g.KW; ++kw) {
-                    const int ti = t + kw * g.dw - g.pw;
-                    if (ti < 0 || ti >= g.T) continue;
-                    acc = fmaf(__ldg(wp + kh * g.KW + kw), __ldg(xp + (size_t)hi * g.T + ti), acc);
-                }
-            }
-        }
-        y[i] = act ? elu_act(acc) : acc;
-    }
-}
-
-// dx[b,ci,hi,t] = sum_{co,kh,kw} W[co,ci,kh,kw] * dz[b,co,ho,to]  with  ho*sh + kh*dh - ph = hi,  to + kw*dw - pw = t
-__global__ void __launch_bounds__(256) conv_bwd_data_f32_kernel(const float* __restrict__ dz, const float* __restrict__ w,
-                                                                float* __restrict__ dx, ConvGeom g) {
-    const long long n = (long long)g.B * g.Cin * g.Hin * g.T;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const int t = (int)(i % g.T);
-        long long r = i / g.T;
-        const int hi = (int)(r % g.Hin); r /= g.Hin;
-        const int ci = (int)(r % g.Cin);
-        const int b = (int)(r / g.Cin);
-        float acc = 0.f;
-        for (int kh = 0; kh < g.KH; ++kh) {
-            const int num = hi + g.ph - kh * g.dh;
-            if (num < 0 || num % g.sh) continue;
-            const int ho = num / g.sh;
-            if (ho >= g.Hout) continue;
-            for (int kw = 0; kw < g.KW; ++kw) {
-                const int to = t + g.pw - kw * g.dw;
-                if (to < 0 || to >= g.T) continue;
-                const float* zp = dz + ((size_t)b * g.Cout * g.Hout + ho) * g.T + to;
-                const float* wp = w + (size_t)ci * g.KH * g.KW + kh * g.KW + kw;
-                for (int co = 0; co < g.Cout; ++co)
-                    acc = fmaf(__ldg(wp + (size_t)co * g.Cin * g.KH * g.KW), __ldg(zp + (size_t)co * g.Hout * g.T), acc);
-            }
-        }
-        dx[i] = acc;
-    }
-}
-
-// Register-tiled versions of the two kernels above: a thread owns kTileC channels x kTileP consecutive frames of one row, so that
-// every loaded input / weight feeds kTileC (resp. kTileP) FMAs (2 FMAs per load instead of 0.5).
-constexpr int kTileC = 4, kTileP = 4;
-#ifndef TT_WG33_CIT
-#define TT_WG33_CIT 1   // (input, output) channel tile of the 3x3 weight-gradient kernel (measured best of (2,4) (4,4) (2,8) (4,2) (1,8))
-#define TT_WG33_COT 8
-#endif
-
-__global__ void __launch_bounds__(256) conv_fwd_f32_tiled_kernel(const float* __restrict__ x, const float* __restrict__ w,
-                                                                 const float* __restrict__ bias, float* __restrict__ y, ConvGeom g, int act) {
-    const int tq = (g.T + kTileP - 1) / kTileP, cq = (g.Cout + kTileC - 1) / kTileC;
-    const long long n = (long long)g.B * cq * g.Hout * tq;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const int t0 = (int)(i % tq) * kTileP;
-        long long r = i / tq;
-        const int ho = (int)(r % g.Hout); r /= g.Hout;
-        const int co0 = (int)(r % cq) * kTileC;
-        const int b = (int)(r / cq);
-        float acc[kTileC][kTileP];
-#pragma unroll
-        for (int o = 0; o < kTileC; ++o)
-#pragma unroll
-            for (int q = 0; q < kTileP; ++q) acc[o][q] = (bias && co0 + o < g.Cout) ? bias[co0 + o] : 0.f;
-        for (int ci = 0; ci < g.Cin; ++ci) {
-            const float* xp = x + ((size_t)b * g.Cin + ci) * g.Hin * g.T;
-            for (int kh = 0; kh < g.KH; ++kh) {
-                const int hi = ho * g.sh + kh * g.dh - g.ph;
-                if (hi < 0 || hi >= g.Hin) continue;
-                for (int kw = 0; kw < g.KW; ++kw) {
-                    const int ti = t0 + kw * g.dw - g.pw;
-                    float v[kTileP], wv[kTileC];
-#pragma unroll
-                    for (int q = 0; q < kTileP; ++q) v[q] = (ti + q >= 0 && ti + q < g.T) ? __ldg(xp + (size_t)hi * g.T + ti + q) : 0.f;
-#pragma unroll
-                    for (int o = 0; o < kTileC; ++o)
-                        wv[o] = co0 + o < g.Cout ? __ldg(w + (((size_t)(co0 + o) * g.Cin + ci) * g.KH + kh) * g.KW + kw) : 0.f;
-#pragma unroll
-                    for (int o = 0; o < kTileC; ++o)
-#pragma unroll
-                        for (int q = 0; q < kTileP; ++q) acc[o][q] = fmaf(wv[o], v[q], acc[o][q]);
-                }
-            }
-        }
-#pragma unroll
-        for (int o = 0; o < kTileC; ++o) {
-            if (co0 + o >= g.Cout) break;
-            float* yp = y + (((size_t)b * g.Cout + co0 + o) * g.Hout + ho) * g.T + t0;
-#pragma unroll
-            for (int q = 0; q < kTileP; ++q)
-                if (t0 + q < g.T) yp[q] = act ? elu_act(acc[o][q]) : acc[o][q];
-        }
-    }
-}
-
-__global__ void __launch_bounds__(256) conv_bwd_data_f32_tiled_kernel(const float* __restrict__ dz, const float* __restrict__ w,
-                                                                      float* __restrict__ dx, ConvGeom g) {
-    const int tq = (g.T + kTileP - 1) / kTileP, cq = (g.Cin + kTileC - 1) / kTileC;
-    const long long n = (long long)g.B * cq * g.Hin * tq;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const int t0 = (int)(i % tq) * kTileP;
-        long long r = i / tq;
-        const int hi = (int)(r % g.Hin); r /= g.Hin;
-        const int ci0 = (int)(r % cq) * kTileC;
-        const int b = (int)(r / cq);
-        float acc[kTileC][kTileP];
-#pragma unroll
-        for (int c = 0; c < kTileC; ++c)
-#pragma unroll
-            for (int q = 0; q < kTileP; ++q) acc[c][q] = 0.f;
-        for (int kh = 0; kh < g.KH; ++kh) {
-            const int num = hi + g.ph - kh * g.dh;
-            if (num < 0 || num % g.sh) continue;
-            const int ho = num / g.sh;
-            if (ho >= g.Hout) continue;
-            for (int kw = 0; kw < g.KW; ++kw) {
-                const int to = t0 + g.pw - kw * g.dw;
-                for (int co = 0; co < g.Cout; ++co) {
-                    const float* zp = dz + (((size_t)b * g.Cout + co) * g.Hout + ho) * g.T;
-                    float v[kTileP], wv[kTileC];
-#pragma unroll
-                    for (int q = 0; q < kTileP; ++q) v[q] = (to + q >= 0 && to + q < g.T) ? __ldg(zp + to + q) : 0.f;
-#pragma unroll
-                    for (int c = 0; c < kTileC; ++c)
-                        wv[c] = ci0 + c < g.Cin ? __ldg(w + (((size_t)co * g.Cin + ci0 + c) * g.KH + kh) * g.KW + kw) : 0.f;
-#pragma unroll
-                    for (int c = 0; c < kTileC; ++c)
-#pragma unroll
-                        for (int q = 0; q < kTileP; ++q) acc[c][q] = fmaf(wv[c], v[q], acc[c][q]);
-                }
-            }
-        }
-#pragma unroll
-        for (int c = 0; c < kTileC; ++c) {
-            if (ci0 + c >= g.Cin) break;
-            float* xp = dx + (((size_t)b * g.Cin + ci0 + c) * g.Hin + hi) * g.T + t0;
-#pragma unroll
-            for (int q = 0; q < kTileP; ++q)
-                if (t0 + q < g.T) xp[q] = acc[c][q];
-        }
-    }
-}
-
-// dW[co,ci,kh,kw] += sum_{b,ho,t} dz[b,co,ho,t] * x[b,ci,hi,ti];  db[co] += sum dz.
-// grid: (pixel chunks, Cout * Cin); each CTA owns one (co, ci) pair and all taps (KH*KW <= 32), reduces its pixel chunk and
-// adds the partial sums atomically (fp32 atomics: the summation order across chunks is not fixed).
-constexpr int kMaxTapsW = 32;
-__global__ void __launch_bounds__(256) conv_bwd_weight_f32_kernel(const float* __restrict__ x, const float* __restrict__ dz,
-                                                                  float* __restrict__ dw, float* __restrict__ db, ConvGeom g) {
-    __shared__ float red[8][kMaxTapsW + 1];
-    const int co = blockIdx.y / g.Cin, ci = blockIdx.y % g.Cin;
-    const int taps = g.KH * g.KW;
-    float acc[kMaxTapsW + 1];
-#pragma unroll
-    for (int k = 0; k <= kMaxTapsW; ++k) acc[k] = 0.f;
-    const long long n = (long long)g.B * g.Hout * g.T;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const int t = (int)(i % g.T);
-        long long r = i / g.T;
-        const int ho = (int)(r % g.Hout);
-        const int b = (int)(r / g.Hout);
-        const float z = __ldg(dz + (((size_t)b * g.Cout + co) * g.Hout + ho) * g.T + t);
-        acc[kMaxTapsW] += z;
-        const float* xp = x + ((size_t)b * g.Cin + ci) * g.Hin * g.T;
-#pragma unroll 1
-        for (int kh = 0; kh < g.KH; ++kh) {
-            const int hi = ho * g.sh + kh * g.dh - g.ph;
-            if (hi < 0 || hi >= g.Hin) continue;
-            for (int kw = 0; kw < g.KW; ++kw) {
-                const int ti = t + kw * g.dw - g.pw;
-                if (ti < 0 || ti >= g.T) continue;
-                const int k = kh * g.KW + kw;
-                const float v = z * __ldg(xp + (size_t)hi * g.T + ti);
-                // acc[] is indexed with a runtime k: keep it in registers by a predicated unrolled update
-#pragma unroll
-                for (int q = 0; q < kMaxTapsW; ++q) acc[q] += (q == k) ? v : 0.f;
-            }
-        }
-    }
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-    for (int k = 0; k <= kMaxTapsW; ++k) {
-        float v = acc[k];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        if (lane == 0) red[warp][k] = v;
-    }
-    __syncthreads();
-    if (threadIdx.x <= kMaxTapsW) {
-        const int k = threadIdx.x;
-        float v = 0.f;
-        for (int wv = 0; wv < 8; ++wv) v += red[wv][k];
-        if (k < taps) atomicAdd(dw + ((size_t)co * g.Cin + ci) * taps + k, v);
-        else if (k == kMaxTapsW && db && ci == 0) atomicAdd(db + co, v);
-    }
-}
-
-// Same reduction, specialised: the tap loops are compile-time (accumulators stay in registers without predicated updates) and one
-// CTA covers a COT x CIT tile of (output, input) channels: per pixel COT gradient values and CIT * KH * KW inputs are loaded for
-// COT * CIT * KH * KW products (3.3 FMAs per load for the 3x3 case; the one-output-channel version did 1 and was bound by its loads).
-template <int KH, int KW, int CIT, int COT>
-__global__ void __launch_bounds__(256) conv_bwd_weight_tiled_kernel(const float* __restrict__ x, const float* __restrict__ dz,
-                                                                    float* __restrict__ dw, float* __restrict__ db, ConvGeom g) {
-    constexpr int TAPS = KH * KW;
-    constexpr int NACC = COT * CIT * TAPS;
-    __shared__ float red[8][NACC + COT];
-    const int n_cib = (g.Cin + CIT - 1) / CIT;
-    const int co0 = (blockIdx.y / n_cib) * COT, ci0 = (blockIdx.y % n_cib) * CIT;
-    float acc[COT][CIT][TAPS];
-    float accb[COT];
-#pragma unroll
-    for (int o = 0; o < COT; ++o) {
-        accb[o] = 0.f;
-#pragma unroll
-        for (int c = 0; c < CIT; ++c)
-#pragma unroll
-            for (int k = 0; k < TAPS; ++k) acc[o][c][k] = 0.f;
-    }
-    const long long n = (long long)g.B * g.Hout * g.T;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const int t = (int)(i % g.T);
-        long long r = i / g.T;
-        const int ho = (int)(r % g.Hout);
-        const int b = (int)(r / g.Hout);
-        float z[COT];
-#pragma unroll
-        for (int o = 0; o < COT; ++o) {
-            z[o] = co0 + o < g.Cout ? __ldg(dz + (((size_t)b * g.Cout + co0 + o) * g.Hout + ho) * g.T + t) : 0.f;
-            accb[o] += z[o];
-        }
-#pragma unroll
-        for (int c = 0; c < CIT; ++c) {
-            if (ci0 + c >= g.Cin) break;
-            const float* xp = x + ((size_t)b * g.Cin + ci0 + c) * g.Hin * g.T;
-#pragma unroll
-            for (int kh = 0; kh < KH; ++kh) {
-                const int hi = ho * g.sh + kh * g.dh - g.ph;
-                const bool h_ok = hi >= 0 && hi < g.Hin;
-#pragma unroll
-                for (int kw = 0; kw < KW; ++kw) {
-                    const int ti = t + kw * g.dw - g.pw;
-                    const float v = (h_ok && ti >= 0 && ti < g.T) ? __ldg(xp + (size_t)hi * g.T + ti) : 0.f;
-#pragma unroll
-                    for (int o = 0; o < COT; ++o) acc[o][c][kh * KW + kw] = fmaf(z[o], v, acc[o][c][kh * KW + kw]);
-                }
-            }
-        }
-    }
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-    for (int o = 0; o < COT; ++o) {
-#pragma unroll
-        for (int c = 0; c < CIT; ++c)
-#pragma unroll
-            for (int k = 0; k < TAPS; ++k) {
-                float v = acc[o][c][k];
-#pragma unroll
-                for (int s = 16; s > 0; s >>= 1) v += __shfl_xor_sync(0xffffffffu, v, s);
-                if (lane == 0) red[warp][(o * CIT + c) * TAPS + k] = v;
-            }
-        float vb = accb[o];
-#pragma unroll
-        for (int s = 16; s > 0; s >>= 1) vb += __shfl_xor_sync(0xffffffffu, vb, s);
-        if (lane == 0) red[warp][NACC + o] = vb;
-    }
-    __syncthreads();
-    for (int k = threadIdx.x; k < NACC + COT; k += 256) {
-        float v = 0.f;
-        for (int wv = 0; wv < 8; ++wv) v += red[wv][k];
-        if (k < NACC) {
-            const int o = k / (CIT * TAPS), c = (k / TAPS) % CIT, tap = k % TAPS;
-            if (co0 + o < g.Cout && ci0 + c < g.Cin) atomicAdd(dw + ((size_t)(co0 + o) * g.Cin + ci0 + c) * TAPS + tap, v);
-        } else if (db && ci0 == 0 && co0 + (k - NACC) < g.Cout) {
-            atomicAdd(db + co0 + (k - NACC), v);
-        }
-    }
-}
-
-// dz = dy * ELU'(z) expressed through the activated output a = ELU(z):  ELU'(z) = 1 (a > 0) or a + 1
-__global__ void elu_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ a, float* __restrict__ dz, long long n) {
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const float av = a[i];
-        dz[i] = dy[i] * (av > 0.f ? 1.f : av + 1.f);
-    }
-}
 
 // objectives.py:11-33 backward: loss = scale * sum (a-b)^2 ;  ga = gout * 2 scale (a-b),  gb = -ga  (either may be null)
 __global__ void sq_diff_bwd_kernel(const float* __restrict__ a, const float* __restrict__ b, const float* __restrict__ gout, float scale,
@@ -371,26 +57,6 @@ __global__ void activations_bwd_kernel(const float2* __restrict__ c, const float
     }
 }
 
-// db[c] += sum_{b,h,t} dz[b,c,h,t]   (bias gradient of the transposed layers); grid.y = channel
-__global__ void channel_sum_kernel(const float* __restrict__ dz, float* __restrict__ db, int B, int C, long long hw) {
-    __shared__ float red[8];
-    const int c = blockIdx.y;
-    float s = 0.f;
-    const long long n = (long long)B * hw;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const long long b = i / hw, r = i - b * hw;
-        s += dz[((size_t)b * C + c) * hw + r];
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        for (int i = 1; i < 8; ++i) s += red[i];
-        atomicAdd(db + c, s);
-    }
-}
-
 // sum of squares of one gradient tensor into a double accumulator (for clip_grad_norm_, train.py:493)
 __global__ void sumsq_kernel(const float* __restrict__ g, long long n, double* __restrict__ acc) {
     __shared__ double red[8];
@@ -432,82 +98,6 @@ static inline int grid_for(long long n) { return (int)std::max<long long>(1, std
 
 using namespace tt;
 
-static int fill_geom(ConvGeom* g, int B, int Cin, int Hin, int T, int Cout, int KH, int KW, int sh, int dh, int dw, int ph, int pw) {
-    g->B = B; g->Cin = Cin; g->Hin = Hin; g->T = T; g->Cout = Cout;
-    g->KH = KH; g->KW = KW; g->sh = sh; g->dh = dh; g->dw = dw; g->ph = ph; g->pw = pw;
-    g->Hout = (Hin + 2 * ph - dh * (KH - 1) - 1) / sh + 1;
-    TT_REQUIRE(g->Hout >= 1 && KH * KW <= kMaxTapsW && sh >= 1, "unsupported conv geometry");
-    return TT_OK;
-}
-
-extern "C" int tt_conv_fwd_f32(const float* x, const float* w, const float* bias, float* y, int B, int Cin, int Hin, int T, int Cout,
-                               int KH, int KW, int sh, int dh, int dw, int ph, int pw, int act_elu, void* stream) {
-    TT_REQUIRE(x && w && y, "null argument");
-    ConvGeom g;
-    if (int rc = fill_geom(&g, B, Cin, Hin, T, Cout, KH, KW, sh, dh, dw, ph, pw)) return rc;
-    const long long n = (long long)B * Cout * g.Hout * T;
-    if (n == 0) return TT_OK;
-    const long long n_tiles = (long long)B * ((Cout + kTileC - 1) / kTileC) * g.Hout * ((T + kTileP - 1) / kTileP);
-    // the tiled kernel wants enough threads to fill the GPU; tiny problems keep one thread per output
-    if (n_tiles >= 148 * 512) conv_fwd_f32_tiled_kernel<<<grid_for(n_tiles), 256, 0, (cudaStream_t)stream>>>(x, w, bias, y, g, act_elu);
-    else conv_fwd_f32_kernel<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>(x, w, bias, y, g, act_elu);
-    TT_CUDA_CHECK(cudaGetLastError());
-    tt_count_launches(1);
-    return TT_OK;
-}
-
-// hout_override > 0: the dz tensor has that many rows (transposed convs with output_padding produce an input-side height that
-// the regular formula cannot infer)
-extern "C" int tt_conv_bwd_data_f32(const float* dz, const float* w, float* dx, int B, int Cin, int Hin, int T, int Cout,
-                                    int KH, int KW, int sh, int dh, int dw, int ph, int pw, int hout_override, void* stream) {
-    TT_REQUIRE(dz && w && dx, "null argument");
-    ConvGeom g;
-    if (int rc = fill_geom(&g, B, Cin, Hin, T, Cout, KH, KW, sh, dh, dw, ph, pw)) return rc;
-    if (hout_override > 0) g.Hout = hout_override;
-    const long long n = (long long)B * Cin * Hin * T;
-    if (n == 0) return TT_OK;
-    const long long n_tiles = (long long)B * ((Cin + kTileC - 1) / kTileC) * Hin * ((T + kTileP - 1) / kTileP);
-    if (n_tiles >= 148 * 512) conv_bwd_data_f32_tiled_kernel<<<grid_for(n_tiles), 256, 0, (cudaStream_t)stream>>>(dz, w, dx, g);
-    else conv_bwd_data_f32_kernel<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>(dz, w, dx, g);
-    TT_CUDA_CHECK(cudaGetLastError());
-    tt_count_launches(1);
-    return TT_OK;
-}
-
-// dw (Cout, Cin, KH, KW) and db (Cout, may be NULL) are ACCUMULATED into (zero them first for a fresh gradient)
-extern "C" int tt_conv_bwd_weight_f32(const float* x, const float* dz, float* dw, float* db, int B, int Cin, int Hin, int T, int Cout,
-                                      int KH, int KW, int sh, int dh, int dw_, int ph, int pw, int hout_override, void* stream) {
-    TT_REQUIRE(x && dz && dw, "null argument");
-    ConvGeom g;
-    if (int rc = fill_geom(&g, B, Cin, Hin, T, Cout, KH, KW, sh, dh, dw_, ph, pw)) return rc;
-    if (hout_override > 0) g.Hout = hout_override;
-    const long long n = (long long)B * g.Hout * T;
-    if (n == 0) return TT_OK;
-    const unsigned gx = (unsigned)std::max<long long>(1, std::min<long long>((n + 256 * 16 - 1) / (256 * 16), 256));
-    cudaStream_t s = (cudaStream_t)stream;
-#define TT_WGRAD(KH_, KW_, CIT_, COT_)                                                                                          \
-    conv_bwd_weight_tiled_kernel<KH_, KW_, CIT_, COT_>                                                                          \
-        <<<dim3(gx, (unsigned)(((Cout + COT_ - 1) / COT_) * ((Cin + CIT_ - 1) / CIT_))), 256, 0, s>>>(x, dz, dw, db, g)
-    if (KH == 3 && KW == 3) TT_WGRAD(3, 3, TT_WG33_CIT, TT_WG33_COT);
-    else if (KH == 1 && KW == 1) TT_WGRAD(1, 1, 8, 4);
-    else if (KH == 4 && KW == 1) TT_WGRAD(4, 1, 4, 4);
-    else if (KH == 31 && KW == 1) TT_WGRAD(31, 1, 1, 2);
-    else conv_bwd_weight_f32_kernel<<<dim3(gx, (unsigned)(Cout * Cin)), 256, 0, s>>>(x, dz, dw, db, g);
-#undef TT_WGRAD
-    TT_CUDA_CHECK(cudaGetLastError());
-    tt_count_launches(1);
-    return TT_OK;
-}
-
-extern "C" int tt_elu_bwd(const float* dy, const float* a, float* dz, int64_t n, void* stream) {
-    TT_REQUIRE(dy && a && dz, "null argument");
-    if (n <= 0) return TT_OK;
-    elu_bwd_kernel<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>(dy, a, dz, n);
-    TT_CUDA_CHECK(cudaGetLastError());
-    tt_count_launches(1);
-    return TT_OK;
-}
-
 extern "C" int tt_sum_sq_diff_bwd(const float* a, const float* b, const float* gout, double scale, float* ga, float* gb, int64_t n,
                                   void* stream) {
     TT_REQUIRE(a && b && gout && (ga || gb), "null argument");
@@ -533,16 +123,6 @@ extern "C" int tt_activations_bwd(const float* coeffs, const float* dact, float*
     TT_REQUIRE(coeffs && dact && dcoeffs, "null argument");
     if (n <= 0) return TT_OK;
     activations_bwd_kernel<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>((const float2*)coeffs, dact, (float2*)dcoeffs, n);
-    TT_CUDA_CHECK(cudaGetLastError());
-    tt_count_launches(1);
-    return TT_OK;
-}
-
-extern "C" int tt_channel_sum(const float* dz, float* db, int B, int C, int64_t hw, void* stream) {
-    TT_REQUIRE(dz && db, "null argument");
-    if (B <= 0 || C <= 0 || hw <= 0) return TT_OK;
-    dim3 grid((unsigned)std::max<long long>(1, std::min<long long>(((long long)B * hw + 256 * 16 - 1) / (256 * 16), 128)), (unsigned)C);
-    channel_sum_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(dz, db, B, C, hw);
     TT_CUDA_CHECK(cudaGetLastError());
     tt_count_launches(1);
     return TT_OK;

@@ -10,12 +10,11 @@
 // So both operands are the rows the TMA brings in, untouched:
 //     A = dZ row   (M = co, 128 lanes of which the first 8 CGo are real)             K = 16 pixels per tcgen05.mma
 //     B = X row of the tap, started (kx-1) d pixels further along K (an address offset), N = ci
-// and every tap owns NPAD fp32 accumulator columns in TMEM for the whole life of the CTA; a tenth "tap" multiplies dZ with a constant
-// ones operand and yields db.  A CTA walks a strip of image rows of one 128-pixel column tile (X rows live in a ring, every row is
-// fetched once per strip, out-of-image rows arrive as zeros from the TMA), then writes its accumulators to a partial buffer; a
-// second kernel sums the partials in a fixed order (deterministic) into the PyTorch weight layout (co, ci, kh, kw).
-#include <stdlib.h>
-
+// A CTA walks a strip of image rows of one 128-pixel column tile (out-of-image rows arrive as zeros from the TMA), accumulates in TMEM
+// for the whole life of the CTA, then writes its accumulators to a partial buffer; a second kernel sums the partials in a fixed order
+// (deterministic) into the PyTorch weight layout (co, ci, kh, kw).  The 3x3 and (4,1) stride-(2,1) layers have row-stationary kernels
+// (wgrad3_kernel, wgrad_ud_kernel); the 1x1 and (H, 1) layers a ring kernel (wgrad_kernel) in which every tap owns NPAD accumulator
+// columns and one more "tap" multiplies dZ with a constant ones operand to yield db (the 1x1 layers sum db in otherwise idle warps).
 #include <algorithm>
 
 #include "../../include/timbre_trap_b200.h"
@@ -25,7 +24,7 @@ namespace tt {
 
 constexpr int kWgThreads = 128;        // warp 0: TMA producer, warp 1: MMA issuer; after the row loop warps 0-1 drain the accumulators
 constexpr int kWgZSlots = 8;           // A-side row ring (upper bound; the launch picks the depth that fits)
-constexpr int kWgMaxTaps = 10;         // 9 conv taps + the bias "tap"
+constexpr int kWgMaxTaps = 10;         // taps + the bias "tap" a partial block of wgrad_kernel has room for (the (H, 1) layers use 7 + 1)
 constexpr int kWgMaxM = 64;            // A-side channels a CTA of the row-walking geometries writes out (TMEM lanes 0..63)
 
 struct WgradParams {
@@ -33,7 +32,6 @@ struct WgradParams {
     int B, T;
     int Hz, Hx;                        // rows of the A-side (dZ) and B-side (X) tensors
     int CGi, CGo;                      // channel groups of the B side (X) and the A side (dZ)
-    int d;                             // dilation of the 3x3 geometry
     int rows_per_strip;
     int z_slots;                       // A-side ring depth (<= kWgZSlots)
     int xring;                         // B-side ring depth (<= 16): the rows one A-side row reaches + the prefetch distance
@@ -41,34 +39,25 @@ struct WgradParams {
                                        // group of `tap_group` consecutive B-side rows = vertical taps (the (31,1) layers)
 };
 
-// Geometry (compile time): KH x KW taps; the B-side row of tap ky for A-side row q is  q * RS + ky * DH + row0  with
-//   3x3 'same' (KH = KW = 3, RS = 1):  DH = d, row0 = -d, horizontal tap offsets (kx - 1) d, column halo d
-//   1x1        (KH = KW = 1, RS = 1):  row0 = 0
-//   (4,1) stride (2,1) (KH = 4, KW = 1, RS = 2):  DH = 1, row0 = 0  (EncoderBlock.sconv; DecoderBlock.tconv with the two sides swapped)
+// Geometry (compile time): KH vertical taps of width 1; the B-side row of tap ky for A-side row q is  q + ky  (relative to the first
+// B-side row of the CTA)
+//   1x1 (KH = 1): A-side row q meets B-side row q
+//   (H, 1) layers (KH = kLatTapGroup, tap_group > 0): the A side has one row, blockIdx.y selects the group of KH B-side rows
 // shared memory plan (bytes): [barriers 1 KB][ones 4 KB][A ring][B ring]; the A operand reads 16 channel groups = 32 KB from its slot, the
 // B operand NPAD/8 groups: both stay inside the allocation because the B ring follows and the allocation is padded (see wgrad_smem)
-// KXN (3x3 with ONE B-side channel group, i.e. C <= 8 - the two largest stages): the three horizontal taps are the N-GROUPS of one
-// MMA - the B descriptor's group stride is the tap step d * 16 bytes instead of the plane stride - so a K step costs 3 + 1 MMAs
-// instead of 9 + 1; accumulator columns of vertical tap ky: [kx][8 channels] (+ one unused group), NPAD = 32.
-template <int NPAD, int KH, int KW, int RS, int MW, bool KXN = false>
+template <int NPAD, int KH, int MW>
 __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_z,
                                                               const WgradParams p) {
-    static_assert(!KXN || (KH == 3 && KW == 3 && NPAD == 32), "KXN is the 3x3 single-group form");
     // 1x1 layers: the "ones" MMA would be every second MMA; instead warps 2-3 (idle otherwise) sum the A-side rows from shared memory
-    constexpr bool BIASW = KH == 1 && KW == 1 && RS == 1;
-    constexpr int TAPS = KXN ? KH : KH * KW;
-    constexpr uint32_t need = (TAPS + 1) * NPAD;
+    constexpr bool BIASW = KH == 1;
+    constexpr uint32_t need = (KH + 1) * NPAD;
     constexpr uint32_t ncols = need <= 32 ? 32 : (need <= 64 ? 64 : (need <= 128 ? 128 : (need <= 256 ? 256 : 512)));
     static_assert(need <= 512, "TMEM columns");
     extern __shared__ __align__(1024) uint8_t smem[];
-    const int d = KW == 3 ? p.d : 0;                  // column halo / horizontal tap step
-    const int DH = KH == 3 ? p.d : 1;                 // vertical tap step in B-side rows
-    const int span = (KH - 1) * DH;                   // B-side rows an A-side row reaches beyond its first one
-    const int TW = kStripTileT + 2 * d;
     const int xring = p.xring;
     const uint32_t z_slot = (uint32_t)p.CGo * kStripTileT * 16u;
-    const uint32_t x_plane = (uint32_t)TW * 16u;
-    const uint32_t x_slot = ((uint32_t)p.CGi * x_plane + 127u) & ~127u;
+    const uint32_t x_plane = (uint32_t)kStripTileT * 16u;
+    const uint32_t x_slot = (uint32_t)p.CGi * x_plane;
     uint64_t* z_full = reinterpret_cast<uint64_t*>(smem);            // [kWgZSlots]
     uint64_t* z_empty = z_full + kWgZSlots;                           // [kWgZSlots]
     uint64_t* x_full = z_empty + kWgZSlots;                           // [xring <= 16]
@@ -86,8 +75,8 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
     const int h1 = p.tap_group ? p.Hz : min(p.Hz, h0 + p.rows_per_strip);
     const int b = blockIdx.z;
     const int n_rows = h1 - h0;                         // A-side rows of this strip
-    const int n_xrows = (n_rows - 1) * RS + span + 1;   // B-side rows, relative index 0 <-> image row x_row0
-    const int x_row0 = p.tap_group ? blockIdx.y * p.tap_group : h0 * RS - (KH == 3 ? d : 0);
+    const int n_xrows = n_rows + KH - 1;                // B-side rows, relative index 0 <-> image row x_row0
+    const int x_row0 = p.tap_group ? blockIdx.y * p.tap_group : h0;
 
     if (warp == 0) umma::tmem_alloc(tmem_slot, ncols);
     if (tid == 32) {
@@ -110,13 +99,13 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
             const int slot = xr % xring;
             if (xr >= xring) umma::mbar_wait(&x_empty[slot], (uint32_t)((xr / xring - 1) & 1));
             mbar_expect_tx(&x_full[slot], (uint32_t)p.CGi * x_plane);
-            tma_load_5d(sX + (size_t)slot * x_slot, &tmap_x, &x_full[slot], 0, t0 - d, x_row0 + xr, 0, b);
+            tma_load_5d(sX + (size_t)slot * x_slot, &tmap_x, &x_full[slot], 0, t0, x_row0 + xr, 0, b);
             ++xr;
         };
         for (int r = 0; r < n_rows; ++r) {
             // as far ahead as the ring allows without waiting for a release that needs THIS iteration's A-side row (deadlock): the
-            // slot of row xr is freed by A-side row (xr - xring) / RS, which must lie before r
-            while (xr < n_xrows && xr <= r * RS + xring - RS - 1) load_x();
+            // slot of row xr is freed by A-side row xr - xring, which must lie before r
+            while (xr < n_xrows && xr <= r + xring - 2) load_x();
             const int slot = r % zslots;
             if (r >= zslots) umma::mbar_wait(&z_empty[slot], (uint32_t)((r / zslots - 1) & 1));
             mbar_expect_tx(&z_full[slot], z_slot);
@@ -130,8 +119,8 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
         for (int r = 0; r < n_rows; ++r) {
             const int zs = r % zslots;
             umma::mbar_wait(&z_full[zs], (uint32_t)((r / zslots) & 1));
-            // B-side rows r RS .. r RS + span; those beyond what row r - 1 already waited for may still be in flight
-            for (int xr = (r == 0 ? 0 : (r - 1) * RS + span + 1); xr <= r * RS + span; ++xr)
+            // B-side rows r .. r + KH - 1; those beyond what row r - 1 already waited for may still be in flight
+            for (int xr = (r == 0 ? 0 : r + KH - 1); xr <= r + KH - 1; ++xr)
                 umma::mbar_wait(&x_full[xr % xring], (uint32_t)((xr / xring) & 1));
             umma::fence_after_sync();
             const uint32_t za = z0 + (uint32_t)zs * z_slot;
@@ -140,33 +129,24 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
             // below is 32-bit adds in the one issuing thread (its instruction stream, not the tensor pipe, bounds this kernel).
             constexpr uint32_t lbo_field = (128u >> 4) << 16;
             const uint32_t hi_a = ((uint32_t)(kStripTileT * 16) >> 4) | (1u << 14);
-            const uint32_t hi_b = ((KXN ? (uint32_t)d * 16u : x_plane) >> 4) | (1u << 14);
+            const uint32_t hi_b = (x_plane >> 4) | (1u << 14);
             const uint32_t lo_a = ((za >> 4) & 0x3FFFu) | lbo_field, lo_ones = ((ones0 >> 4) & 0x3FFFu) | lbo_field;
             uint32_t lo_b[KH];
 #pragma unroll
-            for (int ky = 0; ky < KH; ++ky) lo_b[ky] = (((x0 + (uint32_t)((r * RS + ky * DH) % xring) * x_slot) >> 4) & 0x3FFFu) | lbo_field;
+            for (int ky = 0; ky < KH; ++ky) lo_b[ky] = (((x0 + (uint32_t)((r + ky) % xring) * x_slot) >> 4) & 0x3FFFu) | lbo_field;
             auto d64 = [](uint32_t hi, uint32_t lo) { return ((uint64_t)hi << 32) | lo; };
 #pragma unroll
             for (int s = 0; s < kStripTileT / 16; ++s) {
                 const bool acc = !(first && s == 0);
                 const uint64_t da = d64(hi_a, lo_a + (uint32_t)s * 16u);
 #pragma unroll
-                for (int ky = 0; ky < KH; ++ky) {
-                    if constexpr (KXN) {
-                        umma::mma_bf16(tmem + (uint32_t)(ky * NPAD), da, d64(hi_b, lo_b[ky] + (uint32_t)s * 16u), idesc, acc);
-                    } else {
-#pragma unroll
-                        for (int kx = 0; kx < KW; ++kx)
-                            umma::mma_bf16(tmem + (uint32_t)((ky * KW + kx) * NPAD), da, d64(hi_b, lo_b[ky] + (uint32_t)(kx * d) + (uint32_t)s * 16u), idesc, acc);
-                    }
-                }
-                if constexpr (!BIASW) umma::mma_bf16(tmem + (uint32_t)(TAPS * NPAD), da, d64(hi_a, lo_ones + (uint32_t)s * 16u), idesc, acc);
+                for (int ky = 0; ky < KH; ++ky)
+                    umma::mma_bf16(tmem + (uint32_t)(ky * NPAD), da, d64(hi_b, lo_b[ky] + (uint32_t)s * 16u), idesc, acc);
+                if constexpr (!BIASW) umma::mma_bf16(tmem + (uint32_t)(KH * NPAD), da, d64(hi_a, lo_ones + (uint32_t)s * 16u), idesc, acc);
             }
             first = false;
             umma::commit(&z_empty[zs]);
-            // the first RS B-side rows of this A-side row are not needed by later rows
-#pragma unroll
-            for (int k = 0; k < RS; ++k) umma::commit(&x_empty[(r * RS + k) % xring]);
+            umma::commit(&x_empty[r % xring]);                         // the first B-side row of this A-side row: not needed by later rows
         }
         umma::commit(done);
     } else if (BIASW && warp >= 2) {
@@ -217,13 +197,13 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
         float* dst = p.partial + (cta * kWgMaxTaps * MROWS + warp * 32 + lane) * NPAD;
         const uint32_t lane_addr = tmem + ((uint32_t)(warp * 32) << 16);
         if constexpr (BIASW) {
-            // the reduction reads the bias of channel o at [TAPS][o][0]
+            // the reduction reads the bias of channel o at [KH][o][0]
             const float* sB = reinterpret_cast<const float*>(smem + 640);
             const int o = warp * 32 + lane;
-            if (o < 32) dst[(size_t)TAPS * MROWS * NPAD] = sB[o] + sB[32 + o];       // dst already points at this thread's channel row
+            if (o < 32) dst[(size_t)KH * MROWS * NPAD] = sB[o] + sB[32 + o];       // dst already points at this thread's channel row
         }
 #pragma unroll 1
-        for (int tap = 0; tap < TAPS + (BIASW ? 0 : 1); ++tap) {
+        for (int tap = 0; tap < KH + (BIASW ? 0 : 1); ++tap) {
 #pragma unroll
             for (int c0 = 0; c0 < NPAD; c0 += 16) {
                 float v[16];
@@ -243,8 +223,8 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
 }
 
 // ------------------------------------------------------------------------------------------------------------------------------------
-// 3x3 'same' layers, row-stationary form.  The kernel above issues one MMA per tap and K step (9 + 1 for the bias), and its single
-// issuing thread - ~45 cycles per tcgen05.mma whatever its size - is what bounds it.  Here a B-side (X) row rho meets ALL THREE
+// 3x3 'same' layers, row-stationary form.  One MMA per tap and K step (9 + 1 for the bias) would leave the kernel bound by its single
+// issuing thread - ~45 cycles per tcgen05.mma whatever its size.  Here a B-side (X) row rho meets ALL THREE
 // vertical taps at once: the A operand spans the dZ rows rho - d, rho, rho + d, which lie next to each other in shared memory (a
 // strip's dZ rows are all resident, stored residue class by residue class mod d), i.e. the TMEM lanes are (j, co) with j = 0, 1, 2
 // <-> ky = 2, 1, 0; the horizontal taps are the N groups of the same MMA (one B-side channel group: column kx * 8 + ci) or three
@@ -469,7 +449,7 @@ __global__ void __launch_bounds__(32 * kWg3RedSeg) wgrad3_reduce_kernel(const fl
 //     dW[cc][cf][kh] = sum over (b, q, t) of  coarse[b, cc, q, t] * fine[b, cf, 2 q + kh, t]
 // A fine row rho meets the coarse rows q0 - 1 and q0 = rho / 2 (taps kh = rho % 2 + 2 and rho % 2): the strip's coarse rows are
 // resident and consecutive, so the two are stacked in the MMA's M (TMEM lanes (j, cc), j = 0 <-> q0 - 1), and the row parity selects
-// the accumulator columns: ONE MMA per fine row and K step - two per coarse row where the kernel above needs 4 + 1.  The bias
+// the accumulator columns: ONE MMA per fine row and K step - two per coarse row instead of 4 + 1 with one MMA per tap.  The bias
 // gradient of the strided layer (pixel sums of the coarse tensor) comes from the resident rows through the idle warps.
 // ------------------------------------------------------------------------------------------------------------------------------------
 struct WgradUdParams {
@@ -653,12 +633,10 @@ __global__ void __launch_bounds__(32 * kWg3RedSeg) wgrad_ud_reduce_kernel(const 
     }
 }
 
-// dW (m, n, taps) and db (m) += fixed-order sums of the per-CTA partials (m = A-side channel, n = B-side channel: (co, ci, kh, kw) for a
-// regular conv, (ci, co, kh, kw) - the ConvTranspose2d weight layout - when the two sides are swapped)
-// kxn: the partials hold 3 vertical taps of [kx][8 channels] columns (see KXN above); taps stays 9 for the output layout.
+// dW (m, n, taps) and db (m) += fixed-order sums of the per-CTA partials (m = A-side channel = co, n = B-side channel = ci)
 // One WARP per output element: the lanes stride over the CTAs' partials, then a shuffle tree - a fixed order, so still bit-reproducible.
 __global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float* __restrict__ partial, int n_ctas, int npad, int taps, int m_real, int n_real,
-                                                           float* __restrict__ dw, float* __restrict__ db, int kxn) {
+                                                           float* __restrict__ dw, float* __restrict__ db) {
     const int i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);     // over (tap' in [0, taps], m, n)
     const int lane = threadIdx.x & 31;
     const int total = (taps + 1) * m_real * n_real;
@@ -666,9 +644,7 @@ __global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float* __restri
     const int tap = i / (m_real * n_real), rem = i - tap * m_real * n_real;
     const int o = rem / n_real, c = rem - o * n_real;
     if (tap == taps && (c != 0 || db == nullptr)) return;
-    const int ptap = kxn ? (tap == taps ? 3 : tap / 3) : tap;         // accumulator block inside a CTA's partial
-    const int pcol = tap == taps ? 0 : (kxn ? (tap % 3) * 8 + c : c);
-    const float* src = partial + ((size_t)ptap * kWgMaxM + o) * npad + pcol;
+    const float* src = partial + ((size_t)tap * kWgMaxM + o) * npad + (tap == taps ? 0 : c);
     const size_t stride = (size_t)kWgMaxTaps * kWgMaxM * npad;
     float acc = 0.f;
     for (int k = lane; k < n_ctas; k += 32) acc += src[(size_t)k * stride];
@@ -838,34 +814,32 @@ __global__ void c8_to_p4_kernel(const uint4* __restrict__ c8, uint2* __restrict_
     }
 }
 
-static size_t wgrad_smem(int CGi, int CGo, int halo, int xring, int zslots) {
-    const size_t TW = kStripTileT + 2 * halo;
+static size_t wgrad_smem(int CGi, int CGo, int xring, int zslots) {
     const size_t z_slot = (size_t)CGo * kStripTileT * 16;
-    const size_t x_slot = ((size_t)CGi * TW * 16 + 127) & ~(size_t)127;
-    size_t s = 1024 + 4096 + zslots * z_slot + xring * x_slot + 8 * TW * 16;   // + the padded N groups read past the last B slot
+    const size_t x_slot = (size_t)CGi * kStripTileT * 16;
+    size_t s = 1024 + 4096 + zslots * z_slot + xring * x_slot + 8 * kStripTileT * 16;   // + the padded N groups read past the last B slot
     // the A operand spans 16 channel groups (32 KB) from the start of an A slot, the ones operand NPAD/8 groups: keep both inside
     s = std::max(s, (size_t)1024 + 4096 + (zslots - 1) * z_slot + 16 * (size_t)kStripTileT * 16 + 1024);
     return s;
 }
 
-template <int NPAD, int KH, int KW, int RS, int MW, bool KXN = false>
+template <int NPAD, int KH, int MW>
 static int launch_wgrad(const void* x, const void* dz, const WgradParams& p, dim3 grid, cudaStream_t stream) {
-    const int halo = KW == 3 ? p.d : 0;
     const int xring = p.xring;
-    TT_REQUIRE(xring <= 16 && xring >= (KH - 1) * (KH == 3 ? p.d : 1) + 1 + 2 * RS, "wgrad: ring of %d rows", xring);
-    const size_t smem = wgrad_smem(p.CGi, p.CGo, halo, xring, p.z_slots);
+    TT_REQUIRE(xring <= 16 && xring >= KH + 2, "wgrad: ring of %d rows", xring);
+    const size_t smem = wgrad_smem(p.CGi, p.CGo, xring, p.z_slots);
     TT_REQUIRE(smem <= 227 * 1024, "wgrad: %zu bytes of shared memory", smem);
     static size_t configured = 0;
     if (smem > configured) {
-        TT_CUDA_CHECK(cudaFuncSetAttribute(wgrad_kernel<NPAD, KH, KW, RS, MW, KXN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        TT_CUDA_CHECK(cudaFuncSetAttribute(wgrad_kernel<NPAD, KH, MW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured = smem;
     }
     CUtensorMap mx, mz;
-    int rc = make_row_map(&mx, x, p.B, p.CGi, p.Hx, p.T, kStripTileT + 2 * halo);
+    int rc = make_row_map(&mx, x, p.B, p.CGi, p.Hx, p.T, kStripTileT);
     if (rc) return rc;
     rc = make_row_map(&mz, dz, p.B, p.CGo, p.Hz, p.T, kStripTileT);
     if (rc) return rc;
-    wgrad_kernel<NPAD, KH, KW, RS, MW, KXN><<<grid, kWgThreads, smem, stream>>>(mx, mz, p);
+    wgrad_kernel<NPAD, KH, MW><<<grid, kWgThreads, smem, stream>>>(mx, mz, p);
     TT_CUDA_CHECK(cudaGetLastError());
     tt_count_launches(1);
     return TT_OK;
@@ -891,9 +865,7 @@ static Wg3Plan wg3_plan(int B, int CGi, int CGo, int H, int T, int d) {
     // everything a strip touches of dZ stays resident: rows + 2 d slots, and the A operand reads 32 KB from its first slot
     // one resident strip per SM leaves the tensor pipe idle while the strip's first rows are in flight: with small rows (C <= 16) take
     // half of the shared memory, so that two CTAs share an SM and one computes while the other loads
-    static const int cap_kb = getenv("TT_WG3_SMEM_KB") ? atoi(getenv("TT_WG3_SMEM_KB")) : 112;
-    static const int cap_cgo = getenv("TT_WG3_CAP_CGO") ? atoi(getenv("TT_WG3_CAP_CGO")) : 2;
-    const size_t cap = (size_t)(cap_kb > 0 && CGo <= cap_cgo ? cap_kb : 226) * 1024;
+    const size_t cap = (size_t)(CGo <= 2 ? 112 : 226) * 1024;
     const size_t budget = cap - 2048 - g.xring * x_slot - 32 * 1024;
     int max_rows = (int)std::min<size_t>(budget / z_slot, (size_t)kWg3MaxRows) - (3 * d - 1);   // the residue-class layout rounds the row count up to a multiple of d
     max_rows = std::max(max_rows, 1);
@@ -956,42 +928,31 @@ extern "C" int64_t tt_wgrad_scratch_floats(int B, int H, int T) {
     return need;
 }
 
-// common launch: A side `a` (channels Ca, rows Ha), B side `bsrc` (channels Cb, rows Hb)
-template <int KH, int KW, int RS>
-static int wgrad_any(const void* bsrc, const void* a, float* dw, float* db, int B, int Cb, int Ca, int cb_real, int ca_real, int Hb, int Ha, int T,
-                     int dilation, float* scratch, cudaStream_t stream) {
+// 1x1 layers: the ring kernel, A side dz (channels Cout), B side x (channels Cin)
+static int wgrad1x1(const void* x, const void* dz, float* dw, float* db, int B, int Cin, int Cout, int cin_real, int cout_real, int H, int T,
+                    float* scratch, cudaStream_t stream) {
     WgradParams p;
     p.partial = scratch;
-    p.B = B; p.T = T; p.Hz = Ha; p.Hx = Hb; p.CGi = Cb / 8; p.CGo = Ca / 8; p.d = dilation;
+    p.B = B; p.T = T; p.Hz = H; p.Hx = H; p.CGi = Cin / 8; p.CGo = Cout / 8;
     p.tap_group = 0;
     // ring depths: the loads are 2-16 KB rows with ~1 us latency each, so the prefetch distance - not bandwidth - sets the pace;
-    // take up to 8 A-side rows and up to 8 row-steps of B-side rows ahead, within ~170 KB of shared memory
+    // take up to 8 A-side rows and up to 8 B-side rows ahead, within ~170 KB of shared memory
     {
-        const int span = (KH - 1) * (KH == 3 ? dilation : 1);
-        const size_t z_slot = (size_t)(Ca / 8) * kStripTileT * 16, x_slot = (size_t)(Cb / 8) * (kStripTileT + 2 * (KW == 3 ? dilation : 0)) * 16 + 128;
+        const size_t z_slot = (size_t)(Cout / 8) * kStripTileT * 16, x_slot = (size_t)(Cin / 8) * kStripTileT * 16 + 128;
         p.z_slots = (int)std::max<size_t>(3, std::min<size_t>(kWgZSlots, (48 * 1024) / z_slot));
         int pf = 8;
-        while (pf > 2 && (span + 1 + pf * RS > 16 || (span + 1 + pf * RS) * x_slot > 120 * 1024)) --pf;
-        p.xring = span + 1 + pf * RS;
+        while (pf > 2 && (1 + pf) * x_slot > 120 * 1024) --pf;
+        p.xring = 1 + pf;
     }
-    const long long strips = wgrad_strips(B, Ha, T);
-    p.rows_per_strip = (int)((Ha + strips - 1) / strips);
-    dim3 grid((T + kStripTileT - 1) / kStripTileT, (Ha + p.rows_per_strip - 1) / p.rows_per_strip, B);
+    const long long strips = wgrad_strips(B, H, T);
+    p.rows_per_strip = (int)((H + strips - 1) / strips);
+    dim3 grid((T + kStripTileT - 1) / kStripTileT, (H + p.rows_per_strip - 1) / p.rows_per_strip, B);
     const int n_ctas = (int)(grid.x * grid.y * grid.z);
-    int npad = Cb >= 32 ? 32 : 16;
-    int rc, kxn = 0;
-    if constexpr (KH == 3 && KW == 3) {
-        if (Cb == 8) { kxn = 1; npad = 32; }
-    }
-    if (kxn) {
-        if constexpr (KH == 3 && KW == 3) rc = launch_wgrad<32, KH, KW, RS, 2, true>(bsrc, a, p, grid, stream);
-        else rc = TT_ERR_INVALID;
-    } else {
-        rc = npad == 32 ? launch_wgrad<32, KH, KW, RS, 2>(bsrc, a, p, grid, stream) : launch_wgrad<16, KH, KW, RS, 2>(bsrc, a, p, grid, stream);
-    }
+    const int npad = Cin >= 32 ? 32 : 16;
+    const int rc = npad == 32 ? launch_wgrad<32, 1, 2>(x, dz, p, grid, stream) : launch_wgrad<16, 1, 2>(x, dz, p, grid, stream);
     if (rc) return rc;
-    const int total = (KH * KW + 1) * ca_real * cb_real;
-    wgrad_reduce_kernel<<<(total + 7) / 8, 256, 0, stream>>>(scratch, n_ctas, npad, KH * KW, ca_real, cb_real, dw, db, kxn);
+    const int total = 2 * cout_real * cin_real;
+    wgrad_reduce_kernel<<<(total + 7) / 8, 256, 0, stream>>>(scratch, n_ctas, npad, 1, cout_real, cin_real, dw, db);
     tt_count_launches(1);
     TT_CUDA_CHECK(cudaGetLastError());
     return TT_OK;
@@ -1043,14 +1004,10 @@ extern "C" int tt_conv_wgrad_same(const void* x, const void* dz, float* dw, floa
     TT_REQUIRE((k == 3 && dilation >= 1 && dilation <= 3) || k == 1, "wgrad: 3x3 (dilation 1..3) or 1x1");
     if (B <= 0 || H <= 0 || T <= 0) return TT_OK;
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (k == 3) {
-        static const bool legacy = getenv("TT_WGRAD_LEGACY") != nullptr;       // A/B switch: the one-MMA-per-tap kernel
-        if (!legacy) return wgrad3_dispatch(x, dz, dw, db, B, Cin, Cout, cin_real, cout_real, H, T, dilation, scratch, stream);
-        return wgrad_any<3, 3, 1>(x, dz, dw, db, B, Cin, Cout, cin_real, cout_real, H, H, T, dilation, scratch, stream);
-    }
+    if (k == 3) return wgrad3_dispatch(x, dz, dw, db, B, Cin, Cout, cin_real, cout_real, H, T, dilation, scratch, stream);
     // (1x1 layers through resident strips - plain or with four image rows per MMA - were measured slower than the ring kernel with its
     // co-resident CTAs: 293 vs 205 us at the largest stage; the ring kernel without its "ones" MMA stays)
-    return wgrad_any<1, 1, 1>(x, dz, dw, db, B, Cin, Cout, cin_real, cout_real, H, H, T, 1, scratch, stream);
+    return wgrad1x1(x, dz, dw, db, B, Cin, Cout, cin_real, cout_real, H, T, scratch, stream);
 }
 
 template <int CGC, int CGF>
@@ -1081,6 +1038,15 @@ static int launch_wgrad_ud(const void* fine, const void* coarse, float* dw, floa
     return TT_OK;
 }
 
+static int wgrad_ud_dispatch(const void* fine, const void* coarse, float* dw, float* db, int B, int Cfine, int Ccoarse, int cfine_real,
+                             int ccoarse_real, int Hfine, int Hcoarse, int T, float* scratch, cudaStream_t stream) {
+#define TT_WGUD(CC, CF) if (Ccoarse == CC * 8 && Cfine == CF * 8) return launch_wgrad_ud<CC, CF>(fine, coarse, dw, db, B, cfine_real, ccoarse_real, Hfine, Hcoarse, T, scratch, stream);
+    TT_WGUD(1, 1) TT_WGUD(2, 1) TT_WGUD(4, 2) TT_WGUD(8, 4)
+#undef TT_WGUD
+    tt_set_error("wgrad_updown: no kernel for %d coarse / %d fine channels (padded)", Ccoarse, Cfine);
+    return TT_ERR_UNSUPPORTED;
+}
+
 extern "C" int tt_conv_wgrad_updown(const void* fine, const void* coarse, float* dw, float* db, int B, int Cfine, int Ccoarse, int cfine_real,
                                     int ccoarse_real, int Hfine, int Hcoarse, int T, int transposed, float* scratch, void* stream_) {
     TT_REQUIRE(fine && coarse && dw && scratch, "null argument");
@@ -1090,16 +1056,8 @@ extern "C" int tt_conv_wgrad_updown(const void* fine, const void* coarse, float*
     if (B <= 0 || T <= 0 || Hcoarse <= 0) return TT_OK;
     cudaStream_t stream = (cudaStream_t)stream_;
     // the coarse tensor (sconv: the output gradient; tconv: the layer input) is the A side, the fine one (rows 2q + kh) the B side
-    static const bool legacy = getenv("TT_WGRAD_LEGACY") != nullptr;
-    int rc = TT_ERR_UNSUPPORTED;
-    float* dbc = transposed ? nullptr : db;
-    if (!legacy) {
-#define TT_WGUD(CC, CF) if (Ccoarse == CC * 8 && Cfine == CF * 8) rc = launch_wgrad_ud<CC, CF>(fine, coarse, dw, dbc, B, cfine_real, ccoarse_real, Hfine, Hcoarse, T, scratch, stream);
-        TT_WGUD(1, 1) TT_WGUD(2, 1) TT_WGUD(4, 2) TT_WGUD(8, 4)
-#undef TT_WGUD
-    }
-    if (rc == TT_ERR_UNSUPPORTED)
-        rc = wgrad_any<4, 1, 2>(fine, coarse, dw, dbc, B, Cfine, Ccoarse, cfine_real, ccoarse_real, Hfine, Hcoarse, T, 1, scratch, stream);
+    const int rc = wgrad_ud_dispatch(fine, coarse, dw, transposed ? nullptr : db, B, Cfine, Ccoarse, cfine_real, ccoarse_real, Hfine, Hcoarse, T,
+                                     scratch, stream);
     if (rc || !transposed || !db) return rc;
     // ConvTranspose2d bias: sum of the FINE tensor (the output gradient) over all pixels
     const int CG = Cfine / 8, chunks = 64;
@@ -1128,11 +1086,11 @@ extern "C" int tt_conv_wgrad_lat(const void* tall, const void* flat, float* dw, 
     cudaStream_t stream = (cudaStream_t)stream_;
     WgradParams p;
     p.partial = scratch;
-    p.B = B; p.T = T; p.Hz = 1; p.Hx = H; p.CGi = Ctall / 8; p.CGo = Cflat / 8; p.d = 1;
+    p.B = B; p.T = T; p.Hz = 1; p.Hx = H; p.CGi = Ctall / 8; p.CGo = Cflat / 8;
     p.rows_per_strip = 1; p.z_slots = 1; p.tap_group = kLatTapGroup; p.xring = kLatTapGroup + 2;
     const int groups = (H + kLatTapGroup - 1) / kLatTapGroup;
     dim3 grid((T + kStripTileT - 1) / kStripTileT, groups, B);
-    const int rc = launch_wgrad<64, kLatTapGroup, 1, 1, 4>(tall, flat, p, grid, stream);
+    const int rc = launch_wgrad<64, kLatTapGroup, 4>(tall, flat, p, grid, stream);
     if (rc) return rc;
     const int total = (H + 1) * cflat_real * ctall_real;
     wgrad_reduce_groups_kernel<<<(total + 127) / 128, 128, 0, stream>>>(scratch, (int)grid.x, groups, B, kLatTapGroup, 64, H, cflat_real, ctall_real, dw, db);

@@ -6,11 +6,12 @@ The reference's loss step (reference: experiments/train.py:393-500) on the CUDA 
                                                     losses, backward, gradient all-reduce (NCCL, when a process group is
                                                     given), clip_grad_norm_(10), AdamW
 
-Forward kernels are the inference kernels (tcgen05 strips); every layer is a torch.autograd.Function whose backward calls
-the native gradient kernels of csrc/train_kernels.cu (direct-convolution dgrad / tiled wgrad on fp32 NCHW, CUDA cores); the
-residual blocks recompute their intermediate and take their data gradients on the tensor cores (tt_conv_same, the gradient
-operand split into bf16 hi + lo parts).  PyTorch's autograd engine only walks the graph and accumulates `.grad`; there is no cuDNN / ATen compute on the
-path except layout conversions (permute / dtype copies) between the inference layouts (C8 planar / packed4 bf16) and NCHW.
+Every layer is a torch.autograd.Function whose forward is the inference kernel (tcgen05 strips) and whose backward stays in the
+bf16 inference layouts (C8 planar / packed 4-channel): weight gradients are tcgen05 GEMMs over the pixel axis with a fixed-order
+reduction (csrc/wgrad_tc.cu), data gradients are the forward kernels on transformed weights without activation, and ELU
+derivatives, skip connections and re-layouts are one-pass bf16 kernels; the losses, clip and AdamW have kernels of their own
+(csrc/loss_kernels.cu, csrc/train_kernels.cu).  PyTorch's autograd engine only walks the graph and accumulates `.grad`; there
+is no cuDNN / ATen compute on the path.
 Differences to the reference that do not change values: the CQT target is computed once (the reference computes it twice,
 train.py:404 and modules.py:366 -> :88); no `.item()` host syncs inside the step; activation gradients travel in bf16 between
 layers (the reference runs the forward under fp16 autocast).
@@ -77,131 +78,8 @@ def compute_step_losses(model, audio, ground_truth, multipliers=None, late_start
 
 
 # ---------------------------------------------------------------------------------------------------------------
-# native gradient kernels on fp32 NCHW
-# ---------------------------------------------------------------------------------------------------------------
-def _geom(kh, kw, sh=1, dh=1, dw=1, ph=0, pw=0):
-    return dict(KH=kh, KW=kw, sh=sh, dh=dh, dw=dw, ph=ph, pw=pw)
-
-
-def _conv_fwd(x, w, bias, g, act):
-    B, Cin, Hin, T = x.shape
-    Cout = w.size(0)
-    Hout = (Hin + 2 * g['ph'] - g['dh'] * (g['KH'] - 1) - 1) // g['sh'] + 1
-    y = torch.empty((B, Cout, Hout, T), dtype=torch.float32, device=x.device)
-    _lib.check(_lib.lib().tt_conv_fwd_f32(_p(x), _p(w), _p(bias), _p(y), B, Cin, Hin, T, Cout, g['KH'], g['KW'], g['sh'], g['dh'],
-                                          g['dw'], g['ph'], g['pw'], int(act), _s(x)))
-    return y
-
-
-def _conv_bwd_data(dz, w, x_shape, g):
-    """dz (B, Cout, Hout, T), w (Cout, Cin, KH, KW) -> dx of shape x_shape (B, Cin, Hin, T)."""
-    B, Cin, Hin, T = x_shape
-    Cout, Hout = dz.size(1), dz.size(2)
-    dx = torch.empty(x_shape, dtype=torch.float32, device=dz.device)
-    _lib.check(_lib.lib().tt_conv_bwd_data_f32(_p(dz), _p(w), _p(dx), B, Cin, Hin, T, Cout, g['KH'], g['KW'], g['sh'], g['dh'],
-                                               g['dw'], g['ph'], g['pw'], Hout, _s(dz)))
-    return dx
-
-
-def _conv_bwd_weight(x, dz, w_shape, g, want_bias):
-    """x (B, Cin, Hin, T), dz (B, Cout, Hout, T) -> (dW of shape w_shape, db (Cout) or None)."""
-    B, Cin, Hin, T = x.shape
-    Cout, Hout = dz.size(1), dz.size(2)
-    dw = torch.zeros(w_shape, dtype=torch.float32, device=x.device)
-    db = torch.zeros(Cout, dtype=torch.float32, device=x.device) if want_bias else None
-    _lib.check(_lib.lib().tt_conv_bwd_weight_f32(_p(x), _p(dz), _p(dw), _p(db), B, Cin, Hin, T, Cout, g['KH'], g['KW'], g['sh'],
-                                                 g['dh'], g['dw'], g['ph'], g['pw'], Hout, _s(x)))
-    return dw, db
-
-
-def _elu_bwd(dy, a):
-    dz = torch.empty_like(dy)
-    _lib.check(_lib.lib().tt_elu_bwd(_p(dy), _p(a), _p(dz), dy.numel(), _s(dy)))
-    return dz
-
-
-def _channel_sum(dz):
-    B, C = dz.shape[:2]
-    db = torch.zeros(C, dtype=torch.float32, device=dz.device)
-    _lib.check(_lib.lib().tt_channel_sum(_p(dz), _p(db), B, C, dz.numel() // (B * C), _s(dz)))
-    return db
-
-
-# layout plumbing: inference layouts <-> NCHW fp32
-def _nchw(t, c):
-    """internal activation (C8 planar 5-D, packed4 4-D bf16, or interleaved coefficients (B,F,T,2) fp32) -> (B, c, H, T) fp32."""
-    if t.dtype == torch.float32:
-        return t.permute(0, 3, 1, 2).contiguous()
-    return (P.from_p4(t, c) if t.dim() == 4 else P.from_c8(t, c)).contiguous()
-
-
-def _like(nchw, ref):
-    """(B, c, H, T) fp32 gradient -> the layout / dtype of the forward tensor `ref`."""
-    if ref.dtype == torch.float32:
-        return nchw.permute(0, 2, 3, 1).contiguous()
-    return P.to_p4(nchw) if ref.dim() == 4 else P.to_c8(nchw)
-
-
-# ---------------------------------------------------------------------------------------------------------------
 # autograd Functions: fast forward kernel + native backward kernels
 # ---------------------------------------------------------------------------------------------------------------
-class _ConvFn(torch.autograd.Function):
-    """A regular conv layer (+ optional ELU): forward through `run(x)` (an inference kernel), backward generic."""
-
-    @staticmethod
-    def forward(ctx, x, weight, bias, run, geom, cin, cout, act):
-        y = run(x)
-        ctx.save_for_backward(x, y, weight)
-        ctx.meta = (geom, cin, cout, act)
-        return y
-
-    @staticmethod
-    def backward(ctx, gy):
-        x, y, weight = ctx.saved_tensors
-        geom, cin, cout, act = ctx.meta
-        xn, dy = _nchw(x, cin), _nchw(gy, cout)
-        dz = _elu_bwd(dy, _nchw(y, cout)) if act else dy
-        w = weight.detach().float().contiguous()
-        dw, db = _conv_bwd_weight(xn, dz, w.shape, geom, True)
-        gx = _like(_conv_bwd_data(dz, w, xn.shape, geom), x) if ctx.needs_input_grad[0] else None
-        return gx, dw, db, None, None, None, None, None
-
-
-class _ConvTFn(torch.autograd.Function):
-    """A transposed conv layer + ELU (weight (Cin, Cout, KH, KW)); optional per-row bias table handled by the caller."""
-
-    @staticmethod
-    def forward(ctx, x, weight, bias, run, geom, cin, cout):
-        y = run(x)
-        ctx.save_for_backward(x, y, weight)
-        ctx.meta = (geom, cin, cout)
-        return y
-
-    @staticmethod
-    def backward(ctx, gy):
-        x, y, weight = ctx.saved_tensors
-        geom, cin, cout = ctx.meta
-        xn = _nchw(x, cin)
-        dz = _elu_bwd(_nchw(gy, cout), _nchw(y, cout))
-        w = weight.detach().float().contiguous()               # (cin, cout, KH, KW) = the regular conv y-space -> x-space
-        # weight gradient: regular-conv roles swapped (its input is dz, its output-side gradient is x)
-        dw, _ = _conv_bwd_weight(dz, xn, w.shape, geom, False)
-        db = _channel_sum(dz)
-        gx = _like(_conv_fwd(dz, w, None, geom, False), x)
-        return gx, dw, db, None, None, None, None
-
-
-def _conv_same_hi_lo(dz, wp, c, k, d):
-    """
-    Data-gradient conv on the tensor cores with the gradient operand split into bf16 hi + lo parts (two passes, summed in fp32):
-    the weights are the bf16 values the forward pass used (so they are exact for the function being differentiated), and the split
-    keeps ~16 mantissa bits of dz - weight gradients are long sums with heavy cancellation and do not tolerate 8-bit gradients.
-    """
-    hi = P.to_c8(dz)
-    lo = P.to_c8(dz - P.from_c8(hi, c))
-    return (P.from_c8(ops.conv_same(hi, wp, None, k, d), c) + P.from_c8(ops.conv_same(lo, wp, None, k, d), c)).contiguous()
-
-
 # ---- residual blocks: the whole backward in the inference layouts (bf16), convolutions AND weight gradients on the tensor cores ----
 def _ew(fn_name, *tensors):
     """element-wise bf16 kernel over tensors of one common layout -> new tensor like the first"""
@@ -373,17 +251,16 @@ _LAT_SCRATCH = {}
 
 
 def _wgrad_lat(tall8, flat8, ctall, cflat, dw, db, row_sums):
-    """tt_conv_wgrad_lat: accumulates into dw (cflat.., ctall, H, 1) [first cflat rows], db (cflat) and row_sums (ctall, H) (either may be None)."""
+    """tt_conv_wgrad_lat: accumulates into dw (cflat.., ctall, H, 1) [first cflat rows], db (cflat) and row_sums (ctall, H) (either may be None).
+    The kernel takes up to 128 flat-side channels; wider latents go through it in slices of 128 (a slice of the 1-row latents is a tiny copy)."""
     B, CGt, H, T, _ = tall8.shape
     lib = _lib.lib()
     scratch = _scratch(_LAT_SCRATCH, tall8.device, int(lib.tt_wgrad_lat_scratch_floats(B, H, T)))
-    _lib.check(lib.tt_conv_wgrad_lat(_p(tall8), _p(flat8), _p(dw), _p(db), _p(row_sums), B, CGt * 8, flat8.size(1) * 8, ctall, cflat, H, T,
-                                     _p(scratch), _s(tall8)))
-
-
-def _lat_tc_ok(c_tall, c_flat_pad):
-    """The tensor-core kernels of the two (H, 1)-kernel layers take up to 64 embedding / 128 latent channels (the base model's sizes)."""
-    return P.pad8(c_tall) in (16, 32, 64) and c_flat_pad <= 128
+    for c0 in range(0, cflat, 128):
+        c1 = min(cflat, c0 + 128)
+        flat = flat8[:, c0 // 8:c0 // 8 + 16].contiguous()
+        _lib.check(lib.tt_conv_wgrad_lat(_p(tall8), _p(flat), _p(dw[c0:c1]), _p(None if db is None else db[c0:c1]), _p(row_sums if c0 == 0 else None),
+                                         B, CGt * 8, flat.size(1) * 8, ctall, c1 - c0, H, T, _p(scratch), _s(tall8)))
 
 
 class _LatFn(torch.autograd.Function):
@@ -419,11 +296,6 @@ def _pairs_to_c8(pairs):
     out = torch.empty((B, 1, F_, T, 8), dtype=torch.bfloat16, device=pairs.device)
     _lib.check(_lib.lib().tt_pairs_to_c8(_p(pairs), B * F_ * T, _p(out), _s(pairs)))
     return out
-
-
-def _edge_tc_ok(x_like, c):
-    """The native backward of the first / last 3x3 conv needs the packed 4-channel stage layout (model_complexity 1 and 2)."""
-    return x_like.dim() == 4 and c <= 4
 
 
 class _InFn(torch.autograd.Function):
@@ -566,11 +438,7 @@ def _encoder(enc, coeffs):
     ch = enc.channels
     w_in, b_in, w_lat, b_lat = enc._packed()
     ci = enc.convin[0]
-    if enc.packed4:
-        x = _InFn.apply(coeffs, ci.weight, ci.bias, lambda t: ops.conv_in(t, w_in, b_in, ch[0], packed4=True), ch[0])
-    else:
-        x = _ConvFn.apply(coeffs, ci.weight, ci.bias, lambda t: ops.conv_in(t, w_in, b_in, ch[0], packed4=enc.packed4),
-                          _geom(3, 3, ph=1, pw=1), 2, ch[0], True)
+    x = _InFn.apply(coeffs, ci.weight, ci.bias, lambda t: ops.conv_in(t, w_in, b_in, ch[0], packed4=True), ch[0])
     emb = [x]
     for i, blk in enumerate((enc.block1, enc.block2, enc.block3, enc.block4)):
         for rb in (blk.block1, blk.block2, blk.block3):
@@ -584,10 +452,7 @@ def _encoder(enc, coeffs):
         x = _DownFn.apply(x, sc.weight, sc.bias, run_down, ch[i], ch[i + 1])
         emb.append(x)
     cl = enc.convlat
-    if _lat_tc_ok(ch[4], enc.latent_pad):
-        return _LatFn.apply(x, cl.weight, cl.bias, lambda t: ops.conv_lat(t, w_lat, b_lat, enc.latent_pad), ch[4], enc.latent_size, enc.latent_pad), emb
-    return _ConvFn.apply(x, cl.weight, cl.bias, lambda t: ops.conv_lat(t, w_lat, b_lat, enc.latent_pad),
-                         _geom(cl.weight.size(2), 1), ch[4], enc.latent_size, False), emb
+    return _LatFn.apply(x, cl.weight, cl.bias, lambda t: ops.conv_lat(t, w_lat, b_lat, enc.latent_pad), ch[4], enc.latent_size, enc.latent_pad), emb
 
 
 class _IndicatorFn(torch.autograd.Function):
@@ -608,29 +473,19 @@ class _IndicatorFn(torch.autograd.Function):
     def backward(ctx, gy):
         lat, y, weight = ctx.saved_tensors
         flag, d, c0 = ctx.meta
-        if _lat_tc_ok(c0, lat.size(1) * 8):
-            # inference layouts end to end: ELU derivative, tap-grouped tensor-core weight gradient (rows 0 .. D-1; the indicator row and
-            # the bias are row sums of dz), data gradient = the Encoder.convlat forward kernel on the first D weight rows
-            dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)
-            h0 = y.size(2)
-            dw = torch.zeros(weight.shape, dtype=torch.float32, device=lat.device)
-            rows = torch.zeros((c0, h0), dtype=torch.float32, device=lat.device)
-            _wgrad_lat(dz, lat, c0, d, dw, None, rows)
-            dw[d, :, :, 0] = flag * rows
-            db = rows.sum(dim=1)
-            d_pad = lat.size(1) * 8
-            wl, zl = _bw_pack(weight, 'decinT', lambda: (P.pack_lat(weight.detach().float()[:d], d_pad), torch.zeros(d_pad, device=lat.device)))
-            glat = ops.conv_lat(dz, wl, zl, d_pad)
-            return glat, dw, db, None, None, None, None
-        geom = _geom(weight.size(2), 1)
-        ln = _nchw(lat, d)                                                       # (B, D, 1, T)
-        full = torch.cat((ln, torch.full_like(ln[:, :1], flag)), dim=1)          # (B, D+1, 1, T)
-        dz = _elu_bwd(_nchw(gy, c0), _nchw(y, c0))
-        w = weight.detach().float().contiguous()                                # (D+1, C0, H0, 1)
-        dw, _ = _conv_bwd_weight(dz, full, w.shape, geom, False)
-        db = _channel_sum(dz)
-        gfull = _conv_fwd(dz, w, None, geom, False)                             # (B, D+1, 1, T)
-        return _like(gfull[:, :d].contiguous(), lat), dw, db, None, None, None, None
+        # ELU derivative, tap-grouped tensor-core weight gradient (rows 0 .. D-1; the indicator row and the bias are row sums of dz),
+        # data gradient = the Encoder.convlat forward kernel on the first D weight rows
+        dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)
+        h0 = y.size(2)
+        dw = torch.zeros(weight.shape, dtype=torch.float32, device=lat.device)
+        rows = torch.zeros((c0, h0), dtype=torch.float32, device=lat.device)
+        _wgrad_lat(dz, lat, c0, d, dw, None, rows)
+        dw[d, :, :, 0] = flag * rows
+        db = rows.sum(dim=1)
+        d_pad = lat.size(1) * 8
+        wl, zl = _bw_pack(weight, 'decinT', lambda: (P.pack_lat(weight.detach().float()[:d], d_pad), torch.zeros(d_pad, device=lat.device)))
+        glat = ops.conv_lat(dz, wl, zl, d_pad)
+        return glat, dw, db, None, None, None, None
 
 
 def _decoder(dec, lat, reconstruct, skips=None):
@@ -655,9 +510,7 @@ def _decoder(dec, lat, reconstruct, skips=None):
     if skips is not None:
         x = _SkipAddFn.apply(x, skips[0][1], skips[0][0])
     co = dec.convout
-    if dec.packed4:
-        return _OutFn.apply(x, co.weight, co.bias, lambda t: ops.conv_out(t, w_out, b_out, ch[4]), ch[4])
-    return _ConvFn.apply(x, co.weight, co.bias, lambda t: ops.conv_out(t, w_out, b_out, ch[4]), _geom(3, 3, ph=1, pw=1), ch[4], 2, False)
+    return _OutFn.apply(x, co.weight, co.bias, lambda t: ops.conv_out(t, w_out, b_out, ch[4]), ch[4])
 
 
 def allreduce_mean_gradients(params, group, flat=None):
