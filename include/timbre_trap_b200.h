@@ -209,6 +209,10 @@ int tt_pairs_to_c8(const float* pairs, int64_t n, void* c8, void* stream);
 /* channel 0 of n interleaved pairs through an output non-linearity: 0 identity, 1 relu (TimbreTrapMag.decode, modules.py:976),
  * 2 sigmoid (TimbreTrapMagDB.decode :1052), 3 tanh(relu(.)) (Mag decode + to_activations :996) */
 int tt_channel0_activation(const float* pairs, int64_t n, int mode, float* out, void* stream);
+/* its backward, for the loss step's one-channel tensors kept as pairs (x, 0): pairs_in = the n pre-activation pairs, gpairs_out = the
+ * gradient of the output pairs (f(v0), 0) (channel 0 is read); gpairs_in = (g * f'(v0), 0), relu'(0) = 0.  Same modes; mode 0 is the
+ * backward of taking channel 0 and of widening x -> (x, 0) */
+int tt_channel0_activation_bwd(const float* pairs_in, const float* gpairs_out, int64_t n, int mode, float* gpairs_in, void* stream);
 
 /*
  * ---- audio front-end and evaluation metric on the device (SURVEY.md section 8f-3 / 8f-4) -----------------------------------
@@ -286,6 +290,15 @@ int tt_sum_sq_diff_bwd(const float* a, const float* b, const float* gout, double
 int tt_transcription_loss_bwd(const float* estimate, const float* target, const float* gout, int B, int F, int T,
                               int weight_positive_class, float* gest, void* stream);
 int tt_activations_bwd(const float* coeffs, const float* dact, float* dcoeffs, int64_t n, void* stream);
+/* TimbreTrapFiLM's Decoder.convin (modules.py:801-809, 838-840): ConvTranspose2d(D, C0, (H0, 1)) on gamma * z + beta, with
+ * gamma / beta = film_layer.gamma / .beta of the one-hot condition whose 1 is in column `hot` (0 transcribe, 1 reconstruct).
+ * G (D, C0, H0) and rows (C0, H0) are tt_conv_wgrad_lat's dw and tall_row_sums for flat = latents z, tall = output gradient dz;
+ * w (D, C0, H0) the weight, gamma_w / beta_w (D, 2), gamma_b / beta_b (D) the Linear parameters.  WRITES dw = gamma G + beta rows,
+ * db (C0) = sum_h rows, and the Linear gradients dgamma_w / dbeta_w (D, 2) (column hot = <W[d], G[d]> / <W[d], rows>, the other 0),
+ * dgamma_b / dbeta_b (D).  One CTA per latent channel, fixed-order reductions (bit-reproducible). */
+int tt_film_convin_grad(const float* G, const float* rows, const float* w, const float* gamma_w, const float* gamma_b,
+                        const float* beta_w, const float* beta_b, int D, int C0, int H0, int hot, float* dw, float* db,
+                        float* dgamma_w, float* dgamma_b, float* dbeta_w, float* dbeta_b, void* stream);
 /* clip_grad_norm_ + AdamW (train.py:493-496): accumulate sum g^2 of every gradient tensor into *acc (double, zeroed by the
  * caller), then one tt_adamw_step per tensor applies the common clip factor min(1, max_norm / (norm + 1e-6)) and the update */
 int tt_grad_sumsq(const float* g, int64_t n, double* acc, void* stream);

@@ -1,10 +1,11 @@
-"""Times the loss step of BASELINE.json configs[3] (batch 8 x 9 s per GPU) and checks data-parallel gradients when run under torchrun."""
+"""Times the loss step of BASELINE.json configs[3] (batch 8 x 9 s per GPU) and checks data-parallel gradients when run under torchrun.
+Usage: train_step_bench.py [batch] [steps] [base|film|mag|magdb] - the model class to train (default base = TimbreTrap)."""
 import os, sys, time, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import torch
 import torch.distributed as dist
-from timbre_trap_b200.framework import TimbreTrap
+from timbre_trap_b200.framework import TimbreTrap, TimbreTrapFiLM, TimbreTrapMag, TimbreTrapMagDB
 from timbre_trap_b200.framework.train import TrainStep
 
 rank, world, local = int(os.environ.get('RANK', 0)), int(os.environ.get('WORLD_SIZE', 1)), int(os.environ.get('LOCAL_RANK', 0))
@@ -15,8 +16,12 @@ if world > 1:
     group = dist.group.WORLD
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 8
 steps = int(sys.argv[2]) if len(sys.argv) > 2 else 3
+variant = sys.argv[3] if len(sys.argv) > 3 else 'base'
+classes = dict(base=TimbreTrap, film=TimbreTrapFiLM, mag=TimbreTrapMag, magdb=TimbreTrapMagDB)
+if variant not in classes:
+    sys.exit(f'unknown variant {variant!r}: one of {", ".join(classes)}')
 torch.manual_seed(0)
-model = TimbreTrap(22050, 9, 60, 3, latent_size=128, model_complexity=2).cuda()
+model = classes[variant](22050, 9, 60, 3, latent_size=128, model_complexity=2).cuda()
 g = torch.Generator().manual_seed(100 + rank)
 audio = (torch.rand((B, 1, 3 * 66150), generator=g) * 2 - 1).cuda()
 gt = torch.zeros((B, 540, 3072))
@@ -54,7 +59,7 @@ ms = a.elapsed_time(b) / steps
 if world > 1:
     t = torch.tensor([ms], device='cuda'); dist.all_reduce(t, op=dist.ReduceOp.MAX); ms = float(t)
 if rank == 0:
-    print(json.dumps(dict(workload='loss step, base model, batch %d x 9 s per GPU' % B, n_gpus=world, ms_per_step=ms,
+    print(json.dumps(dict(workload='loss step, %s model, batch %d x 9 s per GPU' % (variant, B), n_gpus=world, ms_per_step=ms,
                           audio_s_per_s=world * B * 9 / (ms * 1e-3), losses={k: float(v) for k, v in res.items()},
                           peak_mem_gb=torch.cuda.max_memory_allocated() / 1e9)))
 if world > 1: dist.destroy_process_group()

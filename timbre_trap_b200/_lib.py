@@ -50,6 +50,7 @@ SIGNATURES = {
     'tt_widen_pairs': (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     'tt_pairs_to_c8': (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     'tt_channel0_activation': (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
+    'tt_channel0_activation_bwd': (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     'tt_resample_mono': (c_int, [c_void_p, c_int, c_int64, c_void_p, c_int, c_int, c_int, c_void_p, c_int64, c_void_p, c_void_p]),
     'tt_rasterise_pitches': (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     'tt_sdr_correlations': (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
@@ -68,6 +69,7 @@ SIGNATURES = {
     'tt_sum_sq_diff_bwd': (c_int, [c_void_p] * 3 + [ctypes.c_double] + [c_void_p] * 2 + [c_int64, c_void_p]),
     'tt_transcription_loss_bwd': (c_int, [c_void_p] * 3 + [c_int] * 4 + [c_void_p, c_void_p]),
     'tt_activations_bwd': (c_int, [c_void_p] * 3 + [c_int64, c_void_p]),
+    'tt_film_convin_grad': (c_int, [c_void_p] * 7 + [c_int] * 4 + [c_void_p] * 7),
     'tt_grad_sumsq': (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     'tt_adamw_step': (c_int, [c_void_p] * 4 + [c_int64, c_void_p] + [ctypes.c_float] * 6 + [c_int, c_void_p]),
     'tt_to_decibels': (c_int, [c_void_p, c_int, c_int64, c_int, c_void_p, c_void_p, c_void_p]),

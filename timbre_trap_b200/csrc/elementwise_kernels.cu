@@ -50,6 +50,27 @@ __global__ void channel0_activation_kernel(const float2* __restrict__ pairs, lon
     }
 }
 
+// backward of channel0_activation seen as pairs -> pairs (f(v0), 0) (the loss step keeps one-channel tensors as such pairs):
+// gin = (gout.x * f'(v0), 0), with relu'(0) = 0 as in torch; gout's channel 1 meets a constant and gets no gradient through
+__global__ void channel0_activation_bwd_kernel(const float2* __restrict__ pairs, const float2* __restrict__ gout, long long n, int mode,
+                                               float2* __restrict__ gin) {
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const float v = ld_stream(pairs + i).x;
+        float g = ld_stream(gout + i).x;
+        if (mode == 1) {
+            g = v > 0.f ? g : 0.f;
+        } else if (mode == 2) {
+            const float s = 1.f / (1.f + expf(-v));
+            g *= (1.f - s) * s;
+        } else if (mode == 3) {
+            const float t = tanhf(v);
+            g = v > 0.f ? g * (1.f - t * t) : 0.f;
+        }
+        st_stream(gin + i, make_float2(g, 0.f));
+    }
+}
+
 // fp32 interleaved pairs (coefficients or their gradient, (B, F, T, 2)) -> C8 planar bf16 with one channel group (B, 1, F, T, 8),
 // channels 2..7 zero: the layout the tensor-core weight-gradient kernel reads
 __global__ void pairs_to_c8_kernel(const float2* __restrict__ pairs, long long n, uint4* __restrict__ c8) {
@@ -124,6 +145,18 @@ extern "C" int tt_channel0_activation(const float* pairs, int64_t n, int mode, f
     TT_REQUIRE(mode >= 0 && mode <= 3, "channel0_activation: mode must be 0..3");
     if (n <= 0) return TT_OK;
     channel0_activation_kernel<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>((const float2*)pairs, n, mode, out);
+    tt_count_launches(1);
+    TT_CUDA_CHECK(cudaGetLastError());
+    return TT_OK;
+}
+
+extern "C" int tt_channel0_activation_bwd(const float* pairs_in, const float* gpairs_out, int64_t n, int mode, float* gpairs_in,
+                                          void* stream) {
+    TT_REQUIRE(pairs_in && gpairs_out && gpairs_in, "null argument");
+    TT_REQUIRE(mode >= 0 && mode <= 3, "channel0_activation_bwd: mode must be 0..3");
+    if (n <= 0) return TT_OK;
+    channel0_activation_bwd_kernel<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>((const float2*)pairs_in, (const float2*)gpairs_out, n,
+                                                                                   mode, (float2*)gpairs_in);
     tt_count_launches(1);
     TT_CUDA_CHECK(cudaGetLastError());
     return TT_OK;

@@ -57,6 +57,64 @@ __global__ void activations_bwd_kernel(const float2* __restrict__ c, const float
     }
 }
 
+// TimbreTrapFiLM's Decoder.convin (modules.py:801-809, 838-840): y = ConvTranspose2d(W (D, C0, H0, 1), b)(u), u = gamma * z + beta per
+// latent channel, gamma = film_layer.gamma(cond), beta = film_layer.beta(cond), cond one-hot with its 1 in column `hot`.  From the
+// tensor-core sums G[d,c,h] = sum_{b,t} dz[c,h,t] z[d,t] and rows[c,h] = sum_{b,t} dz[c,h,t] (tt_conv_wgrad_lat):
+//   dW[d] = gamma[d] G[d] + beta[d] rows,  db[c] = sum_h rows[c,h],  dgamma[d] = <W[d], G[d]>,  dbeta[d] = <W[d], rows>,
+// and the nn.Linear gradients: weight (D, 2) = dgamma (dbeta) in column `hot`, 0 in the other; bias = dgamma (dbeta).
+// One CTA per latent channel, fixed-order reductions (bit-reproducible).
+__global__ void __launch_bounds__(256) film_convin_grad_kernel(const float* __restrict__ G, const float* __restrict__ rows,
+                                                               const float* __restrict__ w, const float* __restrict__ gamma_w,
+                                                               const float* __restrict__ gamma_b, const float* __restrict__ beta_w,
+                                                               const float* __restrict__ beta_b, int C0, int H0, int hot,
+                                                               float* __restrict__ dw, float* __restrict__ db, float* __restrict__ dgamma_w,
+                                                               float* __restrict__ dgamma_b, float* __restrict__ dbeta_w,
+                                                               float* __restrict__ dbeta_b) {
+    const int d = blockIdx.x;
+    const int n = C0 * H0;
+    const float gamma = gamma_w[2 * d + hot] + gamma_b[d];         // F.linear(one-hot cond): the forward's fold reads the same value
+    const float beta = beta_w[2 * d + hot] + beta_b[d];
+    const float* Gd = G + (size_t)d * n;
+    const float* Wd = w + (size_t)d * n;
+    float* dWd = dw + (size_t)d * n;
+    float sg = 0.f, sb = 0.f;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const float g = Gd[i], r = rows[i], wi = Wd[i];
+        dWd[i] = fmaf(gamma, g, beta * r);
+        sg = fmaf(wi, g, sg);
+        sb = fmaf(wi, r, sb);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        sg += __shfl_xor_sync(0xffffffffu, sg, o);
+        sb += __shfl_xor_sync(0xffffffffu, sb, o);
+    }
+    __shared__ float red[2][8];
+    if ((threadIdx.x & 31) == 0) {
+        red[0][threadIdx.x >> 5] = sg;
+        red[1][threadIdx.x >> 5] = sb;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float a = 0.f, b = 0.f;
+        for (int k = 0; k < (int)(blockDim.x >> 5); ++k) {
+            a += red[0][k];
+            b += red[1][k];
+        }
+        dgamma_w[2 * d + hot] = a;
+        dgamma_w[2 * d + 1 - hot] = 0.f;
+        dgamma_b[d] = a;
+        dbeta_w[2 * d + hot] = b;
+        dbeta_w[2 * d + 1 - hot] = 0.f;
+        dbeta_b[d] = b;
+    }
+    for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < C0; c += gridDim.x * blockDim.x) {
+        float s = 0.f;
+        for (int h = 0; h < H0; ++h) s += rows[(size_t)c * H0 + h];
+        db[c] = s;
+    }
+}
+
 // sum of squares of one gradient tensor into a double accumulator (for clip_grad_norm_, train.py:493)
 __global__ void sumsq_kernel(const float* __restrict__ g, long long n, double* __restrict__ acc) {
     __shared__ double red[8];
@@ -123,6 +181,20 @@ extern "C" int tt_activations_bwd(const float* coeffs, const float* dact, float*
     TT_REQUIRE(coeffs && dact && dcoeffs, "null argument");
     if (n <= 0) return TT_OK;
     activations_bwd_kernel<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>((const float2*)coeffs, dact, (float2*)dcoeffs, n);
+    TT_CUDA_CHECK(cudaGetLastError());
+    tt_count_launches(1);
+    return TT_OK;
+}
+
+extern "C" int tt_film_convin_grad(const float* G, const float* rows, const float* w, const float* gamma_w, const float* gamma_b,
+                                   const float* beta_w, const float* beta_b, int D, int C0, int H0, int hot, float* dw, float* db,
+                                   float* dgamma_w, float* dgamma_b, float* dbeta_w, float* dbeta_b, void* stream) {
+    TT_REQUIRE(G && rows && w && gamma_w && gamma_b && beta_w && beta_b && dw && db && dgamma_w && dgamma_b && dbeta_w && dbeta_b,
+               "null argument");
+    TT_REQUIRE(D > 0 && C0 > 0 && H0 > 0, "film_convin_grad: bad shape D %d C0 %d H0 %d", D, C0, H0);
+    TT_REQUIRE(hot == 0 || hot == 1, "film_convin_grad: hot must be 0 (transcribe) or 1 (reconstruct)");
+    film_convin_grad_kernel<<<D, 256, 0, (cudaStream_t)stream>>>(G, rows, w, gamma_w, gamma_b, beta_w, beta_b, C0, H0, hot, dw, db, dgamma_w,
+                                                                dgamma_b, dbeta_w, dbeta_b);
     TT_CUDA_CHECK(cudaGetLastError());
     tt_count_launches(1);
     return TT_OK;

@@ -25,7 +25,7 @@ from .. import _lib
 from . import ops
 from . import packing as P
 from .cqt import CQT
-from .modules import _PackedCache
+from .modules import _PackedCache, _channel0, _widen
 from .objectives import compute_consistency_loss, compute_reconstruction_loss, compute_transcription_loss
 
 __all__ = ['compute_step_losses', 'TrainStep', 'allreduce_mean_gradients']
@@ -47,17 +47,26 @@ def compute_step_losses(model, audio, ground_truth, multipliers=None, late_start
     audio (B, 1, n*L) on the GPU, ground_truth (B_mpe, F, T) with B_mpe <= B (train.py:393-394, 429).
     Returns a dict of 0-dim tensors: reconstruction, transcription, consistency_spectral, consistency_score, total
     (train.py:424-458; `late_start` = True reproduces the epochs before n_epochs_late_start, where only the reconstruction
-    term enters the total).
+    term enters the total).  The model variants are scored as TrainStep optimises them: the reconstruction target is the variant's
+    own encoder input (model._features), the magnitude variants' outputs pass through their head as pairs (h, 0).
     """
     mult = dict(reconstruction=1, transcription=1, consistency=1)
     mult.update(multipliers or {})
+    head = model.HEAD_MODE
+
+    def decode(lat, reconstruct, skips):
+        y = model.decoder.forward_c8(lat, reconstruct, skips)
+        return y if head is None else _widen(_channel0(y, head))
     with torch.no_grad():
-        coefficients = model.sliCQ.encode_interleaved(audio)                      # (B, F, T, 2), the target, computed once
+        coefficients = model._features(audio)                                     # (B, F, T, 2), the target, computed once
         lat, emb = model.encoder.forward_c8(coefficients)
         skips = model._skips_c8(emb)
-        reconstruction = model.decoder.forward_c8(lat, True, skips).permute(0, 3, 1, 2)
-        transcription_coeffs = model.decoder.forward_c8(lat, False, skips)
-        transcription = model.to_activations(transcription_coeffs.permute(0, 3, 1, 2))
+        reconstruction = decode(lat, True, skips).permute(0, 3, 1, 2)
+        transcription_coeffs = decode(lat, False, skips)
+        if head is None:
+            transcription = model.to_activations(transcription_coeffs.permute(0, 3, 1, 2))
+        else:
+            transcription = _channel0(transcription_coeffs, _ACTIVATIONS_MODE[head])
         n_mpe = ground_truth.size(0)
         losses = dict(reconstruction=compute_reconstruction_loss(reconstruction, coefficients.permute(0, 3, 1, 2)),
                       transcription=compute_transcription_loss(transcription[:n_mpe], ground_truth.float(), True))
@@ -65,8 +74,8 @@ def compute_step_losses(model, audio, ground_truth, multipliers=None, late_start
         if mult['consistency']:
             lat_t, emb_t = model.encoder.forward_c8(transcription_coeffs)
             skips_t = model._skips_c8(emb_t)
-            trn_rec = model.decoder.forward_c8(lat_t, True, skips_t).permute(0, 3, 1, 2)
-            trn_scr = model.decoder.forward_c8(lat_t, False, skips_t).permute(0, 3, 1, 2)
+            trn_rec = decode(lat_t, True, skips_t).permute(0, 3, 1, 2)
+            trn_scr = decode(lat_t, False, skips_t).permute(0, 3, 1, 2)
             sp, sc = compute_consistency_loss(trn_rec[:n_mpe], trn_scr[:n_mpe], transcription_coeffs.permute(0, 3, 1, 2)[:n_mpe])
             losses['consistency_spectral'], losses['consistency_score'] = sp, sc
         if not late_start:
@@ -298,10 +307,20 @@ def _pairs_to_c8(pairs):
     return out
 
 
+def _two_channels(w, dim):
+    """A one-channel conv weight of the magnitude variants zero-padded to two channels along `dim`, as the forward packs run it
+    (Encoder._packed / Decoder._packed); two-channel weights pass through."""
+    if w.size(dim) == 2:
+        return w
+    return torch.cat((w, torch.zeros_like(w)), dim=dim)
+
+
 class _InFn(torch.autograd.Function):
     """Encoder.convin + ELU (modules.py:430-433) with a packed 4-channel output.  Backward: ELU derivative on the packed tensor; weight
     gradient on the tensor cores (both operands re-laid out to C8 planar bf16 by one-pass kernels); data gradient (only the consistency
-    pass asks for it) = the Decoder.convout forward kernel on transposed, flipped weights."""
+    pass asks for it) = the Decoder.convout forward kernel on transposed, flipped weights.  The one-channel convin of the magnitude
+    variants (modules.py:908-911) reads pairs (x, 0) against zero-padded weights: its weight gradient is the first input column of the
+    two-channel one."""
 
     @staticmethod
     def forward(ctx, coeffs, weight, bias, run, c0):
@@ -318,15 +337,19 @@ class _InFn(torch.autograd.Function):
         dw, db = _wgrad_same(_pairs_to_c8(coeffs), _as_c8(dz), 2, c0, 3, 1)
         gx = None
         if ctx.needs_input_grad[0]:
-            wt, zb = _bw_pack(weight, 'inT', lambda: (weight.detach().float().transpose(0, 1).flip(2, 3).contiguous(),      # (2, c0, 3, 3)
+            wt, zb = _bw_pack(weight, 'inT', lambda: (_two_channels(weight.detach().float(), 1).transpose(0, 1).flip(2, 3).contiguous(),  # (2, c0, 3, 3)
                                                       torch.zeros(2, device=dz.device)))
             gx = ops.conv_out(dz, wt, zb, c0)
+        if weight.size(1) == 1:
+            dw = dw[:, :1]
         return gx, dw, db, None, None
 
 
 class _OutFn(torch.autograd.Function):
     """Decoder.convout (modules.py:543, no activation) on a packed 4-channel input.  Backward: weight gradient on the tensor cores;
-    data gradient = the Encoder.convin forward kernel without ELU on transposed, flipped weights."""
+    data gradient = the Encoder.convin forward kernel without ELU on transposed, flipped weights.  The one-channel convout of the
+    magnitude variants (modules.py:913) runs as two channels with a zero second one: its gradients are the first rows of the
+    two-channel ones."""
 
     @staticmethod
     def forward(ctx, x, weight, bias, run, c):
@@ -341,11 +364,13 @@ class _OutFn(torch.autograd.Function):
         c = ctx.c
         gy = gy.contiguous()
         dw, db = _wgrad_same(_as_c8(x), _pairs_to_c8(gy), c, 2, 3, 1)
-        wt, zb = _bw_pack(weight, 'outT', lambda: (weight.detach().float().transpose(0, 1).flip(2, 3).contiguous(),         # (c, 2, 3, 3)
+        wt, zb = _bw_pack(weight, 'outT', lambda: (_two_channels(weight.detach().float(), 0).transpose(0, 1).flip(2, 3).contiguous(),  # (c, 2, 3, 3)
                                                    torch.zeros(c, device=gy.device)))
         B, F_, T, _ = gy.shape
         gx = torch.empty((B, F_, T, 4), dtype=torch.bfloat16, device=gy.device)
         _lib.check(_lib.lib().tt_conv_in(_p(gy), _p(gx), _p(wt), _p(zb), B, c, F_, T, 2, _s(gy)))
+        if weight.size(0) == 1:
+            dw, db = dw[:1], db[:1]
         return gx, dw, db, None, None
 
 
@@ -388,6 +413,50 @@ class _ActivationsFn(torch.autograd.Function):
         g = torch.empty_like(coeffs)
         _lib.check(_lib.lib().tt_activations_bwd(_p(coeffs), _p(gact.contiguous()), _p(g), gact.numel(), _s(coeffs)))
         return g
+
+
+def _channel0_bwd(pairs, gpairs, mode):
+    """(g * f'(v0), 0) for the pre-activation pairs v and the output-pair gradient g (tt_channel0_activation_bwd)."""
+    gpairs = gpairs.contiguous()
+    g = torch.empty_like(pairs)
+    _lib.check(_lib.lib().tt_channel0_activation_bwd(_p(pairs), _p(gpairs), pairs.numel() // 2, mode, _p(g), _s(pairs)))
+    return g
+
+
+class _HeadFn(torch.autograd.Function):
+    """The output head of the magnitude variants on the decoder's pairs (modules.py:976, 1052): (B, F, T, 2) -> pairs (f(v0), 0),
+    f = relu (mode 1) or sigmoid (mode 2); the one-channel output stays a pair with a zero second channel."""
+
+    @staticmethod
+    def forward(ctx, pairs, mode):
+        ctx.save_for_backward(pairs)
+        ctx.mode = mode
+        return _widen(_channel0(pairs, mode))
+
+    @staticmethod
+    def backward(ctx, g):
+        (pairs,) = ctx.saved_tensors
+        return _channel0_bwd(pairs, g, ctx.mode), None
+
+
+class _Channel0ActivationsFn(torch.autograd.Function):
+    """to_activations of the magnitude variants on the head's pairs (h, 0) -> (B, F, T): tanh(h) for TimbreTrapMag (modules.py:996;
+    mode 3, tanh(relu(h)) = tanh(h) as h >= 0), h for TimbreTrapMagDB (:1056-1075; mode 0)."""
+
+    @staticmethod
+    def forward(ctx, pairs, mode):
+        ctx.save_for_backward(pairs)
+        ctx.mode = mode
+        return _channel0(pairs, mode)
+
+    @staticmethod
+    def backward(ctx, gact):
+        (pairs,) = ctx.saved_tensors
+        return _channel0_bwd(pairs, _widen(gact), ctx.mode), None
+
+
+# tt_channel0_activation mode of a magnitude variant's to_activations, by its HEAD_MODE: relu head -> tanh, sigmoid head -> identity
+_ACTIVATIONS_MODE = {1: 3, 2: 0}
 
 
 class _SqDiffFn(torch.autograd.Function):
@@ -488,14 +557,71 @@ class _IndicatorFn(torch.autograd.Function):
         return glat, dw, db, None, None, None, None
 
 
+class _FiLMConvInFn(torch.autograd.Function):
+    """
+    TimbreTrapFiLM: the FiLM layer and Decoder.convin (modules.py:801-809, 838-840), y = ELU(convT(gamma * z + beta)) with gamma / beta
+    = film_layer.gamma / .beta of the one-hot condition [transcribe, not transcribe] (`hot` = the column of its 1).  Forward:
+    tt_deconv_in on the folded pack (packing.pack_deconv_in_film).  Backward: ELU derivative; the tensor-core sums G = dz x z and the
+    row sums of dz (tt_conv_wgrad_lat); every parameter gradient from those in one launch (tt_film_convin_grad); latent gradient =
+    the Encoder.convlat forward kernel on W scaled by gamma.
+    """
+
+    @staticmethod
+    def forward(ctx, lat, weight, bias, gamma_w, gamma_b, beta_w, beta_b, run, hot, d, c0):
+        y = run(lat)
+        ctx.save_for_backward(lat, y, weight, gamma_w, gamma_b, beta_w, beta_b)
+        ctx.meta = (hot, d, c0)
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        lat, y, weight, gamma_w, gamma_b, beta_w, beta_b = ctx.saved_tensors
+        hot, d, c0 = ctx.meta
+        dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)
+        return _film_convin_grads(dz, lat, weight, gamma_w, gamma_b, beta_w, beta_b, hot, d, c0) + (None,) * 4
+
+
+def _film_convin_grads(dz, lat, weight, gamma_w, gamma_b, beta_w, beta_b, hot, d, c0):
+    """Gradients of _FiLMConvInFn from dz (C8 planar, after the ELU derivative) and the latents lat (C8 planar, H = 1):
+    (latents (bf16, C8), convin weight, convin bias, gamma.weight, gamma.bias, beta.weight, beta.bias)."""
+    h0 = dz.size(2)
+    dev = lat.device
+    G = torch.zeros(weight.shape, dtype=torch.float32, device=dev)
+    rows = torch.zeros((c0, h0), dtype=torch.float32, device=dev)
+    _wgrad_lat(dz, lat, c0, d, G, None, rows)
+    dw = torch.empty_like(G)
+    db = torch.empty(c0, dtype=torch.float32, device=dev)
+    dgw, dbw = torch.empty_like(gamma_w), torch.empty_like(beta_w)
+    dgb, dbb = torch.empty_like(gamma_b), torch.empty_like(beta_b)
+    _lib.check(_lib.lib().tt_film_convin_grad(_p(G), _p(rows), _p(weight), _p(gamma_w), _p(gamma_b), _p(beta_w), _p(beta_b), d, c0, h0, hot,
+                                              _p(dw), _p(db), _p(dgw), _p(dgb), _p(dbw), _p(dbb), _s(G)))
+    d_pad = lat.size(1) * 8
+
+    def build():
+        gamma = gamma_w.detach()[:, hot] + gamma_b.detach()                          # film_layer.gamma(one-hot cond)
+        return P.pack_lat(weight.detach().float() * gamma.view(-1, 1, 1, 1), d_pad), torch.zeros(d_pad, device=dev)
+    # gamma differs between the two passes and depends on the FiLM parameters, so they are part of the key
+    wl, zl = _bw_pack(weight, ('filmT', hot, gamma_w.data_ptr(), gamma_w._version, gamma_b.data_ptr(), gamma_b._version), build)
+    glat = ops.conv_lat(dz, wl, zl, d_pad)
+    return glat, dw, db, dgw, dgb, dbw, dbb
+
+
 def _decoder(dec, lat, reconstruct, skips=None):
     """skips: None or [(weight 0-dim tensor, embedding)] * 5 in encoder order (modules.py:568-589)"""
     ch = dec.channels
     w_in, tables, w_out, b_out = dec._packed()
     ci = dec.convin[0]
     sw = 1 if reconstruct else 0
-    x = _IndicatorFn.apply(lat, ci.weight, ci.bias, lambda t: ops.deconv_in(t, w_in[sw], tables[sw], P.pad8(ch[0]), dec.embedding_size),
-                           1.0 if reconstruct else 0.0, dec.latent_size, ch[0])
+
+    def run_in(t):
+        return ops.deconv_in(t, w_in[sw], tables[sw], P.pad8(ch[0]), dec.embedding_size)
+    film = dec._film
+    if film is None:
+        x = _IndicatorFn.apply(lat, ci.weight, ci.bias, run_in, 1.0 if reconstruct else 0.0, dec.latent_size, ch[0])
+    else:
+        # TimbreTrapFiLM.decode (modules.py:835-838): condition = one-hot [transcribe, not transcribe]
+        x = _FiLMConvInFn.apply(lat, ci.weight, ci.bias, film.gamma.weight, film.gamma.bias, film.beta.weight, film.beta.bias, run_in,
+                                1 if reconstruct else 0, dec.latent_size, ch[0])
     for i, blk in enumerate((dec.block1, dec.block2, dec.block3, dec.block4)):
         if skips is not None:
             x = _SkipAddFn.apply(x, skips[-1 - i][1], skips[-1 - i][0])
@@ -534,15 +660,18 @@ def allreduce_mean_gradients(params, group, flat=None):
 
 class TrainStep:
     """
-    One optimisation step of experiments/train.py:393-500 for TimbreTrap (with or without skip connections):
-    losses as in compute_step_losses, backward, optional NCCL all-reduce of one flat gradient bucket (mean over ranks),
-    clip_grad_norm_(max_norm) and AdamW (torch defaults: betas (0.9, 0.999), eps 1e-8, weight_decay 1e-2; train.py:334).
+    One optimisation step of experiments/train.py:393-500 for TimbreTrap, TimbreTrapFiLM, TimbreTrapMag or TimbreTrapMagDB (each with
+    or without skip connections): losses as in compute_step_losses, backward, optional NCCL all-reduce of one flat gradient bucket
+    (mean over ranks), clip_grad_norm_(max_norm) and AdamW (torch defaults: betas (0.9, 0.999), eps 1e-8, weight_decay 1e-2;
+    train.py:334).
+
+    The reconstruction target is the variant's own encoder input, `model._features(audio)`, without gradient: the CQT coefficients
+    for TimbreTrap and TimbreTrapFiLM, |c| for TimbreTrapMag and to_decibels(|c|) for TimbreTrapMagDB.  (The reference's loss step
+    takes its target from model.sliCQ(audio), train.py:404, whose two channels cannot be compared with the one-channel output of the
+    magnitude variants.)  Their one-channel tensors run as pairs (x, 0); the loss over such pairs is the one-channel loss.
     """
 
     def __init__(self, model, lr=1e-3, max_norm=10.0, multipliers=None, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2, group=None):
-        if getattr(model, 'HEAD_MODE', None) is not None or hasattr(model, 'film_layer'):
-            raise NotImplementedError('TrainStep covers TimbreTrap with or without skip connections (experiments/train.py:155-161); '
-                                      'the FiLM / magnitude variants run forward only')
         self.model = model
         self.params = [p for p in model.parameters()]
         self.lr, self.max_norm, self.betas, self.eps, self.wd = lr, max_norm, betas, eps, weight_decay
@@ -574,24 +703,30 @@ class TrainStep:
         """The four losses and their total, with the autograd graph attached."""
         model = self.model
         with torch.no_grad():
-            coeffs = model.sliCQ.encode_interleaved(audio)
+            coeffs = model._features(audio)                                     # the reconstruction target (see the class docstring)
+        head = model.HEAD_MODE
+
         def skips_of(emb):
             if model.skip_weights is None:
                 return None
             return [(model.skip_weights[i], e) for i, e in enumerate(emb)]
+
+        def decode(lat, reconstruct, sk):
+            y = _decoder(model.decoder, lat, reconstruct, sk)
+            return y if head is None else _HeadFn.apply(y, head)
         lat, emb = _encoder(model.encoder, coeffs)
         sk = skips_of(emb)
-        rec = _decoder(model.decoder, lat, True, sk)
-        trn = _decoder(model.decoder, lat, False, sk)
-        act = _ActivationsFn.apply(trn)
+        rec = decode(lat, True, sk)
+        trn = decode(lat, False, sk)
+        act = _ActivationsFn.apply(trn) if head is None else _Channel0ActivationsFn.apply(trn, _ACTIVATIONS_MODE[head])
         n = ground_truth.size(0)
         out = dict(reconstruction=_SqDiffFn.apply(rec, coeffs), transcription=_TrnLossFn.apply(act[:n].contiguous(), ground_truth.float().contiguous()))
         total = self.mult['reconstruction'] * out['reconstruction']
         if self.mult['consistency']:
             lat_t, emb_t = _encoder(model.encoder, trn)
             sk_t = skips_of(emb_t)
-            trn_rec = _decoder(model.decoder, lat_t, True, sk_t)
-            trn_scr = _decoder(model.decoder, lat_t, False, sk_t)
+            trn_rec = decode(lat_t, True, sk_t)
+            trn_scr = decode(lat_t, False, sk_t)
             tgt = trn[:n].contiguous()
             out['consistency_spectral'] = _SqDiffFn.apply(trn_rec[:n].contiguous(), tgt)
             out['consistency_score'] = _SqDiffFn.apply(trn_scr[:n].contiguous(), tgt)
