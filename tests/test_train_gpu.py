@@ -113,7 +113,7 @@ def test_tensor_core_weight_gradient(C, H, T, k, d, B):
     """tt_conv_wgrad_same (MN-major tcgen05 GEMM over the pixel axis, deterministic two-stage reduction) against torch autograd on the
     same bf16-rounded operands; products of bf16 values are exact in fp32, so only the summation order differs."""
     import torch.nn.functional as F
-    from timbre_trap_b200.framework import packing as P, train as TR
+    from timbre_trap_b200.framework import layer_grads as LG, packing as P
     g = torch.Generator().manual_seed(C * 100 + H)
     x = torch.randn((B, C, H, T), generator=g).to(torch.bfloat16).float()
     dz = (torch.randn((B, C, H, T), generator=g) * 0.1).to(torch.bfloat16).float()
@@ -122,12 +122,12 @@ def test_tensor_core_weight_gradient(C, H, T, k, d, B):
     pad = d if k == 3 else 0
     y = F.conv2d(x, w, bias, padding=pad, dilation=d if k == 3 else 1)
     (y * dz).sum().backward()
-    dw, db = TR._wgrad_same(P.to_c8(x.cuda()), P.to_c8(dz.cuda()), C, C, k, d)
+    dw, db = LG._wgrad_same(P.to_c8(x.cuda()), P.to_c8(dz.cuda()), C, C, k, d)
     assert dw.shape == w.grad.shape
     scale = float(w.grad.abs().max())
     assert float((dw.cpu() - w.grad).abs().max()) <= 2e-4 * scale + 1e-4, (float((dw.cpu() - w.grad).abs().max()), scale)
     assert float((db.cpu() - bias.grad).abs().max()) <= 2e-4 * float(bias.grad.abs().max()) + 1e-4
-    dw2, db2 = TR._wgrad_same(P.to_c8(x.cuda()), P.to_c8(dz.cuda()), C, C, k, d)
+    dw2, db2 = LG._wgrad_same(P.to_c8(x.cuda()), P.to_c8(dz.cuda()), C, C, k, d)
     assert torch.equal(dw, dw2) and torch.equal(db, db2)                  # fixed reduction order: bit-reproducible
 
 
@@ -135,7 +135,7 @@ def test_tensor_core_weight_gradient(C, H, T, k, d, B):
 def test_tensor_core_weight_gradient_strided_and_transposed(Cf, Cc, Hc, T, op, B):
     """tt_conv_wgrad_updown against torch autograd: EncoderBlock.sconv (fine = input, coarse = output gradient) and DecoderBlock.tconv
     (coarse = input, fine = output gradient, bias gradient = pixel sums of the fine tensor)."""
-    from timbre_trap_b200.framework import packing as P, train as TR
+    from timbre_trap_b200.framework import layer_grads as LG, packing as P
     g = torch.Generator().manual_seed(Cf * 10 + Hc)
     Hf = 2 * Hc + 2 + op
     fine = torch.randn((B, Cf, Hf, T), generator=g).to(torch.bfloat16).float()
@@ -146,7 +146,7 @@ def test_tensor_core_weight_gradient_strided_and_transposed(Cf, Cc, Hc, T, op, B
     y = F.conv2d(fine, w, bias, stride=(2, 1))
     assert y.shape[2] == Hc
     (y * coarse).sum().backward()
-    dw, db = TR._wgrad_updown(P.to_c8(fine.cuda()), P.to_c8(coarse.cuda()), Cf, Cc, False)
+    dw, db = LG._wgrad_updown(P.to_c8(fine.cuda()), P.to_c8(coarse.cuda()), Cf, Cc, False)
     assert float((dw.cpu() - w.grad).abs().max()) <= 2e-4 * float(w.grad.abs().max()) + 1e-4
     assert float((db.cpu() - bias.grad).abs().max()) <= 2e-4 * float(bias.grad.abs().max()) + 1e-4
     # transposed conv: y = convT(coarse, wt (Cc, Cf, 4, 1), stride 2, output_padding op) has Hf rows; fine plays dL/dy
@@ -155,7 +155,7 @@ def test_tensor_core_weight_gradient_strided_and_transposed(Cf, Cc, Hc, T, op, B
     yt = F.conv_transpose2d(coarse, wt, bt, stride=(2, 1), output_padding=(op, 0))
     assert yt.shape[2] == Hf
     (yt * fine).sum().backward()
-    dwt, dbt = TR._wgrad_updown(P.to_c8(fine.cuda()), P.to_c8(coarse.cuda()), Cf, Cc, True)
+    dwt, dbt = LG._wgrad_updown(P.to_c8(fine.cuda()), P.to_c8(coarse.cuda()), Cf, Cc, True)
     assert float((dwt.cpu() - wt.grad).abs().max()) <= 2e-4 * float(wt.grad.abs().max()) + 1e-4
     assert float((dbt.cpu() - bt.grad).abs().max()) <= 2e-4 * float(bt.grad.abs().max()) + 2e-3
 
@@ -164,12 +164,12 @@ def test_tensor_core_weight_gradient_strided_and_transposed(Cf, Cc, Hc, T, op, B
 def test_tensor_core_weight_gradient_tall_kernel_layers(Ct, Cf, H, T, B):
     """tt_conv_wgrad_lat against torch autograd: Encoder.convlat (Conv2d (Cf, Ct, H, 1) over the full height) and Decoder.convin
     (ConvTranspose2d (Cf + 1, Ct, H, 1) with the indicator channel: its weight row and the bias are row sums of the output gradient)."""
-    from timbre_trap_b200.framework import packing as P, train as TR
+    from timbre_trap_b200.framework import layer_grads as LG, packing as P
     g = torch.Generator().manual_seed(Ct + H)
     tall = torch.randn((B, Ct, H, T), generator=g).to(torch.bfloat16).float()
     flat = (torch.randn((B, Cf, 1, T), generator=g) * 0.1).to(torch.bfloat16).float()
     fpad = (Cf + 15) // 16 * 16
-    flat8 = TR.P.to_c8(torch.nn.functional.pad(flat, (0, 0, 0, 0, 0, fpad - Cf)).cuda())
+    flat8 = P.to_c8(torch.nn.functional.pad(flat, (0, 0, 0, 0, 0, fpad - Cf)).cuda())
     tall8 = P.to_c8(tall.cuda())
     # convlat: y = conv(tall, w (Cf, Ct, H, 1)); flat plays dL/dy
     w = torch.zeros((Cf, Ct, H, 1), requires_grad=True)
@@ -177,7 +177,7 @@ def test_tensor_core_weight_gradient_tall_kernel_layers(Ct, Cf, H, T, B):
     (F.conv2d(tall, w, bias) * flat).sum().backward()
     dw = torch.zeros((Cf, Ct, H, 1), device='cuda')
     db = torch.zeros(Cf, device='cuda')
-    TR._wgrad_lat(tall8, flat8, Ct, Cf, dw, db, None)
+    LG._wgrad_lat(tall8, flat8, Ct, Cf, dw, db, None)
     assert float((dw.cpu() - w.grad).abs().max()) <= 2e-4 * float(w.grad.abs().max()) + 1e-4
     assert float((db.cpu() - bias.grad).abs().max()) <= 2e-4 * float(bias.grad.abs().max()) + 1e-4
     # decoder convin: y = convT(cat(flat, indicator), wt (Cf + 1, Ct, H, 1)); tall plays dL/dy
@@ -187,7 +187,7 @@ def test_tensor_core_weight_gradient_tall_kernel_layers(Ct, Cf, H, T, B):
     (F.conv_transpose2d(full, wt, bt) * tall).sum().backward()
     dwt = torch.zeros((Cf + 1, Ct, H, 1), device='cuda')
     rows = torch.zeros((Ct, H), device='cuda')
-    TR._wgrad_lat(tall8, flat8, Ct, Cf, dwt, None, rows)
+    LG._wgrad_lat(tall8, flat8, Ct, Cf, dwt, None, rows)
     dwt[Cf, :, :, 0] = rows
     assert float((dwt.cpu() - wt.grad).abs().max()) <= 2e-4 * float(wt.grad.abs().max()) + 2e-3
     assert float((rows.sum(1).cpu() - bt.grad).abs().max()) <= 2e-4 * float(bt.grad.abs().max()) + 2e-3

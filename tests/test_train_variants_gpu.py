@@ -1,8 +1,9 @@
 """
 GPU parity of the loss step for the model variants TimbreTrapFiLM, TimbreTrapMag and TimbreTrapMagDB (reference modules.py:780-1075):
 whole-step parameter gradients against the CPU oracle's fp32 autograd (same gates as tests/test_train_gpu.py), the two kernels of their
-edges (tt_film_convin_grad, tt_channel0_activation_bwd) against torch autograd, compute_step_losses against the oracle, and a short
-training run per variant.  The reconstruction target of a variant is its own encoder input (oracle features_ref).
+edges (tt_film_convin_grad, tt_channel0_activation_bwd) against torch autograd, compute_step_losses against the oracle and (for the
+base model too) against TrainStep.losses, and a short training run per variant.  The reconstruction target of a variant is its own
+encoder input (oracle features_ref).
 """
 import contextlib
 
@@ -16,7 +17,7 @@ from tests.helpers import tonal_clip
 pytestmark = pytest.mark.gpu
 
 SMALL = dict(sample_rate=8000, n_octaves=6, bins_per_octave=12, secs_per_block=0.5)
-CLASSES = dict(film='TimbreTrapFiLM', mag='TimbreTrapMag', magdb='TimbreTrapMagDB')
+CLASSES = dict(base='TimbreTrap', film='TimbreTrapFiLM', mag='TimbreTrapMag', magdb='TimbreTrapMagDB')
 
 
 def _setup(tag, skip=False, latent=None):
@@ -133,8 +134,8 @@ def test_film_convin_gradients_match_autograd(D, C0, H, T, B, hot):
     conv_transpose2d(film(z)) on the same bf16-rounded z and output gradient, for both conditions.  The weight / bias / Linear gradients
     are fp32 (gate 2e-4 max, as the weight-gradient kernels); the latent gradient is a bf16 tensor computed from the bf16-rounded W * gamma,
     so its reference uses that rounded weight and its gate adds one bf16 rounding of the result (2^-8 relative)."""
-    from timbre_trap_b200.framework import packing as P, train as TR
-    from timbre_trap_b200.framework.modules import _PackedCache, _latent_pad
+    from timbre_trap_b200.framework import layer_grads as LG, packing as P
+    from timbre_trap_b200.framework.modules import _latent_pad
     z, dz, w, film = _film_operands(D, C0, H, T, B, seed=D + hot)
     cond = torch.tensor([1.0 - hot, float(hot)])                        # one-hot [transcribe, not transcribe]
     wt, bt = w.clone().requires_grad_(True), torch.zeros(C0, requires_grad=True)
@@ -147,10 +148,10 @@ def test_film_convin_gradients_match_autograd(D, C0, H, T, B, hot):
     d_pad = _latent_pad(D)
     lat8 = P.to_c8(F.pad(z, (0, 0, 0, d_pad - D)).unsqueeze(2).cuda())
     dz8 = P.to_c8(dz.cuda())
-    _PackedCache.epoch += 1                                             # fresh backward packs for these tensors
+    P._PackedCache.epoch += 1                                           # fresh backward packs for these tensors
     args = (dz8, lat8, w.cuda(), *[f.cuda() for f in film], hot, D, C0)
-    first = TR._film_convin_grads(*args)
-    again = TR._film_convin_grads(*args)
+    first = LG._film_convin_grads(*args)
+    again = LG._film_convin_grads(*args)
     assert all(torch.equal(a, b) for a, b in zip(first, again))        # fixed reduction order: bit-reproducible
     glat, dw, db, dgw, dgb, dbw, dbb = first
     for name, got, want in (('dW', dw, wt.grad), ('db', db, bt.grad), ('gamma.weight', dgw, ft[0].grad), ('gamma.bias', dgb, ft[1].grad),
@@ -172,7 +173,7 @@ def test_film_convin_gradients_match_autograd(D, C0, H, T, B, hot):
 @pytest.mark.parametrize('mode', [0, 1, 2, 3])
 def test_channel0_activation_bwd_matches_autograd(mode):
     from timbre_trap_b200 import _lib
-    from timbre_trap_b200.framework import train as TR
+    from timbre_trap_b200.framework import layer_grads as LG
     g = torch.Generator().manual_seed(mode)
     pairs = torch.randn((2, 37, 129, 2), generator=g)
     pairs[0, :5, :, 0] = 0.0                                            # exact zeros: relu'(0) = 0
@@ -180,11 +181,11 @@ def test_channel0_activation_bwd_matches_autograd(mode):
     v = pairs[..., 0].clone().requires_grad_(True)
     f = {0: lambda x: x, 1: torch.relu, 2: torch.sigmoid, 3: lambda x: torch.tanh(torch.relu(x))}[mode]
     (f(v) * gout[..., 0]).sum().backward()
-    got = TR._channel0_bwd(pairs.cuda(), gout.cuda(), mode).cpu()
+    got = LG._channel0_bwd(pairs.cuda(), gout.cuda(), mode).cpu()
     assert torch.equal(got[..., 1], torch.zeros_like(got[..., 1]))
     np.testing.assert_allclose(got[..., 0].numpy(), v.grad.numpy(), rtol=1e-5, atol=1e-6)
     with pytest.raises(_lib.TimbreTrapB200Error):
-        TR._channel0_bwd(pairs.cuda(), gout.cuda(), 4)
+        LG._channel0_bwd(pairs.cuda(), gout.cuda(), 4)
 
 
 @pytest.mark.parametrize('tag,skip,latent', CASES)
@@ -202,6 +203,21 @@ def test_variant_step_losses_match_oracle(tag, skip, latent):
     for k, v in want.items():
         print(tag, k, float(got[k]), float(v))
         np.testing.assert_allclose(float(got[k]), float(v), rtol=3e-2, atol=(1.5e-2) ** 2 * energy, err_msg=k)
+
+
+@pytest.mark.parametrize('tag,skip,latent', [('base', False, None), ('base', True, None), ('film', True, 24), ('mag', False, None),
+                                             ('magdb', True, None)])
+def test_step_losses_equal_train_step_losses(tag, skip, latent):
+    """compute_step_losses runs the model's inference layers, TrainStep.losses the same layers through their autograd Functions: the
+    same kernels in the same order (the residual blocks' tt_res_block_rs_mid only stores the inner tile tt_res_block_rs stages), so
+    every loss agrees bit for bit."""
+    from timbre_trap_b200.framework.train import TrainStep, compute_step_losses
+    R, model, sd, c, audio, gt = _setup(tag, skip, latent)
+    want = compute_step_losses(model, audio.cuda(), gt.cuda())
+    got = {k: v.detach() for k, v in TrainStep(model).losses(audio.cuda(), gt.cuda()).items()}
+    assert list(got) == list(want)
+    for k in want:
+        assert torch.equal(got[k], want[k]), (k, float(got[k]), float(want[k]))
 
 
 def _oracle_training(R, tag, sd, c, audio, gt, steps, lr):

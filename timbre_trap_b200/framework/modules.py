@@ -19,32 +19,11 @@ from .. import _lib
 from . import ops
 from . import packing as P
 from .cqt import CQT
+from .layer_grads import _DownFn, _FiLMConvInFn, _HeadFn, _IndicatorFn, _InFn, _LatFn, _OutFn, _ResFn, _SkipAddFn, _UpFn
+from .packing import _PackedCache       # also the name under which pickled modules refer to it
 
 __all__ = ['TimbreTrap', 'TimbreTrapFiLM', 'FiLM', 'TimbreTrapMag', 'TimbreTrapMagDB', 'Encoder', 'Decoder', 'EncoderBlock', 'DecoderBlock',
            'ResidualConv2dBlock', 'shard_block_range', 'shard_audio']
-
-
-class _PackedCache:
-    """Packed (kernel-layout) copies of a module's parameters, rebuilt when a parameter is modified or moved."""
-
-    epoch = 0       # bumped by code that updates parameters outside torch's version counter (framework/train.py's AdamW kernel)
-
-    def __init__(self):
-        self._key = None
-        self._val = None
-
-    def __getstate__(self):
-        # pickling / deep-copying a module (the reference checkpoints whole modules, experiments/train.py:511) drops the packed
-        # copies: they are rebuilt lazily from the parameters of the new object
-        return dict(_key=None, _val=None)
-
-    def get(self, params, build):
-        key = (_PackedCache.epoch,) + tuple((p.data_ptr(), p._version, p.device) for p in params)
-        if key != self._key:
-            with torch.no_grad():
-                self._val = build()
-            self._key = key
-        return self._val
 
 
 def _n16(c):
@@ -76,7 +55,14 @@ class ResidualConv2dBlock(nn.Module):
                  'planar': lambda: P.pack_res_rs(*args)}[mode]
         return self._caches.setdefault(mode, _PackedCache()).get(args, build)
 
-    def forward_c8(self, x, out=None, mid_out=None):
+    def forward_c8(self, x, out=None, mid_out=None, grad=False):
+        """`grad`: through _ResFn (framework/layer_grads.py), whose forward is this call with `mid_out`; `out` is inference only."""
+        if grad:
+            if out is not None:
+                raise ValueError('out= is for inference only')
+            c1, c2 = self.conv1[0], self.conv2[0]
+            return _ResFn.apply(x, c1.weight, c1.bias, c2.weight, c2.bias, lambda t, mid: self.forward_c8(t, mid_out=mid), self.channels,
+                                self.dilation)
         # rows of C <= 8 tensors are folded to 16 values (4 or 2 frames per GEMM row) when T allows
         T = x.size(-2)
         if self.packed4:
@@ -118,14 +104,18 @@ class EncoderBlock(nn.Module):
         for blk in (self.block1, self.block2, self.block3):
             blk.packed4 = flag
 
-    def forward_c8(self, x):
-        a = self.block1.forward_c8(x)
-        b = self.block2.forward_c8(a)
-        a = self.block3.forward_c8(b, out=a)
+    def forward_c8(self, x, grad=False):
+        """`grad`: every layer through its autograd Function, and no buffer reused (the Functions keep their tensors for the backward)."""
+        a = self.block1.forward_c8(x, grad=grad)
+        b = self.block2.forward_c8(a, grad=grad)
+        a = self.block3.forward_c8(b, out=None if grad else a, grad=grad)
         c = self.sconv[0]
         pack = P.pack_down_pairs if self.packed4 else P.pack_down_strip
-        (w,) = self._cache.get((c.weight, c.bias), lambda: (pack(c.weight, c.bias),))
-        return ops.conv_down_strip(a, w, P.pad8(self.out_channels))
+
+        def run(t):
+            (w,) = self._cache.get((c.weight, c.bias), lambda: (pack(c.weight, c.bias),))
+            return ops.conv_down_strip(t, w, P.pad8(self.out_channels))
+        return _DownFn.apply(a, c.weight, c.bias, run, self.in_channels, self.out_channels) if grad else run(a)
 
     def forward(self, x):
         return P.from_c8(self.forward_c8(P.to_p4(x) if self.packed4 else P.to_c8(x)), self.out_channels)
@@ -157,14 +147,20 @@ class DecoderBlock(nn.Module):
         for blk in (self.block1, self.block2, self.block3):
             blk.packed4 = flag
 
-    def forward_c8(self, x, out=None):
-        """`out`: where the stage's result goes (e.g. a slice of the all-chunks buffer the fused convout / cross-fade reads)."""
+    def forward_c8(self, x, out=None, grad=False):
+        """`out`: where the stage's result goes (e.g. a slice of the all-chunks buffer the fused convout / cross-fade reads), inference
+        only.  `grad`: every layer through its autograd Function, and no buffer reused."""
+        if grad and out is not None:
+            raise ValueError('out= is for inference only')
         c = self.tconv[0]
-        (w,) = self._cache.get((c.weight, c.bias), lambda: (P.pack_up_strip(c.weight, c.bias),))
-        a = ops.conv_up_strip(x, w, P.pad8(self.out_channels), self.out_pad, packed4_out=self.packed4)
-        b = self.block1.forward_c8(a)
-        a = self.block2.forward_c8(b, out=a)
-        return self.block3.forward_c8(a, out=b if out is None else out)
+
+        def run(t):
+            (w,) = self._cache.get((c.weight, c.bias), lambda: (P.pack_up_strip(c.weight, c.bias),))
+            return ops.conv_up_strip(t, w, P.pad8(self.out_channels), self.out_pad, packed4_out=self.packed4)
+        a = _UpFn.apply(x, c.weight, c.bias, run, c.in_channels, c.out_channels) if grad else run(x)
+        b = self.block1.forward_c8(a, grad=grad)
+        a = self.block2.forward_c8(b, out=None if grad else a, grad=grad)
+        return self.block3.forward_c8(a, out=None if grad else (b if out is None else out), grad=grad)
 
     def forward(self, x):
         y = self.forward_c8(P.to_c8(x))
@@ -220,13 +216,23 @@ class Encoder(nn.Module):
             return w.contiguous(), ci.bias.detach().float().contiguous(), P.pack_lat(cl.weight, self.latent_pad), P.pad_vec(cl.bias, self.latent_pad)
         return self._cache.get((ci.weight, ci.bias, cl.weight, cl.bias), build)
 
-    def forward_c8(self, coeffs_bft2):
-        """coeffs (B, F, T, 2) fp32 interleaved -> (latents C8 (B, Dp/8, 1, T, 8), [5 embeddings C8])."""
+    def forward_c8(self, coeffs_bft2, grad=False):
+        """coeffs (B, F, T, 2) fp32 interleaved -> (latents C8 (B, Dp/8, 1, T, 8), [5 embeddings C8]).  `grad`: every layer through
+        its autograd Function."""
         w_in, b_in, w_lat, b_lat = self._packed()
-        emb = [ops.conv_in(coeffs_bft2, w_in, b_in, self.channels[0], packed4=self.packed4)]
+        ci, cl, ch = self.convin[0], self.convlat, self.channels
+
+        def run_in(t):
+            return ops.conv_in(t, w_in, b_in, ch[0], packed4=self.packed4)
+
+        def run_lat(t):
+            return ops.conv_lat(t, w_lat, b_lat, self.latent_pad)
+        emb = [_InFn.apply(coeffs_bft2, ci.weight, ci.bias, run_in, ch[0]) if grad else run_in(coeffs_bft2)]
         for blk in (self.block1, self.block2, self.block3, self.block4):
-            emb.append(blk.forward_c8(emb[-1]))
-        return ops.conv_lat(emb[-1], w_lat, b_lat, self.latent_pad), emb
+            emb.append(blk.forward_c8(emb[-1], grad=grad))
+        if grad:
+            return _LatFn.apply(emb[-1], cl.weight, cl.bias, run_lat, ch[4], self.latent_size, self.latent_pad), emb
+        return run_lat(emb[-1]), emb
 
     def forward(self, coefficients):
         """Encoder.forward (modules.py:448-483): (B, 2, F, T) -> (latents (B, D, T), embeddings, {}); (B, 1, F, T) for the
@@ -304,27 +310,49 @@ class Decoder(nn.Module):
             return tuple(ws), tuple(tables), w_out.contiguous(), b_out.contiguous()
         return self._cache.get(params, build)
 
-    def last_stage_c8(self, lat_c8, reconstruct, skips=None, out=None, convin=None):
+    def last_stage_c8(self, lat_c8, reconstruct, skips=None, out=None, convin=None, grad=False):
         """Everything before `convout`: latents C8 (B, Dp/8, 1, T, 8) (without the indicator channel) -> the last stage's
-        activations in their internal layout (packed4 (B, F, T, 4) for the supported channel plans), written to `out` if given."""
+        activations in their internal layout (packed4 (B, F, T, 4) for the supported channel plans), written to `out` if given.
+        `grad`: every layer through its autograd Function, and no buffer reused; `out` and `convin` are inference only."""
+        if grad and (out is not None or convin is not None):
+            raise ValueError('out= and convin= are for inference only')
         w_in, tables, _, _ = self._packed()
         sw = 1 if reconstruct else 0
         w_sel, t_sel = (w_in[sw], tables[sw]) if convin is None else convin
-        x = ops.deconv_in(lat_c8, w_sel, t_sel, P.pad8(self.channels[0]), self.embedding_size)
+        ci, film = self.convin[0], self._film
+
+        def run_in(t):
+            return ops.deconv_in(t, w_sel, t_sel, P.pad8(self.channels[0]), self.embedding_size)
+        if not grad:
+            x = run_in(lat_c8)
+        elif film is None:
+            x = _IndicatorFn.apply(lat_c8, ci.weight, ci.bias, run_in, 1.0 if reconstruct else 0.0, self.latent_size, self.channels[0])
+        else:
+            # TimbreTrapFiLM.decode (modules.py:835-838): condition = one-hot [transcribe, not transcribe]
+            x = _FiLMConvInFn.apply(lat_c8, ci.weight, ci.bias, film.gamma.weight, film.gamma.bias, film.beta.weight, film.beta.bias, run_in,
+                                    1 if reconstruct else 0, self.latent_size, self.channels[0])
         blocks = (self.block1, self.block2, self.block3, self.block4)
         for i, blk in enumerate(blocks):
-            if skips is not None:                      # modules.py:568-585: x + weight * encoder embedding, one native pass, in place
-                x = _add_scaled(x, skips[-1 - i][1], skips[-1 - i][0], out=x)
+            if skips is not None:                      # modules.py:568-585: x + weight * encoder embedding, one native pass (in place)
+                w, e = skips[-1 - i]
+                x = _SkipAddFn.apply(x, e, w) if grad else ops.add_scaled(x, e, w, out=x)
             last = i == len(blocks) - 1
-            x = blk.forward_c8(x, out=out if (last and skips is None) else None)
+            x = blk.forward_c8(x, out=out if (last and skips is None) else None, grad=grad)
         if skips is not None:
-            x = _add_scaled(x, skips[0][1], skips[0][0], out=out if out is not None else x)
+            w, e = skips[0]
+            x = _SkipAddFn.apply(x, e, w) if grad else ops.add_scaled(x, e, w, out=out if out is not None else x)
         return x
 
-    def forward_c8(self, lat_c8, reconstruct, skips=None, convin=None):
-        """latents C8 (B, Dp/8, 1, T, 8) (without the indicator channel) -> coefficients (B, F, T, 2) fp32 interleaved."""
+    def forward_c8(self, lat_c8, reconstruct, skips=None, convin=None, grad=False):
+        """latents C8 (B, Dp/8, 1, T, 8) (without the indicator channel) -> coefficients (B, F, T, 2) fp32 interleaved.  `grad`: every
+        layer through its autograd Function; `convin` is inference only."""
         _, _, w_out, b_out = self._packed()
-        return ops.conv_out(self.last_stage_c8(lat_c8, reconstruct, skips, convin=convin), w_out, b_out, self.channels[4])
+        x = self.last_stage_c8(lat_c8, reconstruct, skips, convin=convin, grad=grad)
+        co, c = self.convout, self.channels[4]
+
+        def run_out(t):
+            return ops.conv_out(t, w_out, b_out, c)
+        return _OutFn.apply(x, co.weight, co.bias, run_out, c) if grad else run_out(x)
 
     def forward(self, latents, encoder_embeddings=None):
         """Decoder.forward (modules.py:545-594): latents (B, D+1, T) WITH the indicator channel -> (B, 2, F, T)."""
@@ -352,44 +380,11 @@ class Decoder(nn.Module):
             return pairs.permute(0, 3, 1, 2) if self.convout.out_channels == 2 else pairs[..., :1].permute(0, 3, 1, 2)
 
 
-def _widen(x):
-    """(B, F, T) fp32 -> interleaved (B, F, T, 2) pairs (x, 0) (tt_widen_pairs)."""
-    x = x.detach().float().contiguous()
-    out = torch.empty(tuple(x.shape) + (2,), dtype=torch.float32, device=x.device)
-    if x.numel():
-        with torch.cuda.device(x.device):
-            _lib.check(_lib.lib().tt_widen_pairs(ctypes.c_void_p(x.data_ptr()), x.numel(), ctypes.c_void_p(out.data_ptr()),
-                                                 ctypes.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)))
-    return out
-
-
-def _channel0(pairs, mode):
-    """interleaved (B, F, T, 2) -> (B, F, T): channel 0 through a non-linearity (tt_channel0_activation modes)."""
-    out = torch.empty(pairs.shape[:-1], dtype=torch.float32, device=pairs.device)
-    if out.numel():
-        with torch.cuda.device(pairs.device):
-            _lib.check(_lib.lib().tt_channel0_activation(ctypes.c_void_p(pairs.data_ptr()), out.numel(), mode, ctypes.c_void_p(out.data_ptr()),
-                                                         ctypes.c_void_p(torch.cuda.current_stream(pairs.device).cuda_stream)))
-    return out
-
-
-def _add_scaled(x, e, scale, out=None):
-    """x + scale * e on two bf16 tensors of one layout, one pass (tt_add_scaled_bf16); scale is a 0-dim device tensor."""
-    if x.shape != e.shape or x.dtype != torch.bfloat16 or e.dtype != torch.bfloat16:
-        raise ValueError(f'skip connection: {tuple(x.shape)} {x.dtype} vs {tuple(e.shape)} {e.dtype}')
-    out = torch.empty_like(x) if out is None else out
-    s = scale.detach().float().reshape(1)
-    with torch.cuda.device(x.device):
-        _lib.check(_lib.lib().tt_add_scaled_bf16(ctypes.c_void_p(x.data_ptr()), ctypes.c_void_p(e.contiguous().data_ptr()), ctypes.c_void_p(s.data_ptr()),
-                                                 ctypes.c_void_p(out.data_ptr()), x.numel(), ctypes.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)))
-    return out
-
-
 def _interleave(coefficients):
     """(B, 2, F, T) real (any strides) -> contiguous (B, F, T, 2) fp32 (free for the CQT's own output); a one-channel feature map
     (B, 1, F, T) becomes pairs (x, 0)."""
     if coefficients.size(1) == 1:
-        return _widen(coefficients[:, 0])
+        return ops.widen(coefficients[:, 0])
     c = coefficients.detach().permute(0, 2, 3, 1)
     if c.dtype != torch.float32:
         c = c.float()
@@ -502,19 +497,42 @@ class TimbreTrap(nn.Module):
         """audio (B, 1, n*L) -> the encoder's input as interleaved (B, F, T, 2) fp32: the CQT coefficients (modules.py:88)."""
         return self.sliCQ.encode_interleaved(audio)
 
-    # output head of the variant (tt_channel0_activation mode; None = the two-channel coefficients as they are)
+    # output head of the variant (tt_channel0_activation mode; None = the two-channel coefficients as they are), and the mode of its
+    # to_activations on the head's output (None = tanh|.| of the two-channel coefficients)
     HEAD_MODE = None
+    ACTIVATIONS_MODE = None
 
     def _head(self, pairs):
         """decoder output (B, F, T, 2) interleaved -> what `decode` returns: (B, 2, F, T) view, or (B, 1, F, T) for the magnitude variants."""
         if self.HEAD_MODE is None:
             return pairs.permute(0, 3, 1, 2)
-        return _channel0(pairs, self.HEAD_MODE).unsqueeze(1)
+        return ops.channel0(pairs, self.HEAD_MODE).unsqueeze(1)
 
     def _codes(self, audio):
         """audio (B, 1, n*L) -> (latents C8, skips C8 or None)."""
         lat, emb = self.encoder.forward_c8(self._features(audio))
         return lat, self._skips_c8(emb)
+
+    def _passes(self, features, grad=False):
+        """Encode the encoder input (B, F, T, 2), decode for the reconstruction and for the transcription (modules.py:338-393) ->
+        (reconstruction, transcription, latents C8); the decoder outputs are pairs (B, F, T, 2) after the variant's head, a one-channel
+        output h as (h, 0).  The consistency pass is this method again on the transcription.  `grad`: every layer through its autograd
+        Function (framework/layer_grads.py), as the loss step runs it."""
+        lat, emb = self.encoder.forward_c8(features, grad=grad)
+        skips = self._skips_c8(emb)
+        outs = []
+        for reconstruct in (True, False):
+            y = self.decoder.forward_c8(lat, reconstruct, skips, grad=grad)
+            if self.HEAD_MODE is not None:
+                y = _HeadFn.apply(y, self.HEAD_MODE) if grad else ops.widen(ops.channel0(y, self.HEAD_MODE))
+            outs.append(y)
+        return outs[0], outs[1], lat
+
+    def _output(self, pairs):
+        """A decoder output of _passes -> what `forward` returns: (B, 2, F, T) view, or (B, 1, F, T) for the magnitude variants."""
+        if self.HEAD_MODE is None:
+            return pairs.permute(0, 3, 1, 2)
+        return ops.channel0(pairs, 0).unsqueeze(1)          # mode 0: channel 0 as it is
 
     # ---- reference API -------------------------------------------------------------------------------
     def encode(self, audio):
@@ -614,7 +632,7 @@ class TimbreTrap(nn.Module):
                         if self.HEAD_MODE is not None:
                             # the reference's loop adds the variant's ONE output channel into its hard-coded two-channel buffer
                             # (modules.py:244, 259-263): broadcast, i.e. both channels carry the head's output
-                            y = _channel0(y, self.HEAD_MODE).unsqueeze(-1).expand(-1, -1, -1, 2)
+                            y = ops.channel0(y, self.HEAD_MODE).unsqueeze(-1).expand(-1, -1, -1, 2)
                         stage[c0:c0 + step] = y
                 if early:
                     done = min(B, (c0 + step) // n_chunks)            # clips whose chunks have all been decoded
@@ -765,19 +783,15 @@ class TimbreTrap(nn.Module):
         return _gather_frames(act, -1, M, audio, L, group, world), _gather_frames(wav, -1, L, audio, L, group, world)
 
     def forward(self, audio, consistency=False):
-        """modules.py:338-393 (inference semantics; the training step with gradients is framework.train_step)."""
+        """modules.py:338-393 (inference semantics; the training step with gradients is framework.train.TrainStep)."""
         with torch.no_grad():
-            lat, skips = self._codes(audio)
-            reconstruction = self._head(self.decoder.forward_c8(lat, True, skips))
-            transcription = self._head(self.decoder.forward_c8(lat, False, skips))
-            transcription_rec = transcription_scr = None
+            rec, trn, lat = self._passes(self._features(audio))
+            trn_rec = trn_scr = None
             if consistency:
-                lat_t, emb_t = self.encoder.forward_c8(_interleave(transcription))
-                skips_t = self._skips_c8(emb_t)
-                transcription_rec = self._head(self.decoder.forward_c8(lat_t, True, skips_t))
-                transcription_scr = self._head(self.decoder.forward_c8(lat_t, False, skips_t))
+                trn_rec, trn_scr, _ = self._passes(trn)
+                trn_rec, trn_scr = self._output(trn_rec), self._output(trn_scr)
             latents = P.from_c8(lat, self.encoder.latent_size).squeeze(-2)
-        return reconstruction, latents, transcription, transcription_rec, transcription_scr, dict()
+            return self._output(rec), latents, self._output(trn), trn_rec, trn_scr, dict()
 
     # ---- full-track forward in time tiles (experiments/evaluate.py:81-95 feeds whole tracks through model(audio)) -------------------
     # Only the convolutions see across frames, and only +-1 frame (convin / convout) and +-6 frames per block of three dilated
@@ -804,18 +818,11 @@ class TimbreTrap(nn.Module):
                 t1 = min(T, t0 + tile_frames)
                 a, b = max(0, t0 - h), min(T, t1 + h)
                 keep = slice(t0 - a, t0 - a + (t1 - t0))
-                lat, emb = self.encoder.forward_c8(feats[:, :, a:b].contiguous())
-                skips = self._skips_c8(emb)
-                rec = self._head(self.decoder.forward_c8(lat, True, skips))
-                trn = self._head(self.decoder.forward_c8(lat, False, skips))
-                outs[0][..., t0:t1] = rec[..., keep]
-                outs[1][..., t0:t1] = trn[..., keep]
+                rec, trn, lat = self._passes(feats[:, :, a:b].contiguous())
+                tile = [rec, trn] + (list(self._passes(trn)[:2]) if consistency else [])
+                for out, y in zip(outs, tile):
+                    out[..., t0:t1] = y.permute(0, 3, 1, 2)[:, :n_out, ..., keep]     # a variant's output is channel 0 of its pairs
                 latents[..., t0:t1] = P.from_c8(lat, self.encoder.latent_size).squeeze(-2)[..., keep]
-                if consistency:
-                    lat_t, emb_t = self.encoder.forward_c8(_interleave(trn))
-                    skips_t = self._skips_c8(emb_t)
-                    outs[2][..., t0:t1] = self._head(self.decoder.forward_c8(lat_t, True, skips_t))[..., keep]
-                    outs[3][..., t0:t1] = self._head(self.decoder.forward_c8(lat_t, False, skips_t))[..., keep]
         return outs[0], latents, outs[1], (outs[2] if consistency else None), (outs[3] if consistency else None), dict()
 
 
@@ -856,6 +863,7 @@ class TimbreTrapMag(TimbreTrap):
     """modules.py:892-1001: magnitude-CQT variant - one-channel encoder input |c|, one-channel relu output, tanh activations."""
 
     HEAD_MODE = 1               # relu (modules.py:976)
+    ACTIVATIONS_MODE = 3        # tanh (modules.py:996): tanh(relu(h)) = tanh(h) on the head's output h >= 0
 
     def __init__(self, sample_rate, n_octaves, bins_per_octave, secs_per_block=3, latent_size=None, model_complexity=1, skip_connections=False):
         TimbreTrap.__init__(self, sample_rate, n_octaves, bins_per_octave, secs_per_block, latent_size, model_complexity, skip_connections)
@@ -866,7 +874,7 @@ class TimbreTrapMag(TimbreTrap):
 
     def _features(self, audio):
         """modules.py:947: to_magnitude(sliCQ(audio)) as pairs (|c|, 0)."""
-        return _widen(CQT._magnitude(self.sliCQ.encode_interleaved(audio).permute(0, 3, 1, 2), False))
+        return ops.widen(CQT._magnitude(self.sliCQ.encode_interleaved(audio).permute(0, 3, 1, 2), False))
 
     def to_activations(self, coefficients):
         """modules.py:980-1001: tanh of the (B, 1, F, T) magnitude coefficients -> (B, F, T).  Like the reference's `squeeze(-3)`, a
@@ -879,11 +887,12 @@ class TimbreTrapMagDB(TimbreTrapMag):
     """modules.py:1004-1075: decibel-magnitude variant - encoder input to_decibels(|c|) in [0, 1], sigmoid output, activations = output."""
 
     HEAD_MODE = 2               # sigmoid (modules.py:1052)
+    ACTIVATIONS_MODE = 0        # the head's output as it is (modules.py:1056-1075)
 
     def _features(self, audio):
         """modules.py:1024-1027."""
         mag = CQT._magnitude(self.sliCQ.encode_interleaved(audio).permute(0, 3, 1, 2), False)
-        return _widen(CQT.to_decibels(mag))
+        return ops.widen(CQT.to_decibels(mag))
 
     def to_activations(self, coefficients):
         """modules.py:1056-1075."""

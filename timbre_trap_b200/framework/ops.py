@@ -1,5 +1,5 @@
 """
-Thin torch-tensor wrappers over the conv entry points of the C ABI (include/timbre_trap_b200.h).
+Thin torch-tensor wrappers over the conv and element-wise entry points of the C ABI (include/timbre_trap_b200.h).
 Tensors are C8 planar bf16 (B, CG, H, T, 8) unless noted; weights are already packed (packing.py).
 PyTorch is used for allocation and stream ownership only.
 """
@@ -142,3 +142,33 @@ def conv_same(x, w, bias, k, dilation=1, act=False, times_elu_grad_of=None, plus
         _lib.check(_lib.lib().tt_conv_same_post(_p(x), _p(y), _p(w), _p(bias) if bias is not None else None, B, CG * 8, H, T, k, dilation,
                                                 int(act), post, _p(e) if e is not None else None, _s(x)))
     return y
+
+
+def widen(x):
+    """(B, F, T) fp32 -> interleaved (B, F, T, 2) pairs (x, 0) (tt_widen_pairs)."""
+    x = x.detach().float().contiguous()
+    out = torch.empty(tuple(x.shape) + (2,), dtype=torch.float32, device=x.device)
+    if x.numel():
+        with torch.cuda.device(x.device):
+            _lib.check(_lib.lib().tt_widen_pairs(_p(x), x.numel(), _p(out), _s(x)))
+    return out
+
+
+def channel0(pairs, mode):
+    """interleaved (B, F, T, 2) -> (B, F, T): channel 0 through a non-linearity (tt_channel0_activation modes)."""
+    out = torch.empty(pairs.shape[:-1], dtype=torch.float32, device=pairs.device)
+    if out.numel():
+        with torch.cuda.device(pairs.device):
+            _lib.check(_lib.lib().tt_channel0_activation(_p(pairs), out.numel(), mode, _p(out), _s(pairs)))
+    return out
+
+
+def add_scaled(x, e, scale, out=None):
+    """x + scale * e on two bf16 tensors of one layout, one pass (tt_add_scaled_bf16); scale is a 0-dim device tensor."""
+    if x.shape != e.shape or x.dtype != torch.bfloat16 or e.dtype != torch.bfloat16:
+        raise ValueError(f'skip connection: {tuple(x.shape)} {x.dtype} vs {tuple(e.shape)} {e.dtype}')
+    out = torch.empty_like(x) if out is None else out
+    s = scale.detach().float().reshape(1)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().tt_add_scaled_bf16(_p(x), _p(e.contiguous()), _p(s), _p(out), x.numel(), _s(x)))
+    return out

@@ -16,6 +16,29 @@ __all__ = ['pack_down_pairs', 'pack_res_rs', 'pack_res_rs_pairs', 'pack_res_rs_f
            'pad_vec']
 
 
+class _PackedCache:
+    """Packed (kernel-layout) copies of a module's parameters, rebuilt when a parameter is modified or moved."""
+
+    epoch = 0       # bumped by code that updates parameters outside torch's version counter (framework/train.py's AdamW kernel)
+
+    def __init__(self):
+        self._key = None
+        self._val = None
+
+    def __getstate__(self):
+        # pickling / deep-copying a module (the reference checkpoints whole modules, experiments/train.py:511) drops the packed
+        # copies: they are rebuilt lazily from the parameters of the new object
+        return dict(_key=None, _val=None)
+
+    def get(self, params, build):
+        key = (_PackedCache.epoch,) + tuple((p.data_ptr(), p._version, p.device) for p in params)
+        if key != self._key:
+            with torch.no_grad():
+                self._val = build()
+            self._key = key
+        return self._val
+
+
 def pad8(c):
     return (c + 7) // 8 * 8
 

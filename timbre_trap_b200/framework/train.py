@@ -6,42 +6,51 @@ The reference's loss step (reference: experiments/train.py:393-500) on the CUDA 
                                                     losses, backward, gradient all-reduce (NCCL, when a process group is
                                                     given), clip_grad_norm_(10), AdamW
 
-Every layer is a torch.autograd.Function whose forward is the inference kernel (tcgen05 strips) and whose backward stays in the
-bf16 inference layouts (C8 planar / packed 4-channel): weight gradients are tcgen05 GEMMs over the pixel axis with a fixed-order
-reduction (csrc/wgrad_tc.cu), data gradients are the forward kernels on transformed weights without activation, and ELU
-derivatives, skip connections and re-layouts are one-pass bf16 kernels; the losses, clip and AdamW have kernels of their own
-(csrc/loss_kernels.cu, csrc/train_kernels.cu).  PyTorch's autograd engine only walks the graph and accumulates `.grad`; there
-is no cuDNN / ATen compute on the path.
+The forward is the model's own (TimbreTrap._passes); with gradients every layer runs as a torch.autograd.Function whose forward is the
+inference kernel and whose backward stays in the bf16 inference layouts (framework/layer_grads.py); clip and AdamW have kernels of
+their own (csrc/train_kernels.cu).  PyTorch's autograd engine only walks the graph and accumulates `.grad`; there is no cuDNN / ATen
+compute on the path.
 Differences to the reference that do not change values: the CQT target is computed once (the reference computes it twice,
 train.py:404 and modules.py:366 -> :88); no `.item()` host syncs inside the step; activation gradients travel in bf16 between
 layers (the reference runs the forward under fp16 autocast).
 """
 
-import ctypes
-
 import torch
 
 from .. import _lib
-from . import ops
-from . import packing as P
-from .cqt import CQT
-from .modules import _PackedCache, _channel0, _widen
-from .objectives import compute_consistency_loss, compute_reconstruction_loss, compute_transcription_loss
+from . import packing as P  # noqa: F401
+from .layer_grads import _ActivationsFn, _Channel0ActivationsFn, _p, _s, _SqDiffFn, _TrnLossFn
+# the weight-gradient and edge-kernel wrappers, where code written against the earlier layout of this module reaches them
+from .layer_grads import _channel0_bwd, _film_convin_grads, _wgrad_lat, _wgrad_same, _wgrad_updown  # noqa: F401
+from .packing import _PackedCache
 
 __all__ = ['compute_step_losses', 'TrainStep', 'allreduce_mean_gradients']
 
 
-def _p(t):
-    return ctypes.c_void_p(t.data_ptr()) if t is not None else None
+def _step_losses(model, audio, ground_truth, mult, late_start, grad):
+    """The losses of compute_step_losses / TrainStep.losses; `grad`: the model's layers through their autograd Functions.  The
+    transcription loss is formed before the consistency pass, so that autograd adds up the transcription's gradients in one order."""
+    with torch.no_grad():
+        coeffs = model._features(audio)                                     # the reconstruction target (see TrainStep), computed once
+    rec, trn, _ = model._passes(coeffs, grad)
+    mode = model.ACTIVATIONS_MODE
+    act = _ActivationsFn.apply(trn) if mode is None else _Channel0ActivationsFn.apply(trn, mode)
+    n = ground_truth.size(0)
+    out = dict(reconstruction=_SqDiffFn.apply(rec, coeffs), transcription=_TrnLossFn.apply(act[:n].contiguous(), ground_truth.float().contiguous()))
+    total = mult['reconstruction'] * out['reconstruction']
+    if mult['consistency']:
+        trn_rec, trn_scr, _ = model._passes(trn, grad)
+        tgt = trn[:n].contiguous()
+        out['consistency_spectral'] = _SqDiffFn.apply(trn_rec[:n].contiguous(), tgt)
+        out['consistency_score'] = _SqDiffFn.apply(trn_scr[:n].contiguous(), tgt)
+    if not late_start:
+        total = total + mult['transcription'] * out['transcription']
+        if mult['consistency']:
+            total = total + mult['consistency'] * (out['consistency_spectral'] + out['consistency_score'])
+    out['total'] = total
+    return out
 
 
-def _s(t):
-    return ctypes.c_void_p(torch.cuda.current_stream(t.device).cuda_stream)
-
-
-# ---------------------------------------------------------------------------------------------------------------
-# forward half without a graph
-# ---------------------------------------------------------------------------------------------------------------
 def compute_step_losses(model, audio, ground_truth, multipliers=None, late_start=False):
     """
     audio (B, 1, n*L) on the GPU, ground_truth (B_mpe, F, T) with B_mpe <= B (train.py:393-394, 429).
@@ -52,591 +61,8 @@ def compute_step_losses(model, audio, ground_truth, multipliers=None, late_start
     """
     mult = dict(reconstruction=1, transcription=1, consistency=1)
     mult.update(multipliers or {})
-    head = model.HEAD_MODE
-
-    def decode(lat, reconstruct, skips):
-        y = model.decoder.forward_c8(lat, reconstruct, skips)
-        return y if head is None else _widen(_channel0(y, head))
     with torch.no_grad():
-        coefficients = model._features(audio)                                     # (B, F, T, 2), the target, computed once
-        lat, emb = model.encoder.forward_c8(coefficients)
-        skips = model._skips_c8(emb)
-        reconstruction = decode(lat, True, skips).permute(0, 3, 1, 2)
-        transcription_coeffs = decode(lat, False, skips)
-        if head is None:
-            transcription = model.to_activations(transcription_coeffs.permute(0, 3, 1, 2))
-        else:
-            transcription = _channel0(transcription_coeffs, _ACTIVATIONS_MODE[head])
-        n_mpe = ground_truth.size(0)
-        losses = dict(reconstruction=compute_reconstruction_loss(reconstruction, coefficients.permute(0, 3, 1, 2)),
-                      transcription=compute_transcription_loss(transcription[:n_mpe], ground_truth.float(), True))
-        total = mult['reconstruction'] * losses['reconstruction']
-        if mult['consistency']:
-            lat_t, emb_t = model.encoder.forward_c8(transcription_coeffs)
-            skips_t = model._skips_c8(emb_t)
-            trn_rec = decode(lat_t, True, skips_t).permute(0, 3, 1, 2)
-            trn_scr = decode(lat_t, False, skips_t).permute(0, 3, 1, 2)
-            sp, sc = compute_consistency_loss(trn_rec[:n_mpe], trn_scr[:n_mpe], transcription_coeffs.permute(0, 3, 1, 2)[:n_mpe])
-            losses['consistency_spectral'], losses['consistency_score'] = sp, sc
-        if not late_start:
-            total = total + mult['transcription'] * losses['transcription']
-            if mult['consistency']:
-                total = total + mult['consistency'] * (losses['consistency_spectral'] + losses['consistency_score'])
-        losses['total'] = total
-    return losses
-
-
-# ---------------------------------------------------------------------------------------------------------------
-# autograd Functions: fast forward kernel + native backward kernels
-# ---------------------------------------------------------------------------------------------------------------
-# ---- residual blocks: the whole backward in the inference layouts (bf16), convolutions AND weight gradients on the tensor cores ----
-def _ew(fn_name, *tensors):
-    """element-wise bf16 kernel over tensors of one common layout -> new tensor like the first"""
-    out = torch.empty_like(tensors[0])
-    _lib.check(getattr(_lib.lib(), fn_name)(*[_p(t) for t in tensors], _p(out), out.numel(), _s(out)))
-    return out
-
-
-def _as_c8(t):
-    """packed 4-channel (B, H, T, 4) -> C8 planar (B, 1, H, T, 8) (native re-layout kernel); C8 tensors pass through"""
-    if t.dim() == 5:
-        return t
-    B, H, T, _ = t.shape
-    out = torch.empty((B, 1, H, T, 8), dtype=torch.bfloat16, device=t.device)
-    _lib.check(_lib.lib().tt_p4_to_c8(_p(t), _p(out), B * H * T, _s(t)))
-    return out
-
-
-def _to_layout_of(c8, ref):
-    """C8 planar (B, 1, H, T, 8) -> the layout of `ref` (packed 4-channel or C8)"""
-    if ref.dim() == 5:
-        return c8
-    out = torch.empty_like(ref)
-    _lib.check(_lib.lib().tt_c8_to_p4(_p(c8), _p(out), out.numel() // 4, _s(out)))
-    return out
-
-
-_WGRAD_SCRATCH = {}
-_BW_PACKS = {'epoch': -1}
-
-
-def _scratch(pool, device, n):
-    """One growing fp32 scratch buffer per device (the weight-gradient partials): reused by every layer, reallocated only to grow."""
-    buf = pool.get(device)
-    if buf is None or buf.numel() < n:
-        buf = torch.empty(n, dtype=torch.float32, device=device)
-        pool[device] = buf
-    return buf
-
-
-def _bw_pack(weight, tag, build):
-    """Packed (kernel-layout) weights of the backward pass, built once per optimisation step per layer: the same layer runs backward
-    two to four times per step (two encoder, four decoder passes), and every pack is a handful of tiny launches."""
-    if _BW_PACKS['epoch'] != _PackedCache.epoch:
-        _BW_PACKS.clear()
-        _BW_PACKS['epoch'] = _PackedCache.epoch
-    key = (weight.data_ptr(), weight._version, tag)
-    if key not in _BW_PACKS:
-        with torch.no_grad():
-            _BW_PACKS[key] = build()
-    return _BW_PACKS[key]
-
-
-def _wgrad_same(x8, dz8, cin, cout, k, d):
-    """(dW (cout, cin, k, k), db (cout)) fp32 of a 'same' conv from C8 planar bf16 x and dz (tt_conv_wgrad_same, tensor cores)."""
-    B, CGi, H, T, _ = x8.shape
-    lib = _lib.lib()
-    scratch = _scratch(_WGRAD_SCRATCH, x8.device, int(lib.tt_wgrad_scratch_floats(B, H, T)))
-    dw = torch.zeros((cout, cin, k, k), dtype=torch.float32, device=x8.device)
-    db = torch.zeros(cout, dtype=torch.float32, device=x8.device)
-    _lib.check(lib.tt_conv_wgrad_same(_p(x8), _p(dz8), _p(dw), _p(db), B, CGi * 8, dz8.size(1) * 8, cin, cout, H, T, k, d,
-                                      _p(scratch), _s(x8)))
-    return dw, db
-
-
-class _ResFn(torch.autograd.Function):
-    """ResidualConv2dBlock: fused forward kernel, which also writes the inner activation ELU(W1 * x + b1) it stages in shared memory
-    (tt_res_block_rs_mid) - the backward needs it and a recompute costs a whole 3x3 conv launch per block; the backward stays in bf16
-    C8 planar end to end - both data-gradient convolutions through the tile kernel (tt_conv_same), both weight gradients through the
-    MN-major tcgen05 kernels (tt_conv_wgrad_same), the ELU derivatives / residual add as one-pass element-wise kernels."""
-
-    @staticmethod
-    def forward(ctx, x, w1, b1, w2, b2, run, c, d):
-        a1 = torch.empty_like(x)
-        y = run(x, a1)
-        ctx.save_for_backward(x, y, a1, w1, b1, w2)
-        ctx.meta = (c, d)
-        return y
-
-    @staticmethod
-    def backward(ctx, gy):
-        x, y, a1, w1, b1, w2 = ctx.saved_tensors
-        c, d = ctx.meta
-        w2_t = _bw_pack(w2, 'res1x1T', lambda: P.pack_res1x1(w2.detach().float().transpose(0, 1).contiguous()))
-        w1_t = _bw_pack(w1, 'res3x3T', lambda: P.pack_res3x3(w1.detach().float().transpose(0, 1).flip(2, 3).contiguous()))
-        gy = gy.contiguous()
-        dz2 = _as_c8(_ew('tt_res_out_bwd_bf16', gy, y, x))                       # gy * ELU'(z2), activated 1x1 output = y - x
-        x8 = _as_c8(x)
-        a1 = _as_c8(a1)                                                          # the inner activation, as the forward staged it
-        dw2, db2 = _wgrad_same(a1, dz2, c, c, 1, 1)
-        dz1 = ops.conv_same(dz2, w2_t, None, 1, 1, times_elu_grad_of=a1)         # W2^T dz2, times ELU'(z1): one launch
-        dw1, db1 = _wgrad_same(x8, dz1, c, c, 3, d)
-        if gy.dim() == 5:
-            gx = ops.conv_same(dz1, w1_t, None, 3, d, plus=gy)                   # gx = gy + W1^T (*) dz1: the residual add in the epilogue
-        else:
-            gx = _to_layout_of(ops.conv_same(dz1, w1_t, None, 3, d), x)          # packed 4-channel stage: re-layout, then add
-            one = torch.ones((), dtype=torch.float32, device=gx.device)
-            _lib.check(_lib.lib().tt_add_scaled_bf16(_p(gy), _p(gx), _p(one.reshape(1)), _p(gx), gx.numel(), _s(gx)))
-        return gx, dw1, db1, dw2, db2, None, None, None
-
-
-def _wgrad_updown(fine8, coarse8, cfine, ccoarse, transposed):
-    """Weight / bias gradients of a (4,1) stride-(2,1) layer from C8 planar bf16 tensors (tt_conv_wgrad_updown, tensor cores):
-    sconv: (fine = layer input, coarse = dz) -> dW (ccoarse, cfine, 4, 1), db (ccoarse); tconv (transposed): (fine = dz, coarse = layer
-    input) -> dW (ccoarse, cfine, 4, 1) in the ConvTranspose2d layout, db (cfine)."""
-    B, CGf, Hf, T, _ = fine8.shape
-    Hc = coarse8.size(2)
-    lib = _lib.lib()
-    scratch = _scratch(_WGRAD_SCRATCH, fine8.device, int(lib.tt_wgrad_scratch_floats(B, Hc, T)))
-    dw = torch.zeros((ccoarse, cfine, 4, 1), dtype=torch.float32, device=fine8.device)
-    db = torch.zeros(cfine if transposed else ccoarse, dtype=torch.float32, device=fine8.device)
-    _lib.check(lib.tt_conv_wgrad_updown(_p(fine8), _p(coarse8), _p(dw), _p(db), B, CGf * 8, coarse8.size(1) * 8, cfine, ccoarse, Hf, Hc, T,
-                                        int(transposed), _p(scratch), _s(fine8)))
-    return dw, db
-
-
-class _DownFn(torch.autograd.Function):
-    """EncoderBlock.sconv + ELU (modules.py:626-629).  Backward in the inference layouts: ELU derivative (element-wise), weight gradient
-    (tensor-core GEMM over the pixel axis), data gradient = the transposed-conv forward kernel without activation on W seen as a
-    ConvTranspose2d weight (in = Cout, out = Cin)."""
-
-    @staticmethod
-    def forward(ctx, x, weight, bias, run, cin, cout):
-        y = run(x)
-        ctx.save_for_backward(x, y, weight)
-        ctx.meta = (cin, cout)
-        return y
-
-    @staticmethod
-    def backward(ctx, gy):
-        x, y, weight = ctx.saved_tensors
-        cin, cout = ctx.meta
-        dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)
-        x8 = _as_c8(x)
-        dw, db = _wgrad_updown(x8, dz, cin, cout, False)
-        gx = None
-        if ctx.needs_input_grad[0]:
-            hin, hout = x8.size(2), dz.size(2)
-            wt = _bw_pack(weight, 'downT', lambda: P.pack_up_strip(weight.detach().float(), torch.zeros(cin, device=weight.device)))
-            gx = ops.conv_up_strip(dz, wt, P.pad8(cin), hin - 2 * hout - 2, packed4_out=x.dim() == 4, act=False)
-        return gx, dw, db, None, None, None
-
-
-class _UpFn(torch.autograd.Function):
-    """DecoderBlock.tconv + ELU (modules.py:685-688).  Backward: data gradient = the strided-conv forward kernel without activation on
-    W^T seen as a Conv2d weight (out = Cin, in = Cout)."""
-
-    @staticmethod
-    def forward(ctx, x, weight, bias, run, cin, cout):
-        y = run(x)
-        ctx.save_for_backward(x, y, weight)
-        ctx.meta = (cin, cout)
-        return y
-
-    @staticmethod
-    def backward(ctx, gy):
-        x, y, weight = ctx.saved_tensors
-        cin, cout = ctx.meta
-        dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)                          # layout of y (packed 4-channel for the last stage)
-        dw, db = _wgrad_updown(_as_c8(dz), x, cout, cin, True)
-        # ConvTranspose2d (cin, cout, 4, 1) read as a Conv2d weight (out = cin, in = cout)
-        pack = P.pack_down_pairs if dz.dim() == 4 else P.pack_down_strip
-        wd = _bw_pack(weight, 'upT', lambda: pack(weight.detach().float().contiguous(), torch.zeros(cin, device=weight.device)))
-        gx = ops.conv_down_strip(dz, wd, P.pad8(cin), act=False)
-        return gx, dw, db, None, None, None
-
-
-_LAT_SCRATCH = {}
-
-
-def _wgrad_lat(tall8, flat8, ctall, cflat, dw, db, row_sums):
-    """tt_conv_wgrad_lat: accumulates into dw (cflat.., ctall, H, 1) [first cflat rows], db (cflat) and row_sums (ctall, H) (either may be None).
-    The kernel takes up to 128 flat-side channels; wider latents go through it in slices of 128 (a slice of the 1-row latents is a tiny copy)."""
-    B, CGt, H, T, _ = tall8.shape
-    lib = _lib.lib()
-    scratch = _scratch(_LAT_SCRATCH, tall8.device, int(lib.tt_wgrad_lat_scratch_floats(B, H, T)))
-    for c0 in range(0, cflat, 128):
-        c1 = min(cflat, c0 + 128)
-        flat = flat8[:, c0 // 8:c0 // 8 + 16].contiguous()
-        _lib.check(lib.tt_conv_wgrad_lat(_p(tall8), _p(flat), _p(dw[c0:c1]), _p(None if db is None else db[c0:c1]), _p(row_sums if c0 == 0 else None),
-                                         B, CGt * 8, flat.size(1) * 8, ctall, c1 - c0, H, T, _p(scratch), _s(tall8)))
-
-
-class _LatFn(torch.autograd.Function):
-    """Encoder.convlat (modules.py:446, no activation).  Backward in the inference layouts: weight gradient = tap-grouped tensor-core GEMM
-    over (b, t); data gradient = the Decoder.convin forward kernel (a (H, 1) transposed conv) without activation on the same weights."""
-
-    @staticmethod
-    def forward(ctx, x, weight, bias, run, c4, d, d_pad):
-        y = run(x)
-        ctx.save_for_backward(x, weight)
-        ctx.meta = (c4, d, d_pad)
-        return y
-
-    @staticmethod
-    def backward(ctx, gy):
-        x, weight = ctx.saved_tensors
-        c4, d, d_pad = ctx.meta
-        gy = gy.contiguous()
-        dw = torch.zeros(weight.shape, dtype=torch.float32, device=x.device)
-        db = torch.zeros(d, dtype=torch.float32, device=x.device)
-        _wgrad_lat(x, gy, c4, d, dw, db, None)
-        # gx[ci, h, t] = sum_co W[co, ci, h] gy[co, t]: ConvTranspose2d with weight (in = co, out = ci, H, 1)
-        w, table = _bw_pack(weight, 'latT', lambda: P.pack_deconv_in_film(weight.detach().float(), torch.zeros(c4, device=x.device),
-                                                                          torch.ones(d, device=x.device), torch.zeros(d, device=x.device), d_pad))
-        gx = ops.deconv_in(gy, w, table, P.pad8(c4), x.size(2), act=False)
-        return gx, dw, db, None, None, None, None
-
-
-def _pairs_to_c8(pairs):
-    """fp32 interleaved (B, F, T, 2) -> C8 planar bf16 (B, 1, F, T, 8) (tt_pairs_to_c8)."""
-    pairs = pairs.contiguous()
-    B, F_, T, _ = pairs.shape
-    out = torch.empty((B, 1, F_, T, 8), dtype=torch.bfloat16, device=pairs.device)
-    _lib.check(_lib.lib().tt_pairs_to_c8(_p(pairs), B * F_ * T, _p(out), _s(pairs)))
-    return out
-
-
-def _two_channels(w, dim):
-    """A one-channel conv weight of the magnitude variants zero-padded to two channels along `dim`, as the forward packs run it
-    (Encoder._packed / Decoder._packed); two-channel weights pass through."""
-    if w.size(dim) == 2:
-        return w
-    return torch.cat((w, torch.zeros_like(w)), dim=dim)
-
-
-class _InFn(torch.autograd.Function):
-    """Encoder.convin + ELU (modules.py:430-433) with a packed 4-channel output.  Backward: ELU derivative on the packed tensor; weight
-    gradient on the tensor cores (both operands re-laid out to C8 planar bf16 by one-pass kernels); data gradient (only the consistency
-    pass asks for it) = the Decoder.convout forward kernel on transposed, flipped weights.  The one-channel convin of the magnitude
-    variants (modules.py:908-911) reads pairs (x, 0) against zero-padded weights: its weight gradient is the first input column of the
-    two-channel one."""
-
-    @staticmethod
-    def forward(ctx, coeffs, weight, bias, run, c0):
-        y = run(coeffs)
-        ctx.save_for_backward(coeffs, y, weight)
-        ctx.c0 = c0
-        return y
-
-    @staticmethod
-    def backward(ctx, gy):
-        coeffs, y, weight = ctx.saved_tensors
-        c0 = ctx.c0
-        dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)
-        dw, db = _wgrad_same(_pairs_to_c8(coeffs), _as_c8(dz), 2, c0, 3, 1)
-        gx = None
-        if ctx.needs_input_grad[0]:
-            wt, zb = _bw_pack(weight, 'inT', lambda: (_two_channels(weight.detach().float(), 1).transpose(0, 1).flip(2, 3).contiguous(),  # (2, c0, 3, 3)
-                                                      torch.zeros(2, device=dz.device)))
-            gx = ops.conv_out(dz, wt, zb, c0)
-        if weight.size(1) == 1:
-            dw = dw[:, :1]
-        return gx, dw, db, None, None
-
-
-class _OutFn(torch.autograd.Function):
-    """Decoder.convout (modules.py:543, no activation) on a packed 4-channel input.  Backward: weight gradient on the tensor cores;
-    data gradient = the Encoder.convin forward kernel without ELU on transposed, flipped weights.  The one-channel convout of the
-    magnitude variants (modules.py:913) runs as two channels with a zero second one: its gradients are the first rows of the
-    two-channel ones."""
-
-    @staticmethod
-    def forward(ctx, x, weight, bias, run, c):
-        y = run(x)
-        ctx.save_for_backward(x, weight)
-        ctx.c = c
-        return y
-
-    @staticmethod
-    def backward(ctx, gy):
-        x, weight = ctx.saved_tensors
-        c = ctx.c
-        gy = gy.contiguous()
-        dw, db = _wgrad_same(_as_c8(x), _pairs_to_c8(gy), c, 2, 3, 1)
-        wt, zb = _bw_pack(weight, 'outT', lambda: (_two_channels(weight.detach().float(), 0).transpose(0, 1).flip(2, 3).contiguous(),  # (c, 2, 3, 3)
-                                                   torch.zeros(c, device=gy.device)))
-        B, F_, T, _ = gy.shape
-        gx = torch.empty((B, F_, T, 4), dtype=torch.bfloat16, device=gy.device)
-        _lib.check(_lib.lib().tt_conv_in(_p(gy), _p(gx), _p(wt), _p(zb), B, c, F_, T, 2, _s(gy)))
-        if weight.size(0) == 1:
-            dw, db = dw[:1], db[:1]
-        return gx, dw, db, None, None
-
-
-class _SkipAddFn(torch.autograd.Function):
-    """Decoder skip connection (modules.py:568-589) with TimbreTrap.apply_skip_connections' learnable weight (:110-112):
-    out = x + w * e on two bf16 tensors of one layout, one pass; gradients: x <- g, e <- w * g (one pass), w <- <g, e> (deterministic)."""
-
-    @staticmethod
-    def forward(ctx, x, e, w):
-        scale = w.detach().float().reshape(1)
-        out = torch.empty_like(x)
-        _lib.check(_lib.lib().tt_add_scaled_bf16(_p(x), _p(e), _p(scale), _p(out), x.numel(), _s(x)))
-        ctx.save_for_backward(e, scale)
-        return out
-
-    @staticmethod
-    def backward(ctx, g):
-        e, scale = ctx.saved_tensors
-        g = g.contiguous()
-        lib = _lib.lib()
-        ge = torch.empty_like(g)
-        _lib.check(lib.tt_add_scaled_bf16(_p(g), _p(g), _p(scale - 1.0), _p(ge), g.numel(), _s(g)))        # g + (w - 1) g = w g
-        gw = torch.empty((), dtype=torch.float32, device=g.device)
-        scratch = torch.empty(int(lib.tt_dot_scratch_floats()), dtype=torch.float32, device=g.device)
-        _lib.check(lib.tt_dot_bf16(_p(g), _p(e), g.numel(), _p(gw), _p(scratch), _s(g)))
-        return g, ge, gw
-
-
-class _ActivationsFn(torch.autograd.Function):
-    """TimbreTrap.to_activations (modules.py:271-289) on interleaved coefficients (B, F, T, 2) -> (B, F, T)."""
-
-    @staticmethod
-    def forward(ctx, coeffs):
-        ctx.save_for_backward(coeffs)
-        return CQT._magnitude(coeffs.permute(0, 3, 1, 2), True)
-
-    @staticmethod
-    def backward(ctx, gact):
-        (coeffs,) = ctx.saved_tensors
-        g = torch.empty_like(coeffs)
-        _lib.check(_lib.lib().tt_activations_bwd(_p(coeffs), _p(gact.contiguous()), _p(g), gact.numel(), _s(coeffs)))
-        return g
-
-
-def _channel0_bwd(pairs, gpairs, mode):
-    """(g * f'(v0), 0) for the pre-activation pairs v and the output-pair gradient g (tt_channel0_activation_bwd)."""
-    gpairs = gpairs.contiguous()
-    g = torch.empty_like(pairs)
-    _lib.check(_lib.lib().tt_channel0_activation_bwd(_p(pairs), _p(gpairs), pairs.numel() // 2, mode, _p(g), _s(pairs)))
-    return g
-
-
-class _HeadFn(torch.autograd.Function):
-    """The output head of the magnitude variants on the decoder's pairs (modules.py:976, 1052): (B, F, T, 2) -> pairs (f(v0), 0),
-    f = relu (mode 1) or sigmoid (mode 2); the one-channel output stays a pair with a zero second channel."""
-
-    @staticmethod
-    def forward(ctx, pairs, mode):
-        ctx.save_for_backward(pairs)
-        ctx.mode = mode
-        return _widen(_channel0(pairs, mode))
-
-    @staticmethod
-    def backward(ctx, g):
-        (pairs,) = ctx.saved_tensors
-        return _channel0_bwd(pairs, g, ctx.mode), None
-
-
-class _Channel0ActivationsFn(torch.autograd.Function):
-    """to_activations of the magnitude variants on the head's pairs (h, 0) -> (B, F, T): tanh(h) for TimbreTrapMag (modules.py:996;
-    mode 3, tanh(relu(h)) = tanh(h) as h >= 0), h for TimbreTrapMagDB (:1056-1075; mode 0)."""
-
-    @staticmethod
-    def forward(ctx, pairs, mode):
-        ctx.save_for_backward(pairs)
-        ctx.mode = mode
-        return _channel0(pairs, mode)
-
-    @staticmethod
-    def backward(ctx, gact):
-        (pairs,) = ctx.saved_tensors
-        return _channel0_bwd(pairs, _widen(gact), ctx.mode), None
-
-
-# tt_channel0_activation mode of a magnitude variant's to_activations, by its HEAD_MODE: relu head -> tanh, sigmoid head -> identity
-_ACTIVATIONS_MODE = {1: 3, 2: 0}
-
-
-class _SqDiffFn(torch.autograd.Function):
-    """compute_reconstruction_loss (objectives.py:11-33) on two interleaved coefficient tensors; gradients to both."""
-
-    @staticmethod
-    def forward(ctx, a, b):
-        ctx.save_for_backward(a, b)
-        return compute_reconstruction_loss(a.permute(0, 3, 1, 2), b.permute(0, 3, 1, 2))
-
-    @staticmethod
-    def backward(ctx, gout):
-        a, b = ctx.saved_tensors
-        scale = 1.0 / (a.size(0) * a.size(2))
-        ga = torch.empty_like(a) if ctx.needs_input_grad[0] else None
-        gb = torch.empty_like(b) if ctx.needs_input_grad[1] else None
-        _lib.check(_lib.lib().tt_sum_sq_diff_bwd(_p(a), _p(b), _p(gout.contiguous()), scale, _p(ga), _p(gb), a.numel(), _s(a)))
-        return ga, gb
-
-
-class _TrnLossFn(torch.autograd.Function):
-    """compute_transcription_loss(estimate, target, weight_positive_class=True) (objectives.py:36-74)."""
-
-    @staticmethod
-    def forward(ctx, est, tgt):
-        ctx.save_for_backward(est, tgt)
-        return compute_transcription_loss(est, tgt, True)
-
-    @staticmethod
-    def backward(ctx, gout):
-        est, tgt = ctx.saved_tensors
-        g = torch.empty_like(est)
-        B, F, T = est.shape
-        _lib.check(_lib.lib().tt_transcription_loss_bwd(_p(est), _p(tgt), _p(gout.contiguous()), B, F, T, 1, _p(g), _s(est)))
-        return g, None
-
-
-# ---------------------------------------------------------------------------------------------------------------
-# the differentiable forward (same kernels, same order as Encoder / Decoder .forward_c8)
-# ---------------------------------------------------------------------------------------------------------------
-def _res(blk, x):
-    c1, c2 = blk.conv1[0], blk.conv2[0]
-    return _ResFn.apply(x, c1.weight, c1.bias, c2.weight, c2.bias, lambda t, mid: blk.forward_c8(t, mid_out=mid), blk.channels, blk.dilation)
-
-
-def _encoder(enc, coeffs):
-    """-> (latents C8, [the five embeddings in their internal layouts])"""
-    ch = enc.channels
-    w_in, b_in, w_lat, b_lat = enc._packed()
-    ci = enc.convin[0]
-    x = _InFn.apply(coeffs, ci.weight, ci.bias, lambda t: ops.conv_in(t, w_in, b_in, ch[0], packed4=True), ch[0])
-    emb = [x]
-    for i, blk in enumerate((enc.block1, enc.block2, enc.block3, enc.block4)):
-        for rb in (blk.block1, blk.block2, blk.block3):
-            x = _res(rb, x)
-        sc = blk.sconv[0]
-
-        def run_down(t, blk=blk):
-            pack = P.pack_down_pairs if blk.packed4 else P.pack_down_strip
-            (w,) = blk._cache.get((blk.sconv[0].weight, blk.sconv[0].bias), lambda: (pack(blk.sconv[0].weight, blk.sconv[0].bias),))
-            return ops.conv_down_strip(t, w, P.pad8(blk.out_channels))
-        x = _DownFn.apply(x, sc.weight, sc.bias, run_down, ch[i], ch[i + 1])
-        emb.append(x)
-    cl = enc.convlat
-    return _LatFn.apply(x, cl.weight, cl.bias, lambda t: ops.conv_lat(t, w_lat, b_lat, enc.latent_pad), ch[4], enc.latent_size, enc.latent_pad), emb
-
-
-class _IndicatorFn(torch.autograd.Function):
-    """
-    Decoder.convin on latents + the constant indicator channel (modules.py:139-142, 533-536).  Forward: tt_deconv_in with the
-    indicator folded into the bias table.  Backward: transposed-conv gradients with the indicator channel written out (its weight
-    row receives a gradient, its input does not).
-    """
-
-    @staticmethod
-    def forward(ctx, lat, weight, bias, run, flag, d, c0):
-        y = run(lat)
-        ctx.save_for_backward(lat, y, weight)
-        ctx.meta = (flag, d, c0)
-        return y
-
-    @staticmethod
-    def backward(ctx, gy):
-        lat, y, weight = ctx.saved_tensors
-        flag, d, c0 = ctx.meta
-        # ELU derivative, tap-grouped tensor-core weight gradient (rows 0 .. D-1; the indicator row and the bias are row sums of dz),
-        # data gradient = the Encoder.convlat forward kernel on the first D weight rows
-        dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)
-        h0 = y.size(2)
-        dw = torch.zeros(weight.shape, dtype=torch.float32, device=lat.device)
-        rows = torch.zeros((c0, h0), dtype=torch.float32, device=lat.device)
-        _wgrad_lat(dz, lat, c0, d, dw, None, rows)
-        dw[d, :, :, 0] = flag * rows
-        db = rows.sum(dim=1)
-        d_pad = lat.size(1) * 8
-        wl, zl = _bw_pack(weight, 'decinT', lambda: (P.pack_lat(weight.detach().float()[:d], d_pad), torch.zeros(d_pad, device=lat.device)))
-        glat = ops.conv_lat(dz, wl, zl, d_pad)
-        return glat, dw, db, None, None, None, None
-
-
-class _FiLMConvInFn(torch.autograd.Function):
-    """
-    TimbreTrapFiLM: the FiLM layer and Decoder.convin (modules.py:801-809, 838-840), y = ELU(convT(gamma * z + beta)) with gamma / beta
-    = film_layer.gamma / .beta of the one-hot condition [transcribe, not transcribe] (`hot` = the column of its 1).  Forward:
-    tt_deconv_in on the folded pack (packing.pack_deconv_in_film).  Backward: ELU derivative; the tensor-core sums G = dz x z and the
-    row sums of dz (tt_conv_wgrad_lat); every parameter gradient from those in one launch (tt_film_convin_grad); latent gradient =
-    the Encoder.convlat forward kernel on W scaled by gamma.
-    """
-
-    @staticmethod
-    def forward(ctx, lat, weight, bias, gamma_w, gamma_b, beta_w, beta_b, run, hot, d, c0):
-        y = run(lat)
-        ctx.save_for_backward(lat, y, weight, gamma_w, gamma_b, beta_w, beta_b)
-        ctx.meta = (hot, d, c0)
-        return y
-
-    @staticmethod
-    def backward(ctx, gy):
-        lat, y, weight, gamma_w, gamma_b, beta_w, beta_b = ctx.saved_tensors
-        hot, d, c0 = ctx.meta
-        dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)
-        return _film_convin_grads(dz, lat, weight, gamma_w, gamma_b, beta_w, beta_b, hot, d, c0) + (None,) * 4
-
-
-def _film_convin_grads(dz, lat, weight, gamma_w, gamma_b, beta_w, beta_b, hot, d, c0):
-    """Gradients of _FiLMConvInFn from dz (C8 planar, after the ELU derivative) and the latents lat (C8 planar, H = 1):
-    (latents (bf16, C8), convin weight, convin bias, gamma.weight, gamma.bias, beta.weight, beta.bias)."""
-    h0 = dz.size(2)
-    dev = lat.device
-    G = torch.zeros(weight.shape, dtype=torch.float32, device=dev)
-    rows = torch.zeros((c0, h0), dtype=torch.float32, device=dev)
-    _wgrad_lat(dz, lat, c0, d, G, None, rows)
-    dw = torch.empty_like(G)
-    db = torch.empty(c0, dtype=torch.float32, device=dev)
-    dgw, dbw = torch.empty_like(gamma_w), torch.empty_like(beta_w)
-    dgb, dbb = torch.empty_like(gamma_b), torch.empty_like(beta_b)
-    _lib.check(_lib.lib().tt_film_convin_grad(_p(G), _p(rows), _p(weight), _p(gamma_w), _p(gamma_b), _p(beta_w), _p(beta_b), d, c0, h0, hot,
-                                              _p(dw), _p(db), _p(dgw), _p(dgb), _p(dbw), _p(dbb), _s(G)))
-    d_pad = lat.size(1) * 8
-
-    def build():
-        gamma = gamma_w.detach()[:, hot] + gamma_b.detach()                          # film_layer.gamma(one-hot cond)
-        return P.pack_lat(weight.detach().float() * gamma.view(-1, 1, 1, 1), d_pad), torch.zeros(d_pad, device=dev)
-    # gamma differs between the two passes and depends on the FiLM parameters, so they are part of the key
-    wl, zl = _bw_pack(weight, ('filmT', hot, gamma_w.data_ptr(), gamma_w._version, gamma_b.data_ptr(), gamma_b._version), build)
-    glat = ops.conv_lat(dz, wl, zl, d_pad)
-    return glat, dw, db, dgw, dgb, dbw, dbb
-
-
-def _decoder(dec, lat, reconstruct, skips=None):
-    """skips: None or [(weight 0-dim tensor, embedding)] * 5 in encoder order (modules.py:568-589)"""
-    ch = dec.channels
-    w_in, tables, w_out, b_out = dec._packed()
-    ci = dec.convin[0]
-    sw = 1 if reconstruct else 0
-
-    def run_in(t):
-        return ops.deconv_in(t, w_in[sw], tables[sw], P.pad8(ch[0]), dec.embedding_size)
-    film = dec._film
-    if film is None:
-        x = _IndicatorFn.apply(lat, ci.weight, ci.bias, run_in, 1.0 if reconstruct else 0.0, dec.latent_size, ch[0])
-    else:
-        # TimbreTrapFiLM.decode (modules.py:835-838): condition = one-hot [transcribe, not transcribe]
-        x = _FiLMConvInFn.apply(lat, ci.weight, ci.bias, film.gamma.weight, film.gamma.bias, film.beta.weight, film.beta.bias, run_in,
-                                1 if reconstruct else 0, dec.latent_size, ch[0])
-    for i, blk in enumerate((dec.block1, dec.block2, dec.block3, dec.block4)):
-        if skips is not None:
-            x = _SkipAddFn.apply(x, skips[-1 - i][1], skips[-1 - i][0])
-        tc = blk.tconv[0]
-
-        def run_up(t, blk=blk):
-            (w,) = blk._cache.get((blk.tconv[0].weight, blk.tconv[0].bias), lambda: (P.pack_up_strip(blk.tconv[0].weight, blk.tconv[0].bias),))
-            return ops.conv_up_strip(t, w, P.pad8(blk.out_channels), blk.out_pad, packed4_out=blk.packed4)
-        x = _UpFn.apply(x, tc.weight, tc.bias, run_up, ch[i], ch[i + 1])
-        for rb in (blk.block1, blk.block2, blk.block3):
-            x = _res(rb, x)
-    if skips is not None:
-        x = _SkipAddFn.apply(x, skips[0][1], skips[0][0])
-    co = dec.convout
-    return _OutFn.apply(x, co.weight, co.bias, lambda t: ops.conv_out(t, w_out, b_out, ch[4]), ch[4])
+        return _step_losses(model, audio, ground_truth, mult, late_start, grad=False)
 
 
 def allreduce_mean_gradients(params, group, flat=None):
@@ -701,41 +127,7 @@ class TrainStep:
 
     def losses(self, audio, ground_truth, late_start=False):
         """The four losses and their total, with the autograd graph attached."""
-        model = self.model
-        with torch.no_grad():
-            coeffs = model._features(audio)                                     # the reconstruction target (see the class docstring)
-        head = model.HEAD_MODE
-
-        def skips_of(emb):
-            if model.skip_weights is None:
-                return None
-            return [(model.skip_weights[i], e) for i, e in enumerate(emb)]
-
-        def decode(lat, reconstruct, sk):
-            y = _decoder(model.decoder, lat, reconstruct, sk)
-            return y if head is None else _HeadFn.apply(y, head)
-        lat, emb = _encoder(model.encoder, coeffs)
-        sk = skips_of(emb)
-        rec = decode(lat, True, sk)
-        trn = decode(lat, False, sk)
-        act = _ActivationsFn.apply(trn) if head is None else _Channel0ActivationsFn.apply(trn, _ACTIVATIONS_MODE[head])
-        n = ground_truth.size(0)
-        out = dict(reconstruction=_SqDiffFn.apply(rec, coeffs), transcription=_TrnLossFn.apply(act[:n].contiguous(), ground_truth.float().contiguous()))
-        total = self.mult['reconstruction'] * out['reconstruction']
-        if self.mult['consistency']:
-            lat_t, emb_t = _encoder(model.encoder, trn)
-            sk_t = skips_of(emb_t)
-            trn_rec = decode(lat_t, True, sk_t)
-            trn_scr = decode(lat_t, False, sk_t)
-            tgt = trn[:n].contiguous()
-            out['consistency_spectral'] = _SqDiffFn.apply(trn_rec[:n].contiguous(), tgt)
-            out['consistency_score'] = _SqDiffFn.apply(trn_scr[:n].contiguous(), tgt)
-        if not late_start:
-            total = total + self.mult['transcription'] * out['transcription']
-            if self.mult['consistency']:
-                total = total + self.mult['consistency'] * (out['consistency_spectral'] + out['consistency_score'])
-        out['total'] = total
-        return out
+        return _step_losses(self.model, audio, ground_truth, self.mult, late_start, grad=True)
 
     def backward(self, total):
         self.flat_g.zero_()
