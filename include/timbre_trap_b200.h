@@ -285,10 +285,10 @@ int tt_res_out_bwd_bf16(const void* gy, const void* y, const void* x, void* dz, 
 /* packed 4-channel (B, H, T, 4) <-> C8 planar with one channel group (B, 1, H, T, 8), n_pixels = B * H * T */
 int tt_p4_to_c8(const void* p4, void* c8, int64_t n_pixels, void* stream);
 int tt_c8_to_p4(const void* c8, void* p4, int64_t n_pixels, void* stream);
-/* gradients of tt_sum_sq_diff (both arguments; either output may be NULL), tt_transcription_loss (estimate), tanh|c| */
+/* gradients of tt_sum_sq_diff and tt_transcription_loss (both arguments; either output may be NULL), tanh|c| */
 int tt_sum_sq_diff_bwd(const float* a, const float* b, const float* gout, double scale, float* ga, float* gb, int64_t n, void* stream);
 int tt_transcription_loss_bwd(const float* estimate, const float* target, const float* gout, int B, int F, int T,
-                              int weight_positive_class, float* gest, void* stream);
+                              int weight_positive_class, float* gest, float* gtarget, void* stream);
 int tt_activations_bwd(const float* coeffs, const float* dact, float* dcoeffs, int64_t n, void* stream);
 /* TimbreTrapFiLM's Decoder.convin (modules.py:801-809, 838-840): ConvTranspose2d(D, C0, (H0, 1)) on gamma * z + beta, with
  * gamma / beta = film_layer.gamma / .beta of the one-hot condition whose 1 is in column `hot` (0 transcribe, 1 reconstruct).

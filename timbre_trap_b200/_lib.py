@@ -67,7 +67,7 @@ SIGNATURES = {
     'tt_p4_to_c8': (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
     'tt_c8_to_p4': (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
     'tt_sum_sq_diff_bwd': (c_int, [c_void_p] * 3 + [ctypes.c_double] + [c_void_p] * 2 + [c_int64, c_void_p]),
-    'tt_transcription_loss_bwd': (c_int, [c_void_p] * 3 + [c_int] * 4 + [c_void_p, c_void_p]),
+    'tt_transcription_loss_bwd': (c_int, [c_void_p] * 3 + [c_int] * 4 + [c_void_p] * 3),
     'tt_activations_bwd': (c_int, [c_void_p] * 3 + [c_int64, c_void_p]),
     'tt_film_convin_grad': (c_int, [c_void_p] * 7 + [c_int] * 4 + [c_void_p] * 7),
     'tt_grad_sumsq': (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),

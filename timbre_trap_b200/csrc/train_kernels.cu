@@ -22,26 +22,50 @@ __global__ void sq_diff_bwd_kernel(const float* __restrict__ a, const float* __r
     }
 }
 
-// objectives.py:36-74 backward w.r.t. the estimate (B, F, T); one thread per frame
+// objectives.py:36-74 backward w.r.t. the estimate (B, F, T) and / or the target (either output may be null); one thread per frame.
+// With the positive-class weight S = neg / (pos + eps) (neg = sum_f (1 - t_f), pos = sum_f t_f) on the bins whose target is 1, the
+// target also moves S:  dL/dt_k = -dL/de_k + gout / (B T) * dS/dt_k * sum_{f: t_f = 1} (e_f - t_f)^2,  dS/dt_k = -(neg + pos + eps) / (pos + eps)^2
+// (no such term where S = 0, which the forward replaces by 1).
 __global__ void transcription_bwd_kernel(const float* __restrict__ est, const float* __restrict__ tgt, const float* __restrict__ gout,
-                                         int B, int F, int T, int weighted, float* __restrict__ gest) {
+                                         int B, int F, int T, int weighted, float* __restrict__ gest, float* __restrict__ gtgt) {
     const long long frames = (long long)B * T;
     const float s = 2.f * gout[0] / (float)frames;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < frames; i += (long long)gridDim.x * blockDim.x) {
         const long long b = i / T, t = i - b * T;
         const float* e = est + (size_t)b * F * T + t;
         const float* gt = tgt + (size_t)b * F * T + t;
-        float* ge = gest + (size_t)b * F * T + t;
-        float scale = 1.f;
+        float scale = 1.f, pos = 0.f;
         if (weighted) {
-            float pos = 0.f;
             for (int f = 0; f < F; ++f) pos += gt[(size_t)f * T];
             scale = ((float)F - pos) / (pos + 1.1920928955078125e-07f);
             if (scale == 0.f) scale = 1.f;
         }
-        for (int f = 0; f < F; ++f) {
-            const float gv = gt[(size_t)f * T];
-            ge[(size_t)f * T] = s * (gv == 1.f ? scale : 1.f) * (e[(size_t)f * T] - gv);
+        if (gest) {
+            float* ge = gest + (size_t)b * F * T + t;
+            for (int f = 0; f < F; ++f) {
+                const float gv = gt[(size_t)f * T];
+                ge[(size_t)f * T] = s * (gv == 1.f ? scale : 1.f) * (e[(size_t)f * T] - gv);
+            }
+        }
+        if (gtgt) {
+            float dscale = 0.f;                       // dL/dS * dS/dt_k, the same for every bin of the frame
+            if (weighted && (float)F - pos != 0.f) {
+                float q = 0.f;
+                for (int f = 0; f < F; ++f) {
+                    const float gv = gt[(size_t)f * T];
+                    if (gv == 1.f) {
+                        const float d = e[(size_t)f * T] - gv;
+                        q += d * d;
+                    }
+                }
+                const float den = pos + 1.1920928955078125e-07f;
+                dscale = -0.5f * s * q * ((float)F + 1.1920928955078125e-07f) / (den * den);
+            }
+            float* gg = gtgt + (size_t)b * F * T + t;
+            for (int f = 0; f < F; ++f) {
+                const float gv = gt[(size_t)f * T];
+                gg[(size_t)f * T] = dscale - s * (gv == 1.f ? scale : 1.f) * (e[(size_t)f * T] - gv);
+            }
         }
     }
 }
@@ -167,11 +191,12 @@ extern "C" int tt_sum_sq_diff_bwd(const float* a, const float* b, const float* g
 }
 
 extern "C" int tt_transcription_loss_bwd(const float* estimate, const float* target, const float* gout, int B, int F, int T,
-                                         int weight_positive_class, float* gest, void* stream) {
-    TT_REQUIRE(estimate && target && gout && gest, "null argument");
+                                         int weight_positive_class, float* gest, float* gtarget, void* stream) {
+    TT_REQUIRE(estimate && target && gout && (gest || gtarget), "null argument");
     const long long frames = (long long)B * T;
     if (frames <= 0) return TT_OK;
-    transcription_bwd_kernel<<<grid_for(frames), 256, 0, (cudaStream_t)stream>>>(estimate, target, gout, B, F, T, weight_positive_class, gest);
+    transcription_bwd_kernel<<<grid_for(frames), 256, 0, (cudaStream_t)stream>>>(estimate, target, gout, B, F, T, weight_positive_class, gest,
+                                                                                  gtarget);
     TT_CUDA_CHECK(cudaGetLastError());
     tt_count_launches(1);
     return TT_OK;

@@ -1,23 +1,24 @@
 """
-The layers of the loss step as torch.autograd.Functions (the model runs them with `forward_c8(..., grad=True)`, framework/modules.py),
-and the head, activation and loss Functions of the step (framework/train.py).
+The layers of the model as torch.autograd.Functions (the model runs them with `forward_c8(..., grad=True)`, framework/modules.py),
+and the head and activation Functions (the loss Functions are in framework/objectives.py).
 
 Each layer's forward is the inference kernel, handed in by the module as a closure; its backward stays in the bf16 inference layouts
 (C8 planar / packed 4-channel): weight gradients are tcgen05 GEMMs over the pixel axis with a fixed-order reduction (csrc/wgrad_tc.cu),
 data gradients are the forward kernels on transformed weights without activation, and ELU derivatives, skip connections and
-re-layouts are one-pass bf16 kernels; the losses have kernels of their own (csrc/loss_kernels.cu).  PyTorch's autograd engine only
+re-layouts are one-pass bf16 kernels.  A layer computes its weight and bias gradients only when autograd asks for them
+(`ctx.needs_input_grad`): the weight-gradient launch of a layer whose parameters are all frozen is skipped.  PyTorch's autograd engine only
 walks the graph and accumulates `.grad`; there is no cuDNN / ATen compute on the path.
 """
 
 import ctypes
 
 import torch
+from torch.utils.weak import WeakIdKeyDictionary
 
 from .. import _lib
 from . import ops
 from . import packing as P
 from .cqt import CQT
-from .objectives import compute_reconstruction_loss, compute_transcription_loss
 from .packing import _PackedCache
 
 
@@ -57,7 +58,8 @@ def _to_layout_of(c8, ref):
 
 
 _WGRAD_SCRATCH = {}
-_BW_PACKS = {'epoch': -1}
+# weight tensor -> {tag: (stamp, packed)}: one entry per (weight, tag), dropped with the weight
+_BW_PACKS = WeakIdKeyDictionary()
 
 
 def _scratch(pool, device, n):
@@ -69,17 +71,25 @@ def _scratch(pool, device, n):
     return buf
 
 
-def _bw_pack(weight, tag, build):
+def _bw_pack(weight, tag, build, deps=()):
     """Packed (kernel-layout) weights of the backward pass, built once per optimisation step per layer: the same layer runs backward
-    two to four times per step (two encoder, four decoder passes), and every pack is a handful of tiny launches."""
-    if _BW_PACKS['epoch'] != _PackedCache.epoch:
-        _BW_PACKS.clear()
-        _BW_PACKS['epoch'] = _PackedCache.epoch
-    key = (weight.data_ptr(), weight._version, tag)
-    if key not in _BW_PACKS:
+    two to four times per step (two encoder, four decoder passes), and every pack is a handful of tiny launches.  One entry per
+    (weight, tag), rebuilt in place when the weight or one of `deps` (other tensors the pack is built from) has been modified - a torch
+    optimizer's in-place update bumps the version counter, TrainStep's AdamW kernel bumps _PackedCache.epoch - or moved."""
+    stamp = (_PackedCache.epoch,) + tuple((t.data_ptr(), t._version) for t in (weight,) + tuple(deps))
+    packs = _BW_PACKS.get(weight)
+    if packs is None:
+        packs = _BW_PACKS[weight] = {}
+    hit = packs.get(tag)
+    if hit is None or hit[0] != stamp:
         with torch.no_grad():
-            _BW_PACKS[key] = build()
-    return _BW_PACKS[key]
+            hit = packs[tag] = (stamp, build())
+    return hit[1]
+
+
+def _bw_pack_entries():
+    """Number of packs held (one per (weight, tag))."""
+    return sum(len(v) for v in _BW_PACKS.values())
 
 
 def _wgrad_same(x8, dz8, cin, cout, k, d):
@@ -112,22 +122,33 @@ class _ResFn(torch.autograd.Function):
     def backward(ctx, gy):
         x, y, a1, w1, b1, w2 = ctx.saved_tensors
         c, d = ctx.meta
-        w2_t = _bw_pack(w2, 'res1x1T', lambda: P.pack_res1x1(w2.detach().float().transpose(0, 1).contiguous()))
-        w1_t = _bw_pack(w1, 'res3x3T', lambda: P.pack_res3x3(w1.detach().float().transpose(0, 1).flip(2, 3).contiguous()))
+        need = ctx.needs_input_grad
         gy = gy.contiguous()
         dz2 = _as_c8(_ew('tt_res_out_bwd_bf16', gy, y, x))                       # gy * ELU'(z2), activated 1x1 output = y - x
-        x8 = _as_c8(x)
         a1 = _as_c8(a1)                                                          # the inner activation, as the forward staged it
-        dw2, db2 = _wgrad_same(a1, dz2, c, c, 1, 1)
+        dw1 = db1 = dw2 = db2 = gx = None
+        if need[3] or need[4]:
+            dw2, db2 = _wgrad_same(a1, dz2, c, c, 1, 1)
+        if not (need[0] or need[1] or need[2]):
+            return gx, dw1, db1, _needed(dw2, need[3]), _needed(db2, need[4]), None, None, None
+        w2_t = _bw_pack(w2, 'res1x1T', lambda: P.pack_res1x1(w2.detach().float().transpose(0, 1).contiguous()))
         dz1 = ops.conv_same(dz2, w2_t, None, 1, 1, times_elu_grad_of=a1)         # W2^T dz2, times ELU'(z1): one launch
-        dw1, db1 = _wgrad_same(x8, dz1, c, c, 3, d)
-        if gy.dim() == 5:
-            gx = ops.conv_same(dz1, w1_t, None, 3, d, plus=gy)                   # gx = gy + W1^T (*) dz1: the residual add in the epilogue
-        else:
-            gx = _to_layout_of(ops.conv_same(dz1, w1_t, None, 3, d), x)          # packed 4-channel stage: re-layout, then add
-            one = torch.ones((), dtype=torch.float32, device=gx.device)
-            _lib.check(_lib.lib().tt_add_scaled_bf16(_p(gy), _p(gx), _p(one.reshape(1)), _p(gx), gx.numel(), _s(gx)))
-        return gx, dw1, db1, dw2, db2, None, None, None
+        if need[1] or need[2]:
+            dw1, db1 = _wgrad_same(_as_c8(x), dz1, c, c, 3, d)
+        if need[0]:
+            w1_t = _bw_pack(w1, 'res3x3T', lambda: P.pack_res3x3(w1.detach().float().transpose(0, 1).flip(2, 3).contiguous()))
+            if gy.dim() == 5:
+                gx = ops.conv_same(dz1, w1_t, None, 3, d, plus=gy)               # gx = gy + W1^T (*) dz1: the residual add in the epilogue
+            else:
+                gx = _to_layout_of(ops.conv_same(dz1, w1_t, None, 3, d), x)      # packed 4-channel stage: re-layout, then add
+                one = torch.ones((), dtype=torch.float32, device=gx.device)
+                _lib.check(_lib.lib().tt_add_scaled_bf16(_p(gy), _p(gx), _p(one.reshape(1)), _p(gx), gx.numel(), _s(gx)))
+        return gx, _needed(dw1, need[1]), _needed(db1, need[2]), _needed(dw2, need[3]), _needed(db2, need[4]), None, None, None
+
+
+def _needed(g, flag):
+    """A gradient that one weight-gradient launch produced together with another: handed back only where autograd asked for it."""
+    return g if flag else None
 
 
 def _wgrad_updown(fine8, coarse8, cfine, ccoarse, transposed):
@@ -161,15 +182,17 @@ class _DownFn(torch.autograd.Function):
     def backward(ctx, gy):
         x, y, weight = ctx.saved_tensors
         cin, cout = ctx.meta
+        need = ctx.needs_input_grad
         dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)
         x8 = _as_c8(x)
-        dw, db = _wgrad_updown(x8, dz, cin, cout, False)
-        gx = None
-        if ctx.needs_input_grad[0]:
+        dw = db = gx = None
+        if need[1] or need[2]:
+            dw, db = _wgrad_updown(x8, dz, cin, cout, False)
+        if need[0]:
             hin, hout = x8.size(2), dz.size(2)
             wt = _bw_pack(weight, 'downT', lambda: P.pack_up_strip(weight.detach().float(), torch.zeros(cin, device=weight.device)))
             gx = ops.conv_up_strip(dz, wt, P.pad8(cin), hin - 2 * hout - 2, packed4_out=x.dim() == 4, act=False)
-        return gx, dw, db, None, None, None
+        return gx, _needed(dw, need[1]), _needed(db, need[2]), None, None, None
 
 
 class _UpFn(torch.autograd.Function):
@@ -187,13 +210,17 @@ class _UpFn(torch.autograd.Function):
     def backward(ctx, gy):
         x, y, weight = ctx.saved_tensors
         cin, cout = ctx.meta
+        need = ctx.needs_input_grad
         dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)                          # layout of y (packed 4-channel for the last stage)
-        dw, db = _wgrad_updown(_as_c8(dz), x, cout, cin, True)
-        # ConvTranspose2d (cin, cout, 4, 1) read as a Conv2d weight (out = cin, in = cout)
-        pack = P.pack_down_pairs if dz.dim() == 4 else P.pack_down_strip
-        wd = _bw_pack(weight, 'upT', lambda: pack(weight.detach().float().contiguous(), torch.zeros(cin, device=weight.device)))
-        gx = ops.conv_down_strip(dz, wd, P.pad8(cin), act=False)
-        return gx, dw, db, None, None, None
+        dw = db = gx = None
+        if need[1] or need[2]:
+            dw, db = _wgrad_updown(_as_c8(dz), x, cout, cin, True)
+        if need[0]:
+            # ConvTranspose2d (cin, cout, 4, 1) read as a Conv2d weight (out = cin, in = cout)
+            pack = P.pack_down_pairs if dz.dim() == 4 else P.pack_down_strip
+            wd = _bw_pack(weight, 'upT', lambda: pack(weight.detach().float().contiguous(), torch.zeros(cin, device=weight.device)))
+            gx = ops.conv_down_strip(dz, wd, P.pad8(cin), act=False)
+        return gx, _needed(dw, need[1]), _needed(db, need[2]), None, None, None
 
 
 _LAT_SCRATCH = {}
@@ -227,15 +254,19 @@ class _LatFn(torch.autograd.Function):
     def backward(ctx, gy):
         x, weight = ctx.saved_tensors
         c4, d, d_pad = ctx.meta
+        need = ctx.needs_input_grad
         gy = gy.contiguous()
-        dw = torch.zeros(weight.shape, dtype=torch.float32, device=x.device)
-        db = torch.zeros(d, dtype=torch.float32, device=x.device)
-        _wgrad_lat(x, gy, c4, d, dw, db, None)
-        # gx[ci, h, t] = sum_co W[co, ci, h] gy[co, t]: ConvTranspose2d with weight (in = co, out = ci, H, 1)
-        w, table = _bw_pack(weight, 'latT', lambda: P.pack_deconv_in_film(weight.detach().float(), torch.zeros(c4, device=x.device),
-                                                                          torch.ones(d, device=x.device), torch.zeros(d, device=x.device), d_pad))
-        gx = ops.deconv_in(gy, w, table, P.pad8(c4), x.size(2), act=False)
-        return gx, dw, db, None, None, None, None
+        dw = db = gx = None
+        if need[1] or need[2]:
+            dw = torch.zeros(weight.shape, dtype=torch.float32, device=x.device)
+            db = torch.zeros(d, dtype=torch.float32, device=x.device)
+            _wgrad_lat(x, gy, c4, d, dw, db, None)
+        if need[0]:
+            # gx[ci, h, t] = sum_co W[co, ci, h] gy[co, t]: ConvTranspose2d with weight (in = co, out = ci, H, 1)
+            w, table = _bw_pack(weight, 'latT', lambda: P.pack_deconv_in_film(weight.detach().float(), torch.zeros(c4, device=x.device),
+                                                                              torch.ones(d, device=x.device), torch.zeros(d, device=x.device), d_pad))
+            gx = ops.deconv_in(gy, w, table, P.pad8(c4), x.size(2), act=False)
+        return gx, _needed(dw, need[1]), _needed(db, need[2]), None, None, None, None
 
 
 def _pairs_to_c8(pairs):
@@ -273,16 +304,18 @@ class _InFn(torch.autograd.Function):
     def backward(ctx, gy):
         coeffs, y, weight = ctx.saved_tensors
         c0 = ctx.c0
+        need = ctx.needs_input_grad
         dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)
-        dw, db = _wgrad_same(_pairs_to_c8(coeffs), _as_c8(dz), 2, c0, 3, 1)
-        gx = None
-        if ctx.needs_input_grad[0]:
+        dw = db = gx = None
+        if need[1] or need[2]:
+            dw, db = _wgrad_same(_pairs_to_c8(coeffs), _as_c8(dz), 2, c0, 3, 1)
+            if weight.size(1) == 1:
+                dw = dw[:, :1]
+        if need[0]:
             wt, zb = _bw_pack(weight, 'inT', lambda: (_two_channels(weight.detach().float(), 1).transpose(0, 1).flip(2, 3).contiguous(),  # (2, c0, 3, 3)
                                                       torch.zeros(2, device=dz.device)))
             gx = ops.conv_out(dz, wt, zb, c0)
-        if weight.size(1) == 1:
-            dw = dw[:, :1]
-        return gx, dw, db, None, None
+        return gx, _needed(dw, need[1]), _needed(db, need[2]), None, None
 
 
 class _OutFn(torch.autograd.Function):
@@ -302,16 +335,20 @@ class _OutFn(torch.autograd.Function):
     def backward(ctx, gy):
         x, weight = ctx.saved_tensors
         c = ctx.c
+        need = ctx.needs_input_grad
         gy = gy.contiguous()
-        dw, db = _wgrad_same(_as_c8(x), _pairs_to_c8(gy), c, 2, 3, 1)
-        wt, zb = _bw_pack(weight, 'outT', lambda: (_two_channels(weight.detach().float(), 0).transpose(0, 1).flip(2, 3).contiguous(),  # (c, 2, 3, 3)
-                                                   torch.zeros(c, device=gy.device)))
-        B, F_, T, _ = gy.shape
-        gx = torch.empty((B, F_, T, 4), dtype=torch.bfloat16, device=gy.device)
-        _lib.check(_lib.lib().tt_conv_in(_p(gy), _p(gx), _p(wt), _p(zb), B, c, F_, T, 2, _s(gy)))
-        if weight.size(0) == 1:
-            dw, db = dw[:1], db[:1]
-        return gx, dw, db, None, None
+        dw = db = gx = None
+        if need[1] or need[2]:
+            dw, db = _wgrad_same(_as_c8(x), _pairs_to_c8(gy), c, 2, 3, 1)
+            if weight.size(0) == 1:
+                dw, db = dw[:1], db[:1]
+        if need[0]:
+            wt, zb = _bw_pack(weight, 'outT', lambda: (_two_channels(weight.detach().float(), 0).transpose(0, 1).flip(2, 3).contiguous(),  # (c, 2, 3, 3)
+                                                       torch.zeros(c, device=gy.device)))
+            B, F_, T, _ = gy.shape
+            gx = torch.empty((B, F_, T, 4), dtype=torch.bfloat16, device=gy.device)
+            _lib.check(_lib.lib().tt_conv_in(_p(gy), _p(gx), _p(wt), _p(zb), B, c, F_, T, 2, _s(gy)))
+        return gx, _needed(dw, need[1]), _needed(db, need[2]), None, None
 
 
 class _SkipAddFn(torch.autograd.Function):
@@ -331,11 +368,14 @@ class _SkipAddFn(torch.autograd.Function):
         e, scale = ctx.saved_tensors
         g = g.contiguous()
         lib = _lib.lib()
-        ge = torch.empty_like(g)
-        _lib.check(lib.tt_add_scaled_bf16(_p(g), _p(g), _p(scale - 1.0), _p(ge), g.numel(), _s(g)))        # g + (w - 1) g = w g
-        gw = torch.empty((), dtype=torch.float32, device=g.device)
-        scratch = torch.empty(int(lib.tt_dot_scratch_floats()), dtype=torch.float32, device=g.device)
-        _lib.check(lib.tt_dot_bf16(_p(g), _p(e), g.numel(), _p(gw), _p(scratch), _s(g)))
+        ge = gw = None
+        if ctx.needs_input_grad[1]:
+            ge = torch.empty_like(g)
+            _lib.check(lib.tt_add_scaled_bf16(_p(g), _p(g), _p(scale - 1.0), _p(ge), g.numel(), _s(g)))    # g + (w - 1) g = w g
+        if ctx.needs_input_grad[2]:
+            gw = torch.empty((), dtype=torch.float32, device=g.device)
+            scratch = torch.empty(int(lib.tt_dot_scratch_floats()), dtype=torch.float32, device=g.device)
+            _lib.check(lib.tt_dot_bf16(_p(g), _p(e), g.numel(), _p(gw), _p(scratch), _s(g)))
         return g, ge, gw
 
 
@@ -395,42 +435,6 @@ class _Channel0ActivationsFn(torch.autograd.Function):
         return _channel0_bwd(pairs, ops.widen(gact), ctx.mode), None
 
 
-class _SqDiffFn(torch.autograd.Function):
-    """compute_reconstruction_loss (objectives.py:11-33) on two interleaved coefficient tensors; gradients to both."""
-
-    @staticmethod
-    def forward(ctx, a, b):
-        ctx.save_for_backward(a, b)
-        return compute_reconstruction_loss(a.permute(0, 3, 1, 2), b.permute(0, 3, 1, 2))
-
-    @staticmethod
-    def backward(ctx, gout):
-        a, b = ctx.saved_tensors
-        scale = 1.0 / (a.size(0) * a.size(2))
-        ga = torch.empty_like(a) if ctx.needs_input_grad[0] else None
-        gb = torch.empty_like(b) if ctx.needs_input_grad[1] else None
-        _lib.check(_lib.lib().tt_sum_sq_diff_bwd(_p(a), _p(b), _p(gout.contiguous()), scale, _p(ga), _p(gb), a.numel(), _s(a)))
-        return ga, gb
-
-
-class _TrnLossFn(torch.autograd.Function):
-    """compute_transcription_loss(estimate, target, weight_positive_class=True) (objectives.py:36-74)."""
-
-    @staticmethod
-    def forward(ctx, est, tgt):
-        ctx.save_for_backward(est, tgt)
-        return compute_transcription_loss(est, tgt, True)
-
-    @staticmethod
-    def backward(ctx, gout):
-        est, tgt = ctx.saved_tensors
-        g = torch.empty_like(est)
-        B, F, T = est.shape
-        _lib.check(_lib.lib().tt_transcription_loss_bwd(_p(est), _p(tgt), _p(gout.contiguous()), B, F, T, 1, _p(g), _s(est)))
-        return g, None
-
-
-
 class _IndicatorFn(torch.autograd.Function):
     """
     Decoder.convin on latents + the constant indicator channel (modules.py:139-142, 533-536).  Forward: tt_deconv_in with the
@@ -449,19 +453,23 @@ class _IndicatorFn(torch.autograd.Function):
     def backward(ctx, gy):
         lat, y, weight = ctx.saved_tensors
         flag, d, c0 = ctx.meta
+        need = ctx.needs_input_grad
         # ELU derivative, tap-grouped tensor-core weight gradient (rows 0 .. D-1; the indicator row and the bias are row sums of dz),
         # data gradient = the Encoder.convlat forward kernel on the first D weight rows
         dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)
-        h0 = y.size(2)
-        dw = torch.zeros(weight.shape, dtype=torch.float32, device=lat.device)
-        rows = torch.zeros((c0, h0), dtype=torch.float32, device=lat.device)
-        _wgrad_lat(dz, lat, c0, d, dw, None, rows)
-        dw[d, :, :, 0] = flag * rows
-        db = rows.sum(dim=1)
-        d_pad = lat.size(1) * 8
-        wl, zl = _bw_pack(weight, 'decinT', lambda: (P.pack_lat(weight.detach().float()[:d], d_pad), torch.zeros(d_pad, device=lat.device)))
-        glat = ops.conv_lat(dz, wl, zl, d_pad)
-        return glat, dw, db, None, None, None, None
+        dw = db = glat = None
+        if need[1] or need[2]:
+            h0 = y.size(2)
+            dw = torch.zeros(weight.shape, dtype=torch.float32, device=lat.device)
+            rows = torch.zeros((c0, h0), dtype=torch.float32, device=lat.device)
+            _wgrad_lat(dz, lat, c0, d, dw, None, rows)
+            dw[d, :, :, 0] = flag * rows
+            db = rows.sum(dim=1)
+        if need[0]:
+            d_pad = lat.size(1) * 8
+            wl, zl = _bw_pack(weight, 'decinT', lambda: (P.pack_lat(weight.detach().float()[:d], d_pad), torch.zeros(d_pad, device=lat.device)))
+            glat = ops.conv_lat(dz, wl, zl, d_pad)
+        return glat, _needed(dw, need[1]), _needed(db, need[2]), None, None, None, None
 
 
 class _FiLMConvInFn(torch.autograd.Function):
@@ -484,30 +492,36 @@ class _FiLMConvInFn(torch.autograd.Function):
     def backward(ctx, gy):
         lat, y, weight, gamma_w, gamma_b, beta_w, beta_b = ctx.saved_tensors
         hot, d, c0 = ctx.meta
+        need = ctx.needs_input_grad
         dz = _ew('tt_elu_bwd_bf16', gy.contiguous(), y)
-        return _film_convin_grads(dz, lat, weight, gamma_w, gamma_b, beta_w, beta_b, hot, d, c0) + (None,) * 4
+        grads = _film_convin_grads(dz, lat, weight, gamma_w, gamma_b, beta_w, beta_b, hot, d, c0, params=any(need[1:7]), latents=need[0])
+        return tuple(_needed(g, n) for g, n in zip(grads, need[:7])) + (None,) * 4
 
 
-def _film_convin_grads(dz, lat, weight, gamma_w, gamma_b, beta_w, beta_b, hot, d, c0):
+def _film_convin_grads(dz, lat, weight, gamma_w, gamma_b, beta_w, beta_b, hot, d, c0, params=True, latents=True):
     """Gradients of _FiLMConvInFn from dz (C8 planar, after the ELU derivative) and the latents lat (C8 planar, H = 1):
-    (latents (bf16, C8), convin weight, convin bias, gamma.weight, gamma.bias, beta.weight, beta.bias)."""
+    (latents (bf16, C8), convin weight, convin bias, gamma.weight, gamma.bias, beta.weight, beta.bias); `params` / `latents` False:
+    the six parameter gradients (one weight-gradient and one FiLM launch) / the latent gradient are skipped and come back None."""
     h0 = dz.size(2)
     dev = lat.device
-    G = torch.zeros(weight.shape, dtype=torch.float32, device=dev)
-    rows = torch.zeros((c0, h0), dtype=torch.float32, device=dev)
-    _wgrad_lat(dz, lat, c0, d, G, None, rows)
-    dw = torch.empty_like(G)
-    db = torch.empty(c0, dtype=torch.float32, device=dev)
-    dgw, dbw = torch.empty_like(gamma_w), torch.empty_like(beta_w)
-    dgb, dbb = torch.empty_like(gamma_b), torch.empty_like(beta_b)
-    _lib.check(_lib.lib().tt_film_convin_grad(_p(G), _p(rows), _p(weight), _p(gamma_w), _p(gamma_b), _p(beta_w), _p(beta_b), d, c0, h0, hot,
-                                              _p(dw), _p(db), _p(dgw), _p(dgb), _p(dbw), _p(dbb), _s(G)))
-    d_pad = lat.size(1) * 8
+    dw = db = dgw = dgb = dbw = dbb = glat = None
+    if params:
+        G = torch.zeros(weight.shape, dtype=torch.float32, device=dev)
+        rows = torch.zeros((c0, h0), dtype=torch.float32, device=dev)
+        _wgrad_lat(dz, lat, c0, d, G, None, rows)
+        dw = torch.empty_like(G)
+        db = torch.empty(c0, dtype=torch.float32, device=dev)
+        dgw, dbw = torch.empty_like(gamma_w), torch.empty_like(beta_w)
+        dgb, dbb = torch.empty_like(gamma_b), torch.empty_like(beta_b)
+        _lib.check(_lib.lib().tt_film_convin_grad(_p(G), _p(rows), _p(weight), _p(gamma_w), _p(gamma_b), _p(beta_w), _p(beta_b), d, c0, h0, hot,
+                                                  _p(dw), _p(db), _p(dgw), _p(dgb), _p(dbw), _p(dbb), _s(G)))
+    if latents:
+        d_pad = lat.size(1) * 8
 
-    def build():
-        gamma = gamma_w.detach()[:, hot] + gamma_b.detach()                          # film_layer.gamma(one-hot cond)
-        return P.pack_lat(weight.detach().float() * gamma.view(-1, 1, 1, 1), d_pad), torch.zeros(d_pad, device=dev)
-    # gamma differs between the two passes and depends on the FiLM parameters, so they are part of the key
-    wl, zl = _bw_pack(weight, ('filmT', hot, gamma_w.data_ptr(), gamma_w._version, gamma_b.data_ptr(), gamma_b._version), build)
-    glat = ops.conv_lat(dz, wl, zl, d_pad)
+        def build():
+            gamma = gamma_w.detach()[:, hot] + gamma_b.detach()                          # film_layer.gamma(one-hot cond)
+            return P.pack_lat(weight.detach().float() * gamma.view(-1, 1, 1, 1), d_pad), torch.zeros(d_pad, device=dev)
+        # gamma differs between the two passes (the tag) and depends on the FiLM parameters (rebuilt when they change)
+        wl, zl = _bw_pack(weight, ('filmT', hot), build, deps=(gamma_w, gamma_b))
+        glat = ops.conv_lat(dz, wl, zl, d_pad)
     return glat, dw, db, dgw, dgb, dbw, dbb

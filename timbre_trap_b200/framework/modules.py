@@ -19,7 +19,8 @@ from .. import _lib
 from . import ops
 from . import packing as P
 from .cqt import CQT
-from .layer_grads import _DownFn, _FiLMConvInFn, _HeadFn, _IndicatorFn, _InFn, _LatFn, _OutFn, _ResFn, _SkipAddFn, _UpFn
+from .layer_grads import (_ActivationsFn, _Channel0ActivationsFn, _DownFn, _FiLMConvInFn, _HeadFn, _IndicatorFn, _InFn, _LatFn, _OutFn, _ResFn,
+                          _SkipAddFn, _UpFn)
 from .packing import _PackedCache       # also the name under which pickled modules refer to it
 
 __all__ = ['TimbreTrap', 'TimbreTrapFiLM', 'FiLM', 'TimbreTrapMag', 'TimbreTrapMagDB', 'Encoder', 'Decoder', 'EncoderBlock', 'DecoderBlock',
@@ -391,6 +392,12 @@ def _interleave(coefficients):
     return c if c.is_contiguous() else c.contiguous()
 
 
+def _no_autocast():
+    """The model's own code runs outside autocast: the ATen pieces that build the packed weights (FiLM's nn.Linear, the skip-weight
+    products, re-layouts) would otherwise store autocast-dependent values in caches whose keys do not record the autocast state."""
+    return torch.autocast('cuda', enabled=False)
+
+
 def _unit_skips(embeddings_internal):
     """Already-weighted embeddings (the API form of Decoder.forward / TimbreTrap.decode) as (weight 1, embedding) pairs."""
     one = torch.ones((), dtype=torch.float32, device=embeddings_internal[0].device)
@@ -405,10 +412,10 @@ def _latent_pad(latent_size):
     raise ValueError(f'latent_size {latent_size} is not supported (at most 256)')
 
 
-def _latents_to_c8(latents, latent_pad):
-    """(B, D, T) -> C8 planar (B, Dp/8, 1, T, 8) bf16."""
+def _latents_to_c8(latents, latent_pad, grad=False):
+    """(B, D, T) -> C8 planar (B, Dp/8, 1, T, 8) bf16.  `grad`: the re-layout stays on the autograd graph of `latents`."""
     B, D, T = latents.shape
-    x = latents.detach().float()
+    x = latents.float() if grad else latents.detach().float()
     if D != latent_pad:
         x = torch.nn.functional.pad(x, (0, 0, 0, latent_pad - D))
     return x.reshape(B, latent_pad // 8, 8, 1, T).permute(0, 1, 3, 4, 2).contiguous().to(torch.bfloat16)
@@ -502,10 +509,18 @@ class TimbreTrap(nn.Module):
     HEAD_MODE = None
     ACTIVATIONS_MODE = None
 
-    def _head(self, pairs):
-        """decoder output (B, F, T, 2) interleaved -> what `decode` returns: (B, 2, F, T) view, or (B, 1, F, T) for the magnitude variants."""
+    def _graph(self):
+        """Whether forward / encode / decode build an autograd graph: in train mode with grad mode on.  In eval mode or under no_grad
+        they run the inference path (the same launches, buffer reuse and outputs, no graph)."""
+        return self.training and torch.is_grad_enabled()
+
+    def _head(self, pairs, grad=False):
+        """decoder output (B, F, T, 2) interleaved -> what `decode` returns: (B, 2, F, T) view, or (B, 1, F, T) for the magnitude variants.
+        `grad`: the head through its autograd Function."""
         if self.HEAD_MODE is None:
             return pairs.permute(0, 3, 1, 2)
+        if grad:
+            return _Channel0ActivationsFn.apply(pairs, self.HEAD_MODE).unsqueeze(1)
         return ops.channel0(pairs, self.HEAD_MODE).unsqueeze(1)
 
     def _codes(self, audio):
@@ -528,18 +543,24 @@ class TimbreTrap(nn.Module):
             outs.append(y)
         return outs[0], outs[1], lat
 
-    def _output(self, pairs):
-        """A decoder output of _passes -> what `forward` returns: (B, 2, F, T) view, or (B, 1, F, T) for the magnitude variants."""
+    def _output(self, pairs, grad=False):
+        """A decoder output of _passes -> what `forward` returns: (B, 2, F, T) view, or (B, 1, F, T) for the magnitude variants.
+        `grad`: channel 0 through its autograd Function."""
         if self.HEAD_MODE is None:
             return pairs.permute(0, 3, 1, 2)
+        if grad:
+            return _Channel0ActivationsFn.apply(pairs, 0).unsqueeze(1)
         return ops.channel0(pairs, 0).unsqueeze(1)          # mode 0: channel 0 as it is
 
     # ---- reference API -------------------------------------------------------------------------------
     def encode(self, audio):
-        """modules.py:67-93."""
+        """modules.py:67-93: audio (B, 1, N) -> (latents (B, D, T), embeddings [(B, C, H, T)], {}).  In train mode with grad mode on the
+        result carries an autograd graph to the encoder's parameters (none to the audio: the CQT has no backward, as in the reference);
+        in eval mode or under no_grad it is inference."""
         _lib.require_cuda(audio, 'audio')
-        with torch.no_grad():
-            lat, emb = self.encoder.forward_c8(self._features(audio))
+        grad = self._graph()
+        with _no_autocast(), torch.set_grad_enabled(grad):
+            lat, emb = self.encoder.forward_c8(self._features(audio), grad=grad)
             latents = P.from_c8(lat, self.encoder.latent_size).squeeze(-2)
             embeddings = [P.from_p4(e, c) if e.dim() == 4 else P.from_c8(e, c) for e, c in zip(emb, self.encoder.channels)]
         return latents, embeddings, dict()
@@ -551,12 +572,15 @@ class TimbreTrap(nn.Module):
         return None
 
     def decode(self, latents, embeddings=None, transcribe=False):
-        """modules.py:119-147: latents (B, D, T) -> logits (B, 2, F, T)."""
+        """modules.py:119-147: latents (B, D, T) -> logits (B, 2, F, T) ((B, 1, F, T) for the magnitude variants).  In train mode with
+        grad mode on the result carries an autograd graph to the decoder's parameters and to `latents` and `embeddings` where they
+        require grad; in eval mode or under no_grad it is inference."""
         _lib.require_cuda(latents, 'latents')
-        with torch.no_grad():
-            lat = _latents_to_c8(latents, self.decoder.latent_pad)
+        grad = self._graph()
+        with _no_autocast(), torch.set_grad_enabled(grad):
+            lat = _latents_to_c8(latents, self.decoder.latent_pad, grad=grad)
             skips = None if embeddings is None else _unit_skips(self.decoder._embeddings_internal(embeddings))
-            return self._head(self.decoder.forward_c8(lat, not transcribe, skips))
+            return self._head(self.decoder.forward_c8(lat, not transcribe, skips, grad=grad), grad)
 
     def _inference(self, audio, transcribe=False):
         """modules.py:149-177."""
@@ -689,7 +713,15 @@ class TimbreTrap(nn.Module):
         return (trn if transcribe else rec).permute(0, 3, 1, 2)
 
     def to_activations(self, coefficients):
-        """modules.py:271-289."""
+        """modules.py:271-289: tanh|c| of (B, 2, F, T) coefficients -> (B, F, T).  Differentiable (tt_activations_bwd) when grad mode is on
+        and the coefficients require grad: `forward`'s outputs are views of interleaved pairs and go in as they are, other tensors are
+        copied into pairs first."""
+        if torch.is_grad_enabled() and coefficients.requires_grad:
+            _lib.require_cuda(coefficients, 'coefficients')
+            pairs = coefficients.permute(0, 2, 3, 1)
+            if pairs.dtype != torch.float32 or not pairs.is_contiguous():
+                pairs = pairs.float().contiguous()
+            return _ActivationsFn.apply(pairs)
         return CQT._magnitude(coefficients, True)
 
     def transcribe(self, audio):
@@ -783,15 +815,22 @@ class TimbreTrap(nn.Module):
         return _gather_frames(act, -1, M, audio, L, group, world), _gather_frames(wav, -1, L, audio, L, group, world)
 
     def forward(self, audio, consistency=False):
-        """modules.py:338-393 (inference semantics; the training step with gradients is framework.train.TrainStep)."""
-        with torch.no_grad():
-            rec, trn, lat = self._passes(self._features(audio))
+        """modules.py:338-393: audio (B, 1, N) -> (reconstruction, latents, transcription, transcription_rec, transcription_scr, {}), the
+        last two None unless `consistency` (a bool or an int, as experiments/train.py passes it).
+
+        In train mode with grad mode on, every layer runs through its autograd Function (framework/layer_grads.py) and the outputs carry
+        the graph: the reference's loop body (`model(audio, consistency=True)`, `to_activations`, the objectives, `backward()`) trains
+        the model.  The coefficient outputs are views of the internal interleaved pairs.  In eval mode or under no_grad this is inference:
+        no graph, buffers reused.  Either way the model runs outside autocast (see _no_autocast)."""
+        grad = self._graph()
+        with _no_autocast(), torch.set_grad_enabled(grad):
+            rec, trn, lat = self._passes(self._features(audio), grad)
             trn_rec = trn_scr = None
             if consistency:
-                trn_rec, trn_scr, _ = self._passes(trn)
-                trn_rec, trn_scr = self._output(trn_rec), self._output(trn_scr)
+                trn_rec, trn_scr, _ = self._passes(trn, grad)
+                trn_rec, trn_scr = self._output(trn_rec, grad), self._output(trn_scr, grad)
             latents = P.from_c8(lat, self.encoder.latent_size).squeeze(-2)
-            return self._output(rec), latents, self._output(trn), trn_rec, trn_scr, dict()
+            return self._output(rec, grad), latents, self._output(trn, grad), trn_rec, trn_scr, dict()
 
     # ---- full-track forward in time tiles (experiments/evaluate.py:81-95 feeds whole tracks through model(audio)) -------------------
     # Only the convolutions see across frames, and only +-1 frame (convin / convout) and +-6 frames per block of three dilated
@@ -877,10 +916,11 @@ class TimbreTrapMag(TimbreTrap):
         return ops.widen(CQT._magnitude(self.sliCQ.encode_interleaved(audio).permute(0, 3, 1, 2), False))
 
     def to_activations(self, coefficients):
-        """modules.py:980-1001: tanh of the (B, 1, F, T) magnitude coefficients -> (B, F, T).  Like the reference's `squeeze(-3)`, a
-        two-channel tensor (what the inherited chunk loop produces for this variant) keeps its channel axis."""
+        """modules.py:980-1001: tanh of the (B, 1, F, T) magnitude coefficients -> (B, F, T), differentiable when grad mode is on and the
+        coefficients require grad.  Like the reference's `squeeze(-3)`, a two-channel tensor (what the inherited chunk loop produces for
+        this variant) keeps its channel axis."""
         _lib.require_cuda(coefficients, 'coefficients')
-        return torch.tanh(coefficients.detach().float().squeeze(-3))
+        return torch.tanh(coefficients.float().squeeze(-3))
 
 
 class TimbreTrapMagDB(TimbreTrapMag):
@@ -895,5 +935,5 @@ class TimbreTrapMagDB(TimbreTrapMag):
         return ops.widen(CQT.to_decibels(mag))
 
     def to_activations(self, coefficients):
-        """modules.py:1056-1075."""
+        """modules.py:1056-1075: the sigmoid output as it is (a view; gradients pass straight through)."""
         return coefficients.squeeze(-3)

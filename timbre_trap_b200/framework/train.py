@@ -10,6 +10,8 @@ The forward is the model's own (TimbreTrap._passes); with gradients every layer 
 inference kernel and whose backward stays in the bf16 inference layouts (framework/layer_grads.py); clip and AdamW have kernels of
 their own (csrc/train_kernels.cu).  PyTorch's autograd engine only walks the graph and accumulates `.grad`; there is no cuDNN / ATen
 compute on the path.
+The reference's own loop body on the public API (model.train(), model(audio, consistency=True), to_activations, the compute_*_loss
+functions, backward(), any torch optimizer) runs the same Functions; see INTEGRATION.md section 4.
 Differences to the reference that do not change values: the CQT target is computed once (the reference computes it twice,
 train.py:404 and modules.py:366 -> :88); no `.item()` host syncs inside the step; activation gradients travel in bf16 between
 layers (the reference runs the forward under fp16 autocast).
@@ -19,7 +21,8 @@ import torch
 
 from .. import _lib
 from . import packing as P  # noqa: F401
-from .layer_grads import _ActivationsFn, _Channel0ActivationsFn, _p, _s, _SqDiffFn, _TrnLossFn
+from .layer_grads import _ActivationsFn, _Channel0ActivationsFn, _p, _s
+from .objectives import _sum_sq_diff, _TrnLossFn
 # the weight-gradient and edge-kernel wrappers, where code written against the earlier layout of this module reaches them
 from .layer_grads import _channel0_bwd, _film_convin_grads, _wgrad_lat, _wgrad_same, _wgrad_updown  # noqa: F401
 from .packing import _PackedCache
@@ -36,13 +39,15 @@ def _step_losses(model, audio, ground_truth, mult, late_start, grad):
     mode = model.ACTIVATIONS_MODE
     act = _ActivationsFn.apply(trn) if mode is None else _Channel0ActivationsFn.apply(trn, mode)
     n = ground_truth.size(0)
-    out = dict(reconstruction=_SqDiffFn.apply(rec, coeffs), transcription=_TrnLossFn.apply(act[:n].contiguous(), ground_truth.float().contiguous()))
+    frames = rec.size(0) * rec.size(2)
+    out = dict(reconstruction=_sum_sq_diff(rec, coeffs, frames),
+               transcription=_TrnLossFn.apply(act[:n].contiguous(), ground_truth.float().contiguous(), True))
     total = mult['reconstruction'] * out['reconstruction']
     if mult['consistency']:
         trn_rec, trn_scr, _ = model._passes(trn, grad)
         tgt = trn[:n].contiguous()
-        out['consistency_spectral'] = _SqDiffFn.apply(trn_rec[:n].contiguous(), tgt)
-        out['consistency_score'] = _SqDiffFn.apply(trn_scr[:n].contiguous(), tgt)
+        out['consistency_spectral'] = _sum_sq_diff(trn_rec[:n].contiguous(), tgt, n * tgt.size(2))
+        out['consistency_score'] = _sum_sq_diff(trn_scr[:n].contiguous(), tgt, n * tgt.size(2))
     if not late_start:
         total = total + mult['transcription'] * out['transcription']
         if mult['consistency']:
