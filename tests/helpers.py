@@ -26,6 +26,35 @@ def rel_err(a, b):
     return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-300)), float(np.linalg.norm(a - b) / max(np.linalg.norm(b), 1e-300))
 
 
+def check_step_gradients(got, want, tag, floorless=None):
+    """Each parameter: err <= 0.1 |g| + 0.01 |g_total| (the floor for the tiny bias vectors, whose bf16 noise does not shrink with
+    them), and the global gradient at rel-L2 <= 3e-2.  `floorless`: also err <= floorless * |g| WITHOUT the floor for every parameter
+    whose gradient norm is at least 1e-3 of the total - the floor would let a wrong small layer, bias or skip weight through."""
+    assert set(got) == set(want)
+    total_norm = sum(float(v.norm()) ** 2 for v in want.values()) ** 0.5
+    num = den = 0.0
+    worst = worst_gated = (0.0, None)
+    failed = []
+    for k in want:
+        assert got[k].shape == want[k].shape, k
+        err, ref = float((got[k] - want[k]).norm()), float(want[k].norm())
+        num += err ** 2
+        den += ref ** 2
+        rel = err / max(ref, 1e-12)
+        if rel > worst[0]:
+            worst = (rel, k)
+        if err > 1e-1 * ref + 1e-2 * total_norm:
+            failed.append((k, err, ref, total_norm))
+        if floorless is not None and ref >= 1e-3 * total_norm:
+            if rel > worst_gated[0]:
+                worst_gated = (rel, k)
+            if rel > floorless:
+                failed.append((k, 'floorless', rel, ref / total_norm))
+    print(f'{tag}: global gradient rel-L2 error', (num / den) ** 0.5, 'worst parameter', worst, 'worst of the floorless gate', worst_gated)
+    assert not failed, failed
+    assert (num / den) ** 0.5 <= 3e-2, ((num / den) ** 0.5, worst)
+
+
 def tonal_clip_with_pitches(n_samples, sample_rate, seed):
     """As tonal_clip (one item) but also returns the MIDI pitches of the four fundamentals."""
     rng = np.random.default_rng(seed)

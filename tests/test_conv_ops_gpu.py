@@ -28,23 +28,32 @@ def force_strip_rows():
     _lib.lib().tt_set_strip_rows(0)
 
 
+def _rows(rows, linear):
+    """Parameter rows of a conv with its ELU epilogue (act=True, ids as they were) and `linear` rows of the same conv without it
+    (act=False: the linear epilogue the backward pass runs its data gradients through)."""
+    return ([pytest.param(*r, True, id='-'.join(map(str, r))) for r in rows] +
+            [pytest.param(*r, False, id='-'.join(map(str, r)) + '-linear') for r in linear])
+
+
 def _assert_close(got, want, tol=1.2e-2):
     err = float((got - want).abs().max())
     ref = float(want.abs().max())
     assert err <= tol * ref, (err, ref)
 
 
-@pytest.mark.parametrize('Cin,Cout,H,T,B', [(4, 8, 540, 128, 1), (8, 16, 269, 256, 2), (16, 32, 133, 128, 1), (32, 64, 65, 256, 2),
-                                              (2, 4, 20, 100, 1), (8, 16, 7, 128, 1)])
+@pytest.mark.parametrize('Cin,Cout,H,T,B,act', _rows([(4, 8, 540, 128, 1), (8, 16, 269, 256, 2), (16, 32, 133, 128, 1), (32, 64, 65, 256, 2),
+                                                    (2, 4, 20, 100, 1), (8, 16, 7, 128, 1)],
+                                                   [(32, 64, 65, 1024, 1), (16, 32, 133, 256, 2), (8, 16, 269, 128, 1), (4, 8, 540, 1024, 1)]))
 @pytest.mark.parametrize('strip_rows', [None, 5])
-def test_conv_down_strip(Cin, Cout, H, T, B, strip_rows, force_strip_rows):
+def test_conv_down_strip(Cin, Cout, H, T, B, act, strip_rows, force_strip_rows):
     from timbre_trap_b200.framework import ops, packing as P
     if strip_rows:
         force_strip_rows(strip_rows)
     x = _bf(_rand((B, Cin, H, T), 11))
     w, b = _bf(_rand((Cout, Cin, 4, 1), 12, 0.3)), _rand((Cout,), 13, 0.3)
-    want = F.elu(F.conv2d(x, w, b, stride=(2, 1)))
-    y = ops.conv_down_strip(P.to_c8(x.cuda()), P.pack_down_strip(w.cuda(), b.cuda()), P.pad8(Cout))
+    want = F.conv2d(x, w, b, stride=(2, 1))
+    want = F.elu(want) if act else want
+    y = ops.conv_down_strip(P.to_c8(x.cuda()), P.pack_down_strip(w.cuda(), b.cuda()), P.pad8(Cout), act=act)
     assert y.shape[2] == want.shape[2]
     _assert_close(P.from_c8(y, Cout).cpu(), want)
 
@@ -88,50 +97,69 @@ def test_conv_in_out_packed4():
     _assert_close(yo.permute(0, 3, 1, 2).cpu(), F.conv2d(xo, wo, bo, padding=1), tol=1e-5)
 
 
-@pytest.mark.parametrize('Cin,Cout,H,T,op,B', [(64, 32, 31, 128, 1, 2), (32, 16, 65, 256, 1, 1), (16, 8, 133, 128, 1, 2),
-                                                 (8, 4, 269, 256, 0, 1), (4, 2, 9, 100, 1, 1), (16, 8, 5, 128, 0, 1)])
+@pytest.mark.parametrize('Cin,Cout,H,T,op,B,act', _rows([(64, 32, 31, 128, 1, 2), (32, 16, 65, 256, 1, 1), (16, 8, 133, 128, 1, 2),
+                                                       (8, 4, 269, 256, 0, 1), (4, 2, 9, 100, 1, 1), (16, 8, 5, 128, 0, 1)],
+                                                      [(8, 4, 269, 1024, 0, 1), (16, 8, 133, 256, 1, 2), (32, 16, 65, 1024, 1, 1),
+                                                       (64, 32, 31, 128, 1, 2)]))
 @pytest.mark.parametrize('strip_rows', [None, 3])
-def test_conv_up_strip(Cin, Cout, H, T, op, B, strip_rows, force_strip_rows):
+def test_conv_up_strip(Cin, Cout, H, T, op, B, act, strip_rows, force_strip_rows):
     from timbre_trap_b200.framework import ops, packing as P
     if strip_rows:
         force_strip_rows(strip_rows)
     x = _bf(_rand((B, Cin, H, T), 21))
     w, b = _bf(_rand((Cin, Cout, 4, 1), 22, 0.3)), _rand((Cout,), 23, 0.3)
-    want = F.elu(F.conv_transpose2d(x, w, b, stride=(2, 1), output_padding=(op, 0)))
-    y = ops.conv_up_strip(P.to_c8(x.cuda()), P.pack_up_strip(w.cuda(), b.cuda()), P.pad8(Cout), op)
+    want = F.conv_transpose2d(x, w, b, stride=(2, 1), output_padding=(op, 0))
+    want = F.elu(want) if act else want
+    y = ops.conv_up_strip(P.to_c8(x.cuda()), P.pack_up_strip(w.cuda(), b.cuda()), P.pad8(Cout), op, act=act)
     assert y.shape[2] == want.shape[2]
     _assert_close(P.from_c8(y, Cout).cpu(), want)
 
 
-@pytest.mark.parametrize('C4,H4,D,T,B', [(64, 31, 128, 256, 2), (32, 2, 32, 128, 1), (64, 2, 24, 100, 2)])
-def test_conv_lat_and_deconv_in(C4, H4, D, T, B):
+@pytest.mark.parametrize('C4,H4,D,T,B,act', _rows([(64, 31, 128, 256, 2), (32, 2, 32, 128, 1), (64, 2, 24, 100, 2), (64, 31, 240, 256, 1)],
+                                                  [(64, 31, 128, 1024, 1), (32, 31, 32, 256, 2), (64, 2, 24, 100, 2)]))
+def test_conv_lat_and_deconv_in(C4, H4, D, T, B, act):
+    """act=False: deconv_in's linear epilogue, the data gradient of Encoder.convlat in the loss step."""
     from timbre_trap_b200.framework import ops, packing as P
-    Dp = (D + 15) // 16 * 16
+    from timbre_trap_b200.framework.modules import _latent_pad
+    Dp = _latent_pad(D)
     x = _bf(_rand((B, C4, H4, T), 31))
     w, b = _bf(_rand((D, C4, H4, 1), 32, 0.05)), _rand((D,), 33, 0.3)
     want = F.conv2d(x, w, b)
     lat = ops.conv_lat(P.to_c8(x.cuda()), P.pack_lat(w.cuda(), Dp), P.pad_vec(b.cuda(), Dp), Dp)
     _assert_close(P.from_c8(lat, D).cpu(), want)
+    if Dp > D:                                                          # padded latent channels: zero weights, zero bias
+        assert float(lat.float().permute(0, 1, 4, 2, 3).reshape(B, Dp, T)[:, D:].abs().max()) == 0.0
     # decoder side
     wd, bd = _bf(_rand((D + 1, C4, H4, 1), 34, 0.1)), _rand((C4,), 35, 0.3)
     lat_in = _bf(_rand((B, D, 1, T), 36))
     packed, tables = P.pack_deconv_in(wd.cuda(), bd.cuda(), Dp)
     for mode, flag in ((0, 0.0), (1, 1.0)):
         full = torch.cat((lat_in, torch.full((B, 1, 1, T), flag)), dim=1)
-        wantd = F.elu(F.conv_transpose2d(full, wd, bd))
+        wantd = F.conv_transpose2d(full, wd, bd)
+        wantd = F.elu(wantd) if act else wantd
         y = ops.deconv_in(P.to_c8(lat_in.cuda()) if Dp == P.pad8(D) else P.to_c8(F.pad(lat_in, (0, 0, 0, 0, 0, Dp - D)).cuda()),
-                          packed, tables[mode].contiguous(), P.pad8(C4), H4)
+                          packed, tables[mode].contiguous(), P.pad8(C4), H4, act=act)
         _assert_close(P.from_c8(y, C4).cpu(), wantd)
 
 
-@pytest.mark.parametrize('C0,H,T,B', [(4, 60, 300, 2), (2, 33, 128, 1), (8, 17, 64, 1), (4, 5, 1024, 1), (3, 9, 516, 2)])
-def test_conv_in_out(C0, H, T, B):
+@pytest.mark.parametrize('C0,H,T,B,packed4', [pytest.param(*r, 0, id='-'.join(map(str, r)))
+                                               for r in [(4, 60, 300, 2), (2, 33, 128, 1), (8, 17, 64, 1), (4, 5, 1024, 1), (3, 9, 516, 2)]] +
+                                              [pytest.param(*r, 2, id='-'.join(map(str, r)) + '-packed-linear')
+                                               for r in [(4, 540, 1024, 1), (2, 72, 200, 2), (3, 9, 516, 2)]])
+def test_conv_in_out(C0, H, T, B, packed4):
+    """packed4=2: packed 4-channel output without the ELU, the data gradient of Decoder.convout in the loss step."""
     from timbre_trap_b200.framework import ops, packing as P
     x = _rand((B, 2, H, T), 41)
     w, b = _rand((C0, 2, 3, 3), 42, 0.4), _rand((C0,), 43, 0.3)
-    want = F.elu(F.conv2d(x, w, b, padding=1))
-    y = ops.conv_in(x.permute(0, 2, 3, 1).contiguous().cuda(), w.cuda().contiguous(), b.cuda(), C0)
-    _assert_close(P.from_c8(y, C0).cpu(), want)
+    want = F.conv2d(x, w, b, padding=1)
+    y = ops.conv_in(x.permute(0, 2, 3, 1).contiguous().cuda(), w.cuda().contiguous(), b.cuda(), C0, packed4=packed4)
+    if packed4:
+        assert y.shape == (B, H, T, 4)
+        _assert_close(P.from_p4(y, C0).cpu(), want)
+        if C0 < 4:
+            assert float(y[..., C0:].float().abs().max()) == 0.0
+    else:
+        _assert_close(P.from_c8(y, C0).cpu(), F.elu(want))
     xo = _bf(_rand((B, C0, H, T), 44))
     wo, bo = _rand((2, C0, 3, 3), 45, 0.4), _rand((2,), 46, 0.3)
     wanto = F.conv2d(xo, wo, bo, padding=1)

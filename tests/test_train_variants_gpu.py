@@ -12,28 +12,33 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from tests.helpers import tonal_clip
+from tests.helpers import check_step_gradients, tonal_clip
 
 pytestmark = pytest.mark.gpu
 
 SMALL = dict(sample_rate=8000, n_octaves=6, bins_per_octave=12, secs_per_block=0.5)
+BASE = dict(sample_rate=22050, n_octaves=9, bins_per_octave=60, secs_per_block=3)
+GEOMETRY = dict(small=SMALL, base=BASE)
 CLASSES = dict(base='TimbreTrap', film='TimbreTrapFiLM', mag='TimbreTrapMag', magdb='TimbreTrapMagDB')
 
 
-def _setup(tag, skip=False, latent=None):
+def _setup(tag, skip=False, latent=None, complexity=1, geometry='small'):
+    """SMALL: two blocks of three clips, two of them with transcription targets; BASE: one 3 s block of one clip."""
     from oracle import model_ref as R
     from timbre_trap_b200 import framework as FW
-    model = getattr(FW, CLASSES[tag])(latent_size=latent, model_complexity=1, skip_connections=skip, **SMALL)
-    sd = R.init_state_dict(model.sliCQ.n_bins, latent, 1, seed=3, variant=tag)
+    geo = GEOMETRY[geometry]
+    model = getattr(FW, CLASSES[tag])(latent_size=latent, model_complexity=complexity, skip_connections=skip, **geo)
+    sd = R.init_state_dict(model.sliCQ.n_bins, latent, complexity, seed=3, variant=tag)
     if skip:
         sd['skip_weights'] = torch.tensor([0.9, 1.1, 0.8, 1.2, 0.7])
     model.load_state_dict(sd)
     model = model.cuda()
-    c = R.CQTRef(SMALL['n_octaves'], SMALL['bins_per_octave'], SMALL['sample_rate'], SMALL['secs_per_block'])
-    audio = tonal_clip(2 * c.block_length, SMALL['sample_rate'], seed=4, n_batch=3)
+    c = R.CQTRef(geo['n_octaves'], geo['bins_per_octave'], geo['sample_rate'], geo['secs_per_block'])
+    n_blocks, n_batch, n_gt = (1, 1, 1) if geometry == 'base' else (2, 3, 2)
+    audio = tonal_clip(n_blocks * c.block_length, geo['sample_rate'], seed=4, n_batch=n_batch)
     rng = np.random.default_rng(2)
-    gt = torch.zeros((2, c.n_bins, 2 * c.max_window_length))
-    for b in range(2):
+    gt = torch.zeros((n_gt, c.n_bins, n_blocks * c.max_window_length))
+    for b in range(n_gt):
         for k in rng.integers(5, c.n_bins - 5, size=3):
             gt[b, k, :] = 1.0
             gt[b, k - 1, :] = gt[b, k + 1, :] = 0.6
@@ -44,8 +49,9 @@ def _oracle_losses(R, tag, sd, c, audio, gt):
     rec, lat, trn, trn_rec, trn_scr = R.forward_variant_ref(tag, audio, sd, c, consistency=True)
     act = R.activations_variant_ref(tag, trn)
     losses = dict(reconstruction=R.reconstruction_loss_ref(rec, R.features_ref(tag, audio, c)),
-                  transcription=R.transcription_loss_ref(act[:2], gt, True))
-    losses['consistency_spectral'], losses['consistency_score'] = R.consistency_loss_ref(trn_rec[:2], trn_scr[:2], trn[:2])
+                  transcription=R.transcription_loss_ref(act[:gt.size(0)], gt, True))
+    n = gt.size(0)                                  # the first n clips have transcription targets
+    losses['consistency_spectral'], losses['consistency_score'] = R.consistency_loss_ref(trn_rec[:n], trn_scr[:n], trn[:n])
     return losses
 
 
@@ -81,10 +87,17 @@ def _global_err(got, want):
 CASES = [('film', True, 24), ('film', False, 200), ('mag', False, None), ('magdb', True, None)]
 
 
-@pytest.mark.parametrize('tag,skip,latent', CASES)
-def test_variant_step_gradients_match_oracle_autograd(tag, skip, latent):
+# model_complexity 2 (SMALL geometry): FiLM at latent 128, and MagDB with skips
+STEP_CASES = [pytest.param(*case, 1, 'small', id='-'.join(map(str, case))) for case in CASES] + [
+    pytest.param('film', False, 128, 2, 'small', id='film-False-128-complexity2-small'),
+    pytest.param('magdb', True, None, 2, 'small', id='magdb-True-None-complexity2-small')]
+FLOORLESS = 4e-2       # per-parameter rel-L2 without the floor, complexity 2 (measured on a B200: 2.1e-2 FiLM, 1.1e-2 MagDB)
+
+
+@pytest.mark.parametrize('tag,skip,latent,complexity,geometry', STEP_CASES)
+def test_variant_step_gradients_match_oracle_autograd(tag, skip, latent, complexity, geometry):
     from timbre_trap_b200.framework.train import TrainStep
-    R, model, sd, c, audio, gt = _setup(tag, skip, latent)
+    R, model, sd, c, audio, gt = _setup(tag, skip, latent, complexity, geometry)
     want, want_total = _oracle_grads(R, tag, sd, c, audio, gt)
     masks = None
     if tag == 'mag':
@@ -100,22 +113,10 @@ def test_variant_step_gradients_match_oracle_autograd(tag, skip, latent):
         print(f'{tag}: global gradient rel-L2 error against the plain oracle', _global_err(got, want))
         with _oracle_relu_decisions(masks):
             want, _ = _oracle_grads(R, tag, sd, c, audio, gt)
-    assert set(got) == set(want)
     if tag == 'film':
         assert {'film_layer.gamma.weight', 'film_layer.gamma.bias', 'film_layer.beta.weight', 'film_layer.beta.bias'} <= set(got)
-    total_norm = sum(float(v.norm()) ** 2 for v in want.values()) ** 0.5
-    num = den = 0.0
-    worst = (0.0, None)
-    for k in want:
-        assert got[k].shape == want[k].shape, k
-        err, ref = float((got[k] - want[k]).norm()), float(want[k].norm())
-        num += err ** 2
-        den += ref ** 2
-        if err / max(ref, 1e-12) > worst[0]:
-            worst = (err / max(ref, 1e-12), k)
-        assert err <= 1e-1 * ref + 1e-2 * total_norm, (k, err, ref, total_norm)
-    print(f'{tag} skip={skip} latent={latent}: global gradient rel-L2 error', (num / den) ** 0.5, 'worst parameter', worst)
-    assert (num / den) ** 0.5 <= 3e-2, ((num / den) ** 0.5, worst)
+    check_step_gradients(got, want, f'{tag} skip={skip} latent={latent} complexity={complexity} {geometry}',
+                         floorless=FLOORLESS if complexity == 2 else None)
 
 
 def _film_operands(D, C0, H, T, B, seed):

@@ -351,6 +351,9 @@ extern "C" int tt_deconv_in(const void* lat, void* y, const void* w, const float
 // =========================================================================================================
 namespace tt {
 
+// barriers, TMEM slot and the bias (NL floats) ahead of the two stages; 1024 B would hold only 224 bias values
+constexpr int kLatHeader = 2048;
+
 template <int NL>
 __global__ void __launch_bounds__(128) conv_lat_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ lat,
                                                        const __nv_bfloat16* __restrict__ w, const float* __restrict__ bias,
@@ -359,9 +362,9 @@ __global__ void __launch_bounds__(128) conv_lat_kernel(const __nv_bfloat16* __re
     uint64_t* bar_free = reinterpret_cast<uint64_t*>(smem);          // [2] stage consumed by the tensor core
     uint64_t* bar_done = bar_free + 2;
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + 64);
-    float* sBias = reinterpret_cast<float*>(smem + 128);
+    float* sBias = reinterpret_cast<float*>(smem + 128);                 // NL <= 256 floats: up to smem + 1152
     const uint32_t a_bytes = (uint32_t)CG * kTileT * 16u, b_bytes = (uint32_t)CG * NL * 16u;
-    uint8_t* stage0 = smem + 1024;
+    uint8_t* stage0 = smem + kLatHeader;
     const uint32_t stage_bytes = a_bytes + b_bytes;
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -868,7 +871,7 @@ extern "C" int tt_conv_lat(const void* x, void* lat, const void* w, const float*
     if (B <= 0 || T <= 0) return TT_OK;
     const int CG = C4 / 8;
     dim3 grid((T + kTileT - 1) / kTileT, B);
-    const size_t smem = 1024 + 2 * ((size_t)CG * kTileT * 16 + (size_t)CG * NL * 16);
+    const size_t smem = kLatHeader + 2 * ((size_t)CG * kTileT * 16 + (size_t)CG * NL * 16);
     cudaStream_t s = (cudaStream_t)stream;
 #define TT_LAT_CASE(N)                                                                                               \
     case N:                                                                                                          \
