@@ -79,6 +79,28 @@ int tt_cqt_inverse(tt_cqt_plan* plan, const float* coeffs, int batch, int n_bloc
 int tt_scale_by_peak(float* audio, int64_t n, const float* peak, void* stream);
 
 /*
+ * ---- many clips of different lengths in one call (TimbreTrap.transcribe_many / reconstruct_many) ---------------------------------
+ * A clip table is a device int32 prefix array of n_clips + 1 entries: clip c owns entries [t[c], t[c+1]) (at least one), counted
+ * from t[0], so a slice of a longer table describes the clips it covers.  clip_block0 counts blocks (n_c = ceil(samples / L)),
+ * clip_chunk0 chunks (2 n_c + 1 per clip).  Per-clip tensors follow one another, each in the layout a one-clip call produces.
+ */
+/* tt_cqt_inverse over clips: coeffs = the clips' (F, n_c * M, 2) tensors, audio = their (n_c * L) samples, n_blocks = t[n] - t[0];
+ * peaks (n_clips) fp32 device: max|audio| of each clip before normalisation (reset here); normalise as tt_cqt_inverse, per clip */
+int tt_cqt_inverse_clips(tt_cqt_plan* plan, const float* coeffs, const int* clip_block0, int n_clips, int n_blocks, float* audio,
+                         float* peaks, int normalise, void* stream);
+
+/* audio of the clips of clip_block0 (n_blocks blocks of block_length samples): each divided by its own peak when non-zero */
+int tt_scale_by_clip_peak(float* audio, const int* clip_block0, int n_clips, int n_blocks, int block_length, const float* peaks,
+                          void* stream);
+
+/* the chunk matrix: out row r = chunk chunk_lo + r of the clips (TimbreTrap._chunks, modules.py:226-234, for each clip: padded with
+ * zeros to whole blocks, then by half a block on either side), r < n_rows.
+ *   clips  (n_clips, 2) int64 device: (address of the clip's fp32 samples, number of samples)
+ *   out    (n_rows, block_length) fp32 */
+int tt_gather_chunks(const int64_t* clips, const int* clip_chunk0, int n_clips, int chunk_lo, int n_rows, int block_length,
+                     float* out, void* stream);
+
+/*
  * TimbreTrap.to_activations (modules.py:271-289) = tanh(CQT.to_magnitude) (cqtwrapper.py:122-141)
  *   coeffs (rows, 2) interleaved -> out (rows);  apply_tanh = 0 gives the plain magnitude
  */
@@ -103,6 +125,11 @@ int tt_to_decibels(const float* magnitude, int batch, int64_t per_item, int resc
  */
 int tt_chunk_crossfade(const float* chunks, const float* window, int batch, int n_chunks, int n_bins, int frames_per_chunk,
                        float* coeffs_out, float* act_out, void* stream);
+
+/* tt_chunk_crossfade over the clips of clip_chunk0: chunks (t[n] - t[0], F, M, 2); clip c's outputs (F, (n_c - 1) * M/2 [, 2]) follow
+ * those of the clips before it; max_chunks = the most chunks of any clip */
+int tt_chunk_crossfade_clips(const float* chunks, const float* window, const int* clip_chunk0, int n_clips, int max_chunks, int n_bins,
+                             int frames_per_chunk, float* coeffs_out, float* act_out, void* stream);
 
 /*
  * ---- evaluation post-processing, the step after `transcribe` (SURVEY.md section 8f-1) --------------------------------
@@ -190,6 +217,12 @@ int tt_conv_out(const void* x, float* coeffs, const float* w, const float* bias,
  *   coeffs_out  (batch, H, (n_chunks-1) * M/2, 2) fp32 or NULL;  act_out (batch, H, (n_chunks-1) * M/2) fp32 or NULL */
 int tt_conv_out_crossfade(const void* x, const float* window, const float* w, const float* bias, int batch, int n_chunks, int C,
                           int H, int M, float* coeffs_out, float* act_out, void* stream);
+
+/* tt_conv_out_crossfade over the clips of clip_chunk0 (see tt_cqt_inverse_clips): x (total_chunks, H, M, 4) with total_chunks =
+ * t[n] - t[0]; clip c's outputs (H, (n_c - 1) * M/2 [, 2]) follow those of the clips before it; max_chunks = the most of any clip */
+int tt_conv_out_crossfade_clips(const void* x, const float* window, const float* w, const float* bias, const int* clip_chunk0,
+                                int n_clips, int total_chunks, int max_chunks, int C, int H, int M, float* coeffs_out, float* act_out,
+                                void* stream);
 
 /*
  * ---- model variants and skip connections (modules.py:95-117, 568-589, 780-1075): single-pass element-wise kernels ----------

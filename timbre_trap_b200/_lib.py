@@ -44,6 +44,11 @@ SIGNATURES = {
     'tt_conv_in': (c_int, [c_void_p] * 4 + [c_int] * 5 + [c_void_p]),
     'tt_conv_out': (c_int, [c_void_p] * 4 + [c_int] * 5 + [c_void_p]),
     'tt_conv_out_crossfade': (c_int, [c_void_p] * 4 + [c_int] * 5 + [c_void_p] * 3),
+    'tt_cqt_inverse_clips': (c_int, [c_void_p] * 3 + [c_int] * 2 + [c_void_p] * 2 + [c_int, c_void_p]),
+    'tt_scale_by_clip_peak': (c_int, [c_void_p] * 2 + [c_int] * 3 + [c_void_p] * 2),
+    'tt_gather_chunks': (c_int, [c_void_p] * 2 + [c_int] * 4 + [c_void_p] * 2),
+    'tt_chunk_crossfade_clips': (c_int, [c_void_p] * 3 + [c_int] * 4 + [c_void_p] * 3),
+    'tt_conv_out_crossfade_clips': (c_int, [c_void_p] * 5 + [c_int] * 6 + [c_void_p] * 3),
     'tt_add_scaled_bf16': (c_int, [c_void_p] * 4 + [c_int64, c_void_p]),
     'tt_dot_scratch_floats': (c_int, []),
     'tt_dot_bf16': (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),

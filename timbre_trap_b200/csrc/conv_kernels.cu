@@ -663,10 +663,13 @@ __global__ void __launch_bounds__(128) conv_out_p4_kernel(const uint2* __restric
 // fp32 activation) per output frame.  Products are rounded separately and added in chunk order, like the reference's
 // `coefficients[...] += window * chunk` (and like crossfade_kernel, which remains for the un-fused API path).
 //   x (batch * n_chunks, H, M, 4) bf16 packed4;  coeffs_out (batch, H, (n_chunks-1) M/2, 2) and / or act_out (batch, H, (n_chunks-1) M/2)
+// blockIdx.z is the item.  With clip_chunk0 (the many-clip calls) it is clip z of the chunk prefix table instead (find_clip): its
+// n = clip_chunk0[z + 1] - clip_chunk0[z] chunks and its (H, (n - 1) M/2) outputs follow those of the clips before it, and the grid
+// covers the longest clip (a CTA never straddles two clips; the CTAs past a shorter clip's end do nothing).
 __global__ void __launch_bounds__(128) conv_out_xfade_p4_kernel(const uint2* __restrict__ x, const float* __restrict__ window,
                                                                 const float* __restrict__ w /* [2][C][3][3] */, const float* __restrict__ bias,
                                                                 int C, int H, int M, int n_chunks, int rows, float2* __restrict__ coeffs_out,
-                                                                float* __restrict__ act_out) {
+                                                                float* __restrict__ act_out, const int* __restrict__ clip_chunk0) {
     __shared__ __align__(16) float2 sw[3][3][4];     // [ky][kx][c] -> (w for output 0, w for output 1)
     __shared__ float2 sb;
     for (int i = threadIdx.x; i < 36; i += 128) {
@@ -676,15 +679,22 @@ __global__ void __launch_bounds__(128) conv_out_xfade_p4_kernel(const uint2* __r
     if (threadIdx.x == 0) sb = make_float2(bias[0], bias[1]);
     __syncthreads();
     const int half = M / 2;
+    const int b = blockIdx.z, h0 = blockIdx.y * rows, h1 = min(H, h0 + rows);
+    size_t chunk0 = (size_t)b * n_chunks;                        // the item's first chunk
+    if (clip_chunk0) {
+        chunk0 = (size_t)(__ldg(clip_chunk0 + b) - __ldg(clip_chunk0));
+        n_chunks = __ldg(clip_chunk0 + b + 1) - __ldg(clip_chunk0 + b);
+    }
     const long long n_out = (long long)(n_chunks - 1) * half;
     const long long t0 = ((long long)blockIdx.x * 128 + threadIdx.x) * 4;
     if (t0 >= n_out) return;
-    const int b = blockIdx.z, h0 = blockIdx.y * rows, h1 = min(H, h0 + rows);
+    // the item's outputs: after those of its predecessors, (n_c - 1) M/2 frames of H rows each, i.e. chunk0 - b times H * half
+    const size_t out0 = (size_t)H * half * (chunk0 - b);
     const int i1 = (int)(t0 / half) + 1;                         // the later chunk; the earlier one is i1 - 1
     const int p1 = (int)(t0 - (long long)(i1 - 1) * half);       // position in the later chunk; + half in the earlier one
     // source s = 0: earlier chunk at frames p1 + half .., s = 1: later chunk at frames p1 ..
     const int pos[2] = {p1 + half, p1};
-    const uint2* xs[2] = {x + ((size_t)b * n_chunks + i1 - 1) * H * M + pos[0], x + ((size_t)b * n_chunks + i1) * H * M + pos[1]};
+    const uint2* xs[2] = {x + (chunk0 + i1 - 1) * H * M + pos[0], x + (chunk0 + i1) * H * M + pos[1]};
     const float4 wv0 = __ldg(reinterpret_cast<const float4*>(window + pos[0])), wv1 = __ldg(reinterpret_cast<const float4*>(window + pos[1]));
     const float win[2][4] = {{wv0.x, wv0.y, wv0.z, wv0.w}, {wv1.x, wv1.y, wv1.z, wv1.w}};
     const float2 bias2 = sb;
@@ -740,7 +750,7 @@ __global__ void __launch_bounds__(128) conv_out_xfade_p4_kernel(const uint2* __r
                 r[f].x = __fadd_rn(__fmul_rn(win[0][f], A[0][f].x), __fmul_rn(win[1][f], A[1][f].x));
                 r[f].y = __fadd_rn(__fmul_rn(win[0][f], A[0][f].y), __fmul_rn(win[1][f], A[1][f].y));
             }
-            const size_t o = ((size_t)b * H + ho) * n_out + t0;
+            const size_t o = out0 + (size_t)ho * n_out + t0;
             if (coeffs_out) {
                 float4* dst = reinterpret_cast<float4*>(coeffs_out + o);
                 __stcs(dst, make_float4(r[0].x, r[0].y, r[1].x, r[1].y));
@@ -940,7 +950,28 @@ extern "C" int tt_conv_out_crossfade(const void* x, const float* window, const f
     while (rows > 6 && (long long)batch * col_ctas * ((H + rows - 1) / rows) < 4 * 148) rows /= 2;
     TT_REQUIRE(col_ctas < (1ll << 31), "conv_out_crossfade: clip too long for one launch");
     conv_out_xfade_p4_kernel<<<dim3((unsigned)col_ctas, (H + rows - 1) / rows, batch), 128, 0, (cudaStream_t)stream>>>(
-        (const uint2*)x, window, w, bias, C, H, M, n_chunks, rows, (float2*)coeffs_out, act_out);
+        (const uint2*)x, window, w, bias, C, H, M, n_chunks, rows, (float2*)coeffs_out, act_out, nullptr);
+    tt_count_launches(1);
+    TT_CUDA_CHECK(cudaGetLastError());
+    return TT_OK;
+}
+
+extern "C" int tt_conv_out_crossfade_clips(const void* x, const float* window, const float* w, const float* bias, const int* clip_chunk0,
+                                           int n_clips, int total_chunks, int max_chunks, int C, int H, int M, float* coeffs_out,
+                                           float* act_out, void* stream) {
+    TT_REQUIRE(x && window && w && bias && clip_chunk0 && (coeffs_out || act_out), "null argument");
+    TT_REQUIRE(C >= 1 && C <= 4, "conv_out_crossfade: the packed layout holds at most 4 channels");
+    TT_REQUIRE(max_chunks >= 2 && M >= 8 && M % 8 == 0, "conv_out_crossfade: at least two chunks, chunk length a multiple of 8 (got %d, %d)", max_chunks, M);
+    TT_REQUIRE(n_clips <= 65535, "conv_out_crossfade: at most 65535 clips per call (got %d)", n_clips);
+    if (n_clips <= 0 || H <= 0) return TT_OK;
+    const long long col_ctas = ((long long)(max_chunks - 1) * (M / 2) / 4 + 127) / 128;
+    // strip height from the CTAs that do work (as if the chunks were one uniform batch), not from the padded grid
+    const long long busy_ctas = ((long long)(total_chunks - n_clips) * (M / 2) / 4 + 127) / 128;
+    int rows = 36;
+    while (rows > 6 && busy_ctas * ((H + rows - 1) / rows) < 4 * 148) rows /= 2;
+    TT_REQUIRE(col_ctas < (1ll << 31), "conv_out_crossfade: clip too long for one launch");
+    conv_out_xfade_p4_kernel<<<dim3((unsigned)col_ctas, (H + rows - 1) / rows, n_clips), 128, 0, (cudaStream_t)stream>>>(
+        (const uint2*)x, window, w, bias, C, H, M, 0, rows, (float2*)coeffs_out, act_out, clip_chunk0);
     tt_count_launches(1);
     TT_CUDA_CHECK(cudaGetLastError());
     return TT_OK;

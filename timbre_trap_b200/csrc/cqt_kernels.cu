@@ -168,6 +168,23 @@ struct BinTables {
     const float* dual;   // dual window  (synthesis)
 };
 
+// Offset (in float2) of the row of bin k in block gb of a (items, F, n_blocks * M) interleaved coefficient tensor.  Uniform items of
+// n_blocks_item blocks, or - clip_block0 non-null - clips of clip_block0[c + 1] - clip_block0[c] blocks packed one after the other
+// (the many-clip calls, find_clip), each in the layout a one-clip call has.
+__device__ __forceinline__ size_t coeff_row(int gb, int k, int F, int M, int n_blocks_item, const int* __restrict__ clip_block0,
+                                            int n_clips) {
+    int first, n;
+    if (clip_block0) {
+        const int c = find_clip(clip_block0, n_clips, gb);
+        first = __ldg(clip_block0 + c) - __ldg(clip_block0);
+        n = __ldg(clip_block0 + c + 1) - __ldg(clip_block0 + c);
+    } else {
+        first = gb / n_blocks_item * n_blocks_item;
+        n = n_blocks_item;
+    }
+    return (size_t)first * F * M + (size_t)k * n * M + (size_t)(gb - first) * M;
+}
+
 template <int Z>
 __device__ __forceinline__ void bin_fwd_stage1(const float2* __restrict__ spec_taps, const float* __restrict__ win,
                                                int len, int shift, int lane, float2 (&B)[32]) {
@@ -295,7 +312,8 @@ __device__ __forceinline__ void bin_inv_stage3(float2 (&E)[32], float2* __restri
 
 __global__ void __launch_bounds__(kBinWarps * 32, 6)
 bins_inv_kernel(const float* __restrict__ coeffs, float2* __restrict__ S, BinTables tab, int F, int SP,
-                int n_blocks_item, int block0, int n_blocks_launch, const float2* __restrict__ tw_m) {
+                int n_blocks_item, int block0, int n_blocks_launch, const float2* __restrict__ tw_m,
+                const int* __restrict__ clip_block0, int n_clips) {
     constexpr int M = 1024;
     extern __shared__ float2 smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -305,11 +323,7 @@ bins_inv_kernel(const float* __restrict__ coeffs, float2* __restrict__ S, BinTab
     if (w >= (long long)n_blocks_launch * F) return;
     const int lb = (int)(w / F);
     const int k = (int)(w - (long long)lb * F);
-    const int gb = block0 + lb;
-    const int item = gb / n_blocks_item, blk = gb - item * n_blocks_item;
-
-    const float2* in = reinterpret_cast<const float2*>(coeffs) +
-                       ((size_t)item * F + k) * ((size_t)n_blocks_item * M) + (size_t)blk * M;
+    const float2* in = reinterpret_cast<const float2*>(coeffs) + coeff_row(block0 + lb, k, F, M, n_blocks_item, clip_block0, n_clips);
     float2 v[32];
 #pragma unroll
     for (int n1 = 0; n1 < 32; ++n1) v[n1] = ld_stream(in + lane + 32 * n1);
@@ -381,7 +395,8 @@ bins_fwd_generic_kernel(const float2* __restrict__ S, float* __restrict__ coeffs
 
 __global__ void __launch_bounds__(128)
 bins_inv_generic_kernel(const float* __restrict__ coeffs, float2* __restrict__ S, BinTables tab, int F, int SP,
-                        int n_blocks_item, int block0, FftSpec spec, const float2* __restrict__ tw_m_fwd) {
+                        int n_blocks_item, int block0, FftSpec spec, const float2* __restrict__ tw_m_fwd,
+                        const int* __restrict__ clip_block0, int n_clips) {
     extern __shared__ float2 smem[];
     const int M = spec.n;
     float2* buf_a = smem;
@@ -389,10 +404,7 @@ bins_inv_generic_kernel(const float* __restrict__ coeffs, float2* __restrict__ S
     float2* tw = smem + 2 * M;
     const int tid = threadIdx.x;
     const int k = blockIdx.x, lb = blockIdx.y;
-    const int gb = block0 + lb;
-    const int item = gb / n_blocks_item, blk = gb - item * n_blocks_item;
-    const float2* in = reinterpret_cast<const float2*>(coeffs) +
-                       ((size_t)item * F + k) * ((size_t)n_blocks_item * M) + (size_t)blk * M;
+    const float2* in = reinterpret_cast<const float2*>(coeffs) + coeff_row(block0 + lb, k, F, M, n_blocks_item, clip_block0, n_clips);
     for (int i = tid; i < M; i += 128) {
         tw[i] = tw_m_fwd[i];
         buf_a[i] = ld_stream(in + i);
@@ -452,10 +464,12 @@ rows_inv_kernel(const float2* __restrict__ S, float2* __restrict__ T, FftSpec sp
 // ---------------------------------------------------------------------------------------------
 // S3: inverse column transforms + 1/L + peak.   y[N2 n1 + n2] = (1/L) sum_k1 G[k1][n2] w_N1^{-k1 n1},
 // G Hermitian in k1; two real columns share one complex transform (Z = Ga + i Gb -> ya = Re, yb = Im).
+// One peak for the whole call, or - clip_block0 non-null - one per clip (block block0 + blockIdx.y is in clip find_clip(..)).
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kFftThreads)
 cols_inv_kernel(const float2* __restrict__ T, float* __restrict__ audio, FftSpec spec, int N2, int K1, int L,
-                const float2* __restrict__ tw_n1, unsigned int* __restrict__ peak_bits) {
+                const float2* __restrict__ tw_n1, unsigned int* __restrict__ peak_bits, const int* __restrict__ clip_block0,
+                int n_clips, int block0) {
     extern __shared__ float2 smem[];
     const int N1 = spec.n;
     constexpr int G = kColsPerCta;
@@ -499,7 +513,8 @@ cols_inv_kernel(const float2* __restrict__ T, float* __restrict__ audio, FftSpec
     __syncthreads();
     if (tid == 0) {
         for (int i = 1; i < kFftThreads / 32; ++i) peak = fmaxf(peak, red[i]);
-        atomicMax(peak_bits, __float_as_uint(peak));   // non-negative floats order like their bit patterns
+        const int clip = clip_block0 ? find_clip(clip_block0, n_clips, block0 + (int)blockIdx.y) : 0;
+        atomicMax(peak_bits + clip, __float_as_uint(peak));   // non-negative floats order like their bit patterns
     }
 }
 
@@ -508,6 +523,15 @@ __global__ void scale_by_peak_kernel(float* __restrict__ audio, long long n, con
     if (!(p > 0.f)) return;
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) audio[i] = audio[i] / p;
+}
+
+// the same per clip: block blockIdx.y (L samples) is divided by the peak of its clip
+__global__ void scale_by_clip_peak_kernel(float* __restrict__ audio, int L, const int* __restrict__ clip_block0, int n_clips,
+                                          const float* __restrict__ peaks) {
+    const float p = peaks[find_clip(clip_block0, n_clips, blockIdx.y)];
+    if (!(p > 0.f)) return;
+    float* a = audio + (size_t)blockIdx.y * L;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < L; i += gridDim.x * blockDim.x) a[i] = a[i] / p;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -553,14 +577,23 @@ __global__ void decibels_kernel(const float* __restrict__ x, long long per_item,
 // frame t (after the M/2 trim) receives chunk i1 = (t + M/2) / (M/2) at position p1 = (t + M/2) mod (M/2) and chunk
 // i1 - 1 at position p1 + M/2, each scaled by the window.  Products are rounded separately and added in chunk order,
 // like the reference's `coefficients[...] += window * output_chunk`.
+// blockIdx.z is the item: batch items of n_chunks chunks each, or - clip_chunk0 non-null - clip z of the chunk prefix table
+// (find_clip), whose chunks and whose (F, (n - 1) M/2) output rows follow those of the clips before it.
 __global__ void crossfade_kernel(const float2* __restrict__ chunks, const float* __restrict__ window, int n_chunks, int F,
-                                 int M, float2* __restrict__ coeffs_out, float* __restrict__ act_out) {
+                                 int M, float2* __restrict__ coeffs_out, float* __restrict__ act_out, const int* __restrict__ clip_chunk0) {
     const int half = M / 2;
-    const long long n_out = (long long)(n_chunks - 1) * half;
     const int b = blockIdx.z, f = blockIdx.y;
-    const float2* base = chunks + ((size_t)b * n_chunks * F + f) * M;       // chunk i of item b: + i * F * M
+    size_t chunk0 = (size_t)b * n_chunks, out0 = (size_t)b * F * ((size_t)(n_chunks - 1) * half);
+    if (clip_chunk0) {
+        const int c0 = __ldg(clip_chunk0 + b) - __ldg(clip_chunk0);
+        n_chunks = __ldg(clip_chunk0 + b + 1) - __ldg(clip_chunk0 + b);
+        chunk0 = (size_t)c0;
+        out0 = (size_t)F * half * (size_t)(c0 - b);       // sum over earlier clips of F (n_c - 1) M/2
+    }
+    const long long n_out = (long long)(n_chunks - 1) * half;
+    const float2* base = chunks + (chunk0 * F + f) * M;       // chunk i of the item: + i * F * M
     const size_t chunk_stride = (size_t)F * M;
-    const size_t out_row = ((size_t)b * F + f) * n_out;
+    const size_t out_row = out0 + (size_t)f * n_out;
     for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < n_out; t += (long long)gridDim.x * blockDim.x) {
         const long long tf = t + half;
         const int i1 = (int)(tf / half);
@@ -573,6 +606,24 @@ __global__ void crossfade_kernel(const float2* __restrict__ chunks, const float*
         r.y = __fadd_rn(__fmul_rn(w0, c0.y), __fmul_rn(w1, c1.y));
         if (coeffs_out) coeffs_out[out_row + t] = r;
         if (act_out) act_out[out_row + t] = tanhf(sqrtf(r.x * r.x + r.y * r.y));
+    }
+}
+
+// The chunk matrix of the many-clip calls (TimbreTrap._chunks of every clip, modules.py:226-234): clip c of n_c samples, zero-padded
+// to a whole number of blocks and by half a block on either side, cut into 50 %-overlapped chunks of L samples.  Row r of `out` is
+// chunk chunk_lo + r of the clip list; clip_chunk0 is the chunk prefix table (find_clip), clips[c] = (address, samples) of clip c.
+__global__ void gather_chunks_kernel(const longlong2* __restrict__ clips, const int* __restrict__ clip_chunk0, int n_clips,
+                                     int chunk_lo, int L, float* __restrict__ out) {
+    const int g = chunk_lo + (int)blockIdx.y;
+    const int c = find_clip(clip_chunk0, n_clips, g);
+    const longlong2 clip = clips[c];
+    const float* x = reinterpret_cast<const float*>(clip.x);
+    const int hop = L / 2;
+    const long long s0 = (long long)(g - (__ldg(clip_chunk0 + c) - __ldg(clip_chunk0))) * hop - hop;
+    float* o = out + (size_t)blockIdx.y * L;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < L; i += gridDim.x * blockDim.x) {
+        const long long s = s0 + i;
+        o[i] = (s >= 0 && s < clip.y) ? __ldg(x + s) : 0.f;
     }
 }
 
@@ -816,14 +867,11 @@ extern "C" int tt_scale_by_peak(float* audio, int64_t n, const float* peak, void
     return TT_OK;
 }
 
-extern "C" int tt_cqt_inverse(tt_cqt_plan* p, const float* coeffs, int batch, int n_blocks, float* audio, float* peak,
-                              int normalise, void* stream_) {
-    TT_REQUIRE(p && coeffs && audio && peak, "null argument");
-    TT_REQUIRE(batch >= 0 && n_blocks >= 0, "negative sizes");
-    cudaStream_t user = (cudaStream_t)stream_;
-    const long long total = (long long)batch * n_blocks;
+// batch uniform items of n_blocks_item blocks (one peak), or the clips of clip_block0 (one peak each); `total` blocks in all
+static int cqt_inverse(tt_cqt_plan* p, const float* coeffs, long long total, int n_blocks_item, const int* clip_block0, int n_clips,
+                       float* audio, float* peak, cudaStream_t user) {
     const BinTables tab = bin_tables(p);
-    TT_CUDA_CHECK(cudaMemsetAsync(peak, 0, sizeof(float), user));
+    TT_CUDA_CHECK(cudaMemsetAsync(peak, 0, (clip_block0 ? n_clips : 1) * sizeof(float), user));
     if (total == 0) return TT_OK;
     const int n_groups = (int)((total + p->max_blocks - 1) / p->max_blocks);
     const int n_lanes = std::min(n_groups, p->n_lanes);
@@ -838,19 +886,20 @@ extern "C" int tt_cqt_inverse(tt_cqt_plan* p, const float* coeffs, int batch, in
         if (p->M == 1024) {
             const long long warps = (long long)nb * p->F;
             const unsigned g1 = (unsigned)((warps + kBinWarps - 1) / kBinWarps);
-            bins_inv_kernel<<<g1, kBinWarps * 32, bins_smem(), stream>>>(coeffs, S, tab, p->F, p->SP, n_blocks, (int)b0, nb,
-                                                                          p->d_tw_m_inv);
+            bins_inv_kernel<<<g1, kBinWarps * 32, bins_smem(), stream>>>(coeffs, S, tab, p->F, p->SP, n_blocks_item, (int)b0, nb,
+                                                                          p->d_tw_m_inv, clip_block0, n_clips);
         } else {
             dim3 g1(p->F, nb);
-            bins_inv_generic_kernel<<<g1, 128, 3 * p->M * sizeof(float2), stream>>>(coeffs, S, tab, p->F, p->SP, n_blocks,
-                                                                                     (int)b0, p->spec_m, p->d_tw_m_fwd);
+            bins_inv_generic_kernel<<<g1, 128, 3 * p->M * sizeof(float2), stream>>>(coeffs, S, tab, p->F, p->SP, n_blocks_item,
+                                                                                     (int)b0, p->spec_m, p->d_tw_m_fwd, clip_block0,
+                                                                                     n_clips);
         }
         dim3 g2((p->K1 + kRowsPerCta - 1) / kRowsPerCta, nb);
         rows_inv_kernel<<<g2, kFftThreads, rows_smem(p), stream>>>(S, T, p->spec_n2, p->N1, p->K1, p->L, p->SP, p->d_tw_n2,
                                                                     p->d_tw_L);
         dim3 g3((p->N2 + kColsPerCta - 1) / kColsPerCta, nb);
         cols_inv_kernel<<<g3, kFftThreads, cols_smem(p), stream>>>(T, audio + (size_t)b0 * p->L, p->spec_n1, p->N2, p->K1, p->L,
-                                                                    p->d_tw_n1, (unsigned int*)peak);
+                                                                    p->d_tw_n1, (unsigned int*)peak, clip_block0, n_clips, (int)b0);
         tt_count_launches(3);
     }
     TT_CUDA_CHECK(cudaGetLastError());
@@ -858,7 +907,40 @@ extern "C" int tt_cqt_inverse(tt_cqt_plan* p, const float* coeffs, int batch, in
         TT_CUDA_CHECK(cudaEventRecord(p->ev_done[i], p->lane[i]));
         TT_CUDA_CHECK(cudaStreamWaitEvent(user, p->ev_done[i], 0));
     }
+    return TT_OK;
+}
+
+extern "C" int tt_cqt_inverse(tt_cqt_plan* p, const float* coeffs, int batch, int n_blocks, float* audio, float* peak,
+                              int normalise, void* stream_) {
+    TT_REQUIRE(p && coeffs && audio && peak, "null argument");
+    TT_REQUIRE(batch >= 0 && n_blocks >= 0, "negative sizes");
+    const long long total = (long long)batch * n_blocks;
+    const int rc = cqt_inverse(p, coeffs, total, n_blocks, nullptr, 0, audio, peak, (cudaStream_t)stream_);
+    if (rc != TT_OK || total == 0) return rc;
     if (normalise) return tt_scale_by_peak(audio, total * p->L, peak, stream_);
+    return TT_OK;
+}
+
+extern "C" int tt_scale_by_clip_peak(float* audio, const int* clip_block0, int n_clips, int n_blocks, int block_length,
+                                     const float* peaks, void* stream_) {
+    TT_REQUIRE(audio && clip_block0 && peaks, "null argument");
+    TT_REQUIRE(n_blocks <= 65535, "at most 65535 blocks per call (got %d)", n_blocks);
+    if (n_clips <= 0 || n_blocks <= 0 || block_length <= 0) return TT_OK;
+    dim3 grid((unsigned)std::min((block_length + 1023) / 1024, 64), n_blocks);
+    scale_by_clip_peak_kernel<<<grid, 256, 0, (cudaStream_t)stream_>>>(audio, block_length, clip_block0, n_clips, peaks);
+    tt_count_launches(1);
+    TT_CUDA_CHECK(cudaGetLastError());
+    return TT_OK;
+}
+
+extern "C" int tt_cqt_inverse_clips(tt_cqt_plan* p, const float* coeffs, const int* clip_block0, int n_clips, int n_blocks,
+                                    float* audio, float* peaks, int normalise, void* stream_) {
+    TT_REQUIRE(p && coeffs && clip_block0 && audio && peaks, "null argument");
+    TT_REQUIRE(n_clips >= 0 && n_blocks >= 0, "negative sizes");
+    if (n_clips == 0) return TT_OK;
+    const int rc = cqt_inverse(p, coeffs, n_blocks, 1, clip_block0, n_clips, audio, peaks, (cudaStream_t)stream_);
+    if (rc != TT_OK || n_blocks == 0) return rc;
+    if (normalise) return tt_scale_by_clip_peak(audio, clip_block0, n_clips, n_blocks, p->L, peaks, stream_);
     return TT_OK;
 }
 
@@ -895,7 +977,36 @@ extern "C" int tt_chunk_crossfade(const float* chunks, const float* window, int 
     const long long n_out = (long long)(n_chunks - 1) * (frames_per_chunk / 2);
     dim3 grid((unsigned)std::min<long long>((n_out + 255) / 256, 64), n_bins, batch);
     crossfade_kernel<<<grid, 256, 0, (cudaStream_t)stream_>>>((const float2*)chunks, window, n_chunks, n_bins, frames_per_chunk,
-                                                              (float2*)coeffs_out, act_out);
+                                                              (float2*)coeffs_out, act_out, nullptr);
+    tt_count_launches(1);
+    TT_CUDA_CHECK(cudaGetLastError());
+    return TT_OK;
+}
+
+extern "C" int tt_chunk_crossfade_clips(const float* chunks, const float* window, const int* clip_chunk0, int n_clips,
+                                        int max_chunks, int n_bins, int frames_per_chunk, float* coeffs_out, float* act_out,
+                                        void* stream_) {
+    TT_REQUIRE(chunks && window && clip_chunk0 && (coeffs_out || act_out), "null argument");
+    TT_REQUIRE(max_chunks >= 2 && frames_per_chunk % 2 == 0, "need at least two chunks and an even chunk length");
+    TT_REQUIRE(n_clips <= 65535, "at most 65535 clips per call (got %d)", n_clips);
+    if (n_clips <= 0 || n_bins <= 0) return TT_OK;
+    const long long n_out = (long long)(max_chunks - 1) * (frames_per_chunk / 2);
+    dim3 grid((unsigned)std::min<long long>((n_out + 255) / 256, 64), n_bins, n_clips);
+    crossfade_kernel<<<grid, 256, 0, (cudaStream_t)stream_>>>((const float2*)chunks, window, 0, n_bins, frames_per_chunk,
+                                                              (float2*)coeffs_out, act_out, clip_chunk0);
+    tt_count_launches(1);
+    TT_CUDA_CHECK(cudaGetLastError());
+    return TT_OK;
+}
+
+extern "C" int tt_gather_chunks(const int64_t* clips, const int* clip_chunk0, int n_clips, int chunk_lo, int n_rows, int block_length,
+                                float* out, void* stream_) {
+    TT_REQUIRE(clips && clip_chunk0 && out, "null argument");
+    TT_REQUIRE(n_rows <= 65535, "at most 65535 chunks per call (got %d)", n_rows);
+    if (n_clips <= 0 || n_rows <= 0 || block_length <= 0) return TT_OK;
+    dim3 grid((unsigned)std::min((block_length + 2047) / 2048, 64), n_rows);
+    gather_chunks_kernel<<<grid, 256, 0, (cudaStream_t)stream_>>>((const longlong2*)clips, clip_chunk0, n_clips, chunk_lo,
+                                                                  block_length, out);
     tt_count_launches(1);
     TT_CUDA_CHECK(cudaGetLastError());
     return TT_OK;

@@ -56,4 +56,17 @@ __device__ __forceinline__ void st_stream(float4* p, float4 v) { __stcs(p, v); }
 __device__ __forceinline__ float2 ld_stream(const float2* p) { return __ldcs(p); }
 __device__ __forceinline__ float4 ld_stream(const float4* p) { return __ldcs(p); }
 
+// Clip tables of the many-clip calls: prefix[c] is the first block (or chunk) of clip c and prefix[n] the end, all relative to
+// prefix[0] (a slice of a longer table works unchanged).  Every clip holds at least one entry.  Returns the clip holding x.
+__device__ __forceinline__ int find_clip(const int* __restrict__ prefix, int n, int x) {
+    const int base = __ldg(prefix);
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (__ldg(prefix + mid) - base <= x) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+
 }  // namespace tt

@@ -12,6 +12,7 @@ Activations between layers live in the C8 planar bf16 layout (B, ceil(C/8), H, T
 
 import ctypes
 
+import numpy as np
 import torch
 import torch.nn as nn
 
@@ -25,6 +26,10 @@ from .packing import _PackedCache       # also the name under which pickled modu
 
 __all__ = ['TimbreTrap', 'TimbreTrapFiLM', 'FiLM', 'TimbreTrapMag', 'TimbreTrapMagDB', 'Encoder', 'Decoder', 'EncoderBlock', 'DecoderBlock',
            'ResidualConv2dBlock', 'shard_block_range', 'shard_audio']
+
+
+def _ptr(t):
+    return ctypes.c_void_p(t.data_ptr())
 
 
 def _n16(c):
@@ -613,6 +618,10 @@ class TimbreTrap(nn.Module):
         chunks = audio.unfold(-1, L, hop)[:, :, :n_chunks]                 # (B, 1, n_chunks, L) view
         return chunks.reshape(audio.size(0) * n_chunks, 1, L), n_chunks
 
+    def _fused_convout(self):
+        """Whether the chunked paths run convout + cross-fade as one kernel (tt_conv_out_crossfade) on the packed last stage."""
+        return self.FUSE_CONVOUT_CROSSFADE and self.decoder.packed4 and self.sliCQ.max_window_length % 8 == 0 and self.HEAD_MODE is None
+
     def _chunked(self, audio, want_transcription, want_reconstruction, activations=True, prepadded=False, on_activations=None):
         """
         Batched form of chunked_inference (modules.py:204-269) for one or both switch settings with a shared
@@ -633,7 +642,7 @@ class TimbreTrap(nn.Module):
             chunks, n_chunks = self._chunks(audio.detach().float(), prepadded)
             n_out = (n_chunks - 1) * (M // 2)
             window = self._window(audio.device)
-            fused = self.FUSE_CONVOUT_CROSSFADE and self.decoder.packed4 and M % 8 == 0 and self.HEAD_MODE is None
+            fused = self._fused_convout()
             wants = (want_transcription, want_reconstruction)
             if fused:
                 stages = [torch.empty((B * n_chunks, F, M, 4), dtype=torch.bfloat16, device=audio.device) if w else None for w in wants]
@@ -759,6 +768,144 @@ class TimbreTrap(nn.Module):
         `on_activations`: see _chunked (early hand-over of finished clips' activations; the returned tensors are the same)."""
         act, rec = self._chunked(audio, True, True, on_activations=on_activations)
         return act, self._decode_shared_peak(rec.permute(0, 3, 1, 2), group)
+
+    # ---- many clips of different lengths in one batched pass ----------------------------------------------------------------
+    # The clips' chunks are cut straight from the clips by one kernel (tt_gather_chunks) and run through the encoder / decoder in
+    # batches of MAX_CHUNKS_PER_BATCH that cross clip boundaries; the cross-fade, the inverse CQT and the normalise read a clip table
+    # (int32 prefix sums of chunks and blocks per clip), so the launches follow the number of chunks, not of clips.  Clips go in
+    # groups of whole clips of at most MAX_CHUNKS_PER_GROUP chunks (or the longest clip's, if more): the per-chunk stage buffers
+    # (4.4 MB per chunk at the base model) stay bounded whatever the number of clips.
+    MAX_CHUNKS_PER_GROUP = 1024
+
+    def transcribe_many(self, clips):
+        """transcribe() of each of a list of clips of any lengths in one batched pass: `clips` (N_i,) or (1, N_i) CUDA tensors on one
+        device -> a list of activations, the i-th equal bit for bit to transcribe(clips[i].view(1, 1, -1))[0].  Views of one buffer."""
+        return self._many(clips, True, False)[0]
+
+    def reconstruct_many(self, clips):
+        """reconstruct() of each clip (see transcribe_many) -> a list of (1, N_i') audio, each normalised by its OWN peak - what
+        reconstruct(clips[i].view(1, 1, -1))[0] returns, bit for bit (a silent clip comes back as zeros).  Views of one buffer."""
+        return self._many(clips, False, True)[1]
+
+    def transcribe_and_reconstruct_many(self, clips):
+        """Both lists of transcribe_many and reconstruct_many from ONE encoder pass."""
+        return self._many(clips, True, True)
+
+    def _clip_table(self, clips):
+        """Validate a list of clips -> (flat fp32 contiguous clips, samples, blocks, chunks per clip as int64 numpy arrays)."""
+        device, flat = None, []
+        for i, c in enumerate(clips):
+            _lib.require_cuda(c, f'clips[{i}]')
+            if not (c.dim() == 1 or (c.dim() == 2 and c.size(0) == 1)):
+                raise ValueError(f'clips[{i}]: expected a mono clip of shape (N,) or (1, N), got {tuple(c.shape)}')
+            if c.numel() == 0:
+                raise ValueError(f'clips[{i}] is empty')
+            if device is None:
+                device = c.device
+            elif c.device != device:
+                raise ValueError(f'clips[{i}] is on {c.device}, clips[0] on {device}: all clips must be on one device')
+            x = c.detach().reshape(-1)
+            flat.append((x if x.dtype == torch.float32 else x.float()).contiguous())
+        L, hop = self.sliCQ.block_length, self.sliCQ.block_length // 2
+        samples = np.array([x.numel() for x in flat], dtype=np.int64)
+        blocks = -(-samples // L)
+        chunks = (blocks * L + hop) // hop              # _chunks: (n L + 2 hop - hop) // hop per clip
+        return flat, samples, blocks, chunks
+
+    def _many(self, clips, want_transcription, want_reconstruction):
+        """(activations list or None, audio list or None) of the *_many calls."""
+        clips = list(clips)
+        if not clips:
+            return [] if want_transcription else None, [] if want_reconstruction else None
+        flat, samples, blocks, chunks = self._clip_table(clips)
+        device = flat[0].device
+        n = len(flat)
+        F, M, L = self.sliCQ.n_bins, self.sliCQ.max_window_length, self.sliCQ.block_length
+        half = M // 2
+        chunk0 = np.concatenate(([0], np.cumsum(chunks)))
+        block0 = np.concatenate(([0], np.cumsum(blocks)))
+        out0 = np.concatenate(([0], np.cumsum((chunks - 1) * half)))          # first output frame of each clip
+        # groups of whole clips: [groups[g], groups[g + 1])
+        cap = max(self.MAX_CHUNKS_PER_GROUP, int(chunks.max()))
+        groups = [0]
+        for i in range(n):
+            if chunk0[i + 1] - chunk0[groups[-1]] > cap:
+                groups.append(i)
+        groups.append(n)
+        rows = max(int(chunk0[groups[g + 1]] - chunk0[groups[g]]) for g in range(len(groups) - 1))
+        with torch.no_grad(), torch.cuda.device(device):
+            tab = torch.from_numpy(np.concatenate((chunk0, block0)).astype(np.int32)).to(device)
+            clip_tab = torch.from_numpy(np.stack((np.array([x.data_ptr() for x in flat], dtype=np.int64), samples), 1)).to(device)
+            t_chunk0, t_block0 = tab[:n + 1], tab[n + 1:]
+            stream = ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+            window = self._window(device)
+            fused = self._fused_convout()
+            as_act = self.HEAD_MODE is None                  # the BASE model's tanh|.| is fused into the cross-fade
+            _, _, w_out, b_out = self.decoder._packed()
+            step = self.MAX_CHUNKS_PER_BATCH
+            f32 = dict(dtype=torch.float32, device=device)
+            batch = torch.empty((min(step, rows), L), **f32)
+            wants = (want_transcription, want_reconstruction)
+            if fused:
+                stages = [torch.empty((rows, F, M, 4), dtype=torch.bfloat16, device=device) if w else None for w in wants]
+            else:
+                stages = [torch.empty((rows, F, M, 2), **f32) if w else None for w in wants]
+            total_out = int(out0[-1])
+            trn = torch.empty((F * total_out * (1 if as_act else 2),), **f32) if want_transcription else None
+            audio = torch.empty((int(block0[-1]) * L,), **f32) if want_reconstruction else None
+            peaks = torch.empty((n,), **f32) if want_reconstruction else None
+            for g in range(len(groups) - 1):
+                lo, hi = groups[g], groups[g + 1]
+                c_lo, c_hi = int(chunk0[lo]), int(chunk0[hi])
+                for c0 in range(c_lo, c_hi, step):
+                    m = min(step, c_hi - c0)
+                    _lib.check(_lib.lib().tt_gather_chunks(_ptr(clip_tab), _ptr(t_chunk0), n, c0, m, L, _ptr(batch), stream))
+                    lat, skips = self._codes(batch[:m].view(m, 1, L))
+                    for stage, reconstruct in zip(stages, (False, True)):
+                        if stage is None:
+                            continue
+                        part = stage[c0 - c_lo:c0 - c_lo + m]
+                        if fused:
+                            self.decoder.last_stage_c8(lat, reconstruct, skips, out=part)
+                        else:
+                            y = self.decoder.forward_c8(lat, reconstruct, skips)
+                            if self.HEAD_MODE is not None:          # both channels carry the head's output, as in _chunked
+                                y = ops.channel0(y, self.HEAD_MODE).unsqueeze(-1).expand(-1, -1, -1, 2)
+                            part.copy_(y)
+                tab_g = ctypes.c_void_p(t_chunk0.data_ptr() + 4 * lo)
+                max_chunks = int(chunks[lo:hi].max())
+                for stage, reconstruct in zip(stages, (False, True)):
+                    if stage is None:
+                        continue
+                    o = F * int(out0[lo])
+                    if not reconstruct:
+                        dst = (None, _ptr(trn[o:])) if as_act else (_ptr(trn[2 * o:]), None)
+                    else:
+                        coeffs = torch.empty((F * int(out0[hi] - out0[lo]), 2), **f32)
+                        dst = (_ptr(coeffs), None)
+                    if fused:
+                        _lib.check(_lib.lib().tt_conv_out_crossfade_clips(_ptr(stage), _ptr(window), _ptr(w_out), _ptr(b_out), tab_g, hi - lo,
+                                                                          c_hi - c_lo, max_chunks, self.decoder.channels[4], F, M, *dst, stream))
+                    else:
+                        _lib.check(_lib.lib().tt_chunk_crossfade_clips(_ptr(stage), _ptr(window), tab_g, hi - lo, max_chunks, F, M, *dst,
+                                                                       stream))
+                    if reconstruct:
+                        _lib.check(_lib.lib().tt_cqt_inverse_clips(self.sliCQ._plan(device).handle, _ptr(coeffs),
+                                                                   ctypes.c_void_p(t_block0.data_ptr() + 4 * lo), hi - lo,
+                                                                   int(block0[hi] - block0[lo]), _ptr(audio[int(block0[lo]) * L:]),
+                                                                   _ptr(peaks[lo:]), 1, stream))
+            acts = wavs = None
+            if want_transcription:
+                if not as_act:
+                    # a variant's own activation function, once over the whole buffer (element-wise: the same values as per clip)
+                    pairs = self.to_activations(trn.view(1, 1, -1, 2).permute(0, 3, 1, 2)).permute(0, 2, 3, 1)
+                    trn = pairs.reshape(-1) if pairs.is_contiguous() else pairs.contiguous().reshape(-1)
+                    acts = [trn[2 * F * a:2 * F * b].view(F, b - a, 2).permute(2, 0, 1) for a, b in zip(out0[:-1].tolist(), out0[1:].tolist())]
+                else:
+                    acts = [trn[F * a:F * b].view(F, b - a) for a, b in zip(out0[:-1].tolist(), out0[1:].tolist())]
+            if want_reconstruction:
+                wavs = [audio[L * a:L * b].view(1, L * (b - a)) for a, b in zip(block0[:-1].tolist(), block0[1:].tolist())]
+            return acts, wavs
 
     # ---- one long clip over several GPUs (BASELINE.json configs[4]) ---------------------------------------------------
     # Blocks are independent except for the 50 % cross-fade with the two neighbouring chunks (modules.py:259-263): a rank that
