@@ -79,10 +79,11 @@ int tt_cqt_inverse(tt_cqt_plan* plan, const float* coeffs, int batch, int n_bloc
 int tt_scale_by_peak(float* audio, int64_t n, const float* peak, void* stream);
 
 /*
- * ---- many clips of different lengths in one call (TimbreTrap.transcribe_many / reconstruct_many) ---------------------------------
+ * ---- clips in one call: the chunked paths, and clips of different lengths (TimbreTrap.transcribe_many / reconstruct_many) --------
  * A clip table is a device int32 prefix array of n_clips + 1 entries: clip c owns entries [t[c], t[c+1]) (at least one), counted
  * from t[0], so a slice of a longer table describes the clips it covers.  clip_block0 counts blocks (n_c = ceil(samples / L)),
- * clip_chunk0 chunks (2 n_c + 1 per clip).  Per-clip tensors follow one another, each in the layout a one-clip call produces.
+ * clip_chunk0 chunks (2 n_c + 1 per clip; a batch of B equal clips of n chunks is [0, n, 2n, ..., Bn]).  Per-clip tensors follow
+ * one another, each in the layout a one-clip call produces.
  */
 /* tt_cqt_inverse over clips: coeffs = the clips' (F, n_c * M, 2) tensors, audio = their (n_c * L) samples, n_blocks = t[n] - t[0];
  * peaks (n_clips) fp32 device: max|audio| of each clip before normalisation (reset here); normalise as tt_cqt_inverse, per clip */
@@ -116,18 +117,15 @@ int tt_to_decibels(const float* magnitude, int batch, int64_t per_item, int resc
                    float* item_max, void* stream);
 
 /*
- * Hann cross-fade of 50 %-overlapped chunk outputs + trim (TimbreTrap.chunked_inference, modules.py:237-267).
- *   chunks      (batch * n_chunks, F, M, 2) fp32 - chunk i of item b at index b * n_chunks + i
+ * Hann cross-fade of 50 %-overlapped chunk outputs + trim (TimbreTrap.chunked_inference, modules.py:237-267) for the n_clips clips
+ * of the chunk prefix table t = clip_chunk0 (the clip table above).
+ *   chunks      (t[n_clips] - t[0], F, M, 2) fp32 - clip c's chunks at rows t[c] - t[0] ..
  *   window      (M) fp32 device (torch.signal.windows.hann, modules.py:239)
- *   coeffs_out  (batch, F, (n_chunks-1) * M/2, 2) or NULL
- *   act_out     (batch, F, (n_chunks-1) * M/2)    or NULL: tanh(|.|) of the cross-faded coefficients
+ *   coeffs_out  clip after clip, (F, (n_c - 1) * M/2, 2) each, or NULL
+ *   act_out     clip after clip, (F, (n_c - 1) * M/2) each, or NULL: tanh(|.|) of the cross-faded coefficients
  *               (TimbreTrap.to_activations, modules.py:271-289, fused for transcribe())
+ *   max_chunks  the most chunks of any clip
  */
-int tt_chunk_crossfade(const float* chunks, const float* window, int batch, int n_chunks, int n_bins, int frames_per_chunk,
-                       float* coeffs_out, float* act_out, void* stream);
-
-/* tt_chunk_crossfade over the clips of clip_chunk0: chunks (t[n] - t[0], F, M, 2); clip c's outputs (F, (n_c - 1) * M/2 [, 2]) follow
- * those of the clips before it; max_chunks = the most chunks of any clip */
 int tt_chunk_crossfade_clips(const float* chunks, const float* window, const int* clip_chunk0, int n_clips, int max_chunks, int n_bins,
                              int frames_per_chunk, float* coeffs_out, float* act_out, void* stream);
 
@@ -211,15 +209,9 @@ int tt_conv_out(const void* x, float* coeffs, const float* w, const float* bias,
 
 /* Decoder.convout FUSED with the Hann cross-fade + trim of TimbreTrap.chunked_inference (modules.py:237-267) and, for act_out,
  * with TimbreTrap.to_activations (modules.py:271-289): the last decoder stage of ALL chunks in, cross-faded results out - the
- * per-chunk coefficients never exist in memory.
- *   x           (batch * n_chunks, H, M, 4) bf16 packed 4-channel layout - chunk i of item b at index b * n_chunks + i
- *   window      (M) fp32 device (torch.signal.windows.hann, modules.py:239);  w fp32 [2][C][3][3], bias fp32 [2]
- *   coeffs_out  (batch, H, (n_chunks-1) * M/2, 2) fp32 or NULL;  act_out (batch, H, (n_chunks-1) * M/2) fp32 or NULL */
-int tt_conv_out_crossfade(const void* x, const float* window, const float* w, const float* bias, int batch, int n_chunks, int C,
-                          int H, int M, float* coeffs_out, float* act_out, void* stream);
-
-/* tt_conv_out_crossfade over the clips of clip_chunk0 (see tt_cqt_inverse_clips): x (total_chunks, H, M, 4) with total_chunks =
- * t[n] - t[0]; clip c's outputs (H, (n_c - 1) * M/2 [, 2]) follow those of the clips before it; max_chunks = the most of any clip */
+ * per-chunk coefficients never exist in memory.  Clips, outputs and max_chunks as for tt_chunk_crossfade_clips.
+ *   x           (total_chunks, H, M, 4) bf16 packed 4-channel layout, total_chunks = t[n_clips] - t[0]
+ *   window      (M) fp32 device (torch.signal.windows.hann, modules.py:239);  w fp32 [2][C][3][3], bias fp32 [2] */
 int tt_conv_out_crossfade_clips(const void* x, const float* window, const float* w, const float* bias, const int* clip_chunk0,
                                 int n_clips, int total_chunks, int max_chunks, int C, int H, int M, float* coeffs_out, float* act_out,
                                 void* stream);

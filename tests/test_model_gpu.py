@@ -140,8 +140,8 @@ def test_chunk_batching_is_invisible():
 
 @pytest.mark.parametrize('cfg,latent,complexity', [(SMALL, None, 1), (BASE, 128, 2)])
 def test_fused_convout_crossfade_is_bit_identical(cfg, latent, complexity):
-    """tt_conv_out_crossfade (convout + Hann cross-fade + trim + tanh|.| over all chunks in one kernel) against the un-fused
-    sequence convout per chunk -> tt_chunk_crossfade: same products, same order, identical bits."""
+    """tt_conv_out_crossfade_clips (convout + Hann cross-fade + trim + tanh|.| over all chunks in one kernel) against the un-fused
+    sequence convout per chunk -> tt_chunk_crossfade_clips: same products, same order, identical bits."""
     model, sd, c = _build(cfg, latent, complexity, False, seed=1)
     audio = tonal_clip(int(2.6 * c.block_length), cfg['sample_rate'], seed=6, n_batch=2).cuda()
     act, rec = model._chunked(audio, True, True)

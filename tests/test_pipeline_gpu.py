@@ -43,6 +43,23 @@ def test_early_activations_equal_whole(max_chunks):
     assert torch.equal(torch.cat([a for _, _, a in seen]), act)
 
 
+def test_transcribe_and_reconstruct_does_not_wait_for_the_device():
+    """No host synchronisation in the call, with or without the early hand-over: HostPipeline keeps two steps in flight only if
+    submitting one does not wait for the other."""
+    model = _model()
+    audio = _batches(model, 1, 3)[0].cuda()
+    model.MAX_CHUNKS_PER_BATCH = 4
+    hook = lambda lo, hi, a: None
+    model.transcribe_and_reconstruct(audio, on_activations=hook)       # warm-up: plans, packed weights, windows
+    torch.cuda.synchronize()
+    torch.cuda.set_sync_debug_mode('error')
+    try:
+        model.transcribe_and_reconstruct(audio)
+        model.transcribe_and_reconstruct(audio, on_activations=hook)
+    finally:
+        torch.cuda.set_sync_debug_mode('default')
+
+
 @pytest.mark.parametrize('early,depth,max_chunks', [(False, 2, 256), (True, 3, 256), (True, 3, 7), (True, 2, 11)])
 def test_pipeline_returns_the_device_results(early, depth, max_chunks):
     from timbre_trap_b200.framework import HostPipeline

@@ -31,7 +31,6 @@ SIGNATURES = {
     'tt_cqt_inverse': (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p]),
     'tt_scale_by_peak': (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     'tt_magnitude': (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
-    'tt_chunk_crossfade': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     'tt_res_block_rs': (c_int, [c_void_p] * 5 + [c_int] * 7 + [c_void_p]),
     'tt_res_block_rs_mid': (c_int, [c_void_p] * 6 + [c_int] * 7 + [c_void_p]),
     'tt_set_strip_rows': (c_int, [c_int]),
@@ -43,7 +42,6 @@ SIGNATURES = {
     'tt_deconv_in': (c_int, [c_void_p] * 4 + [c_int] * 6 + [c_void_p]),
     'tt_conv_in': (c_int, [c_void_p] * 4 + [c_int] * 5 + [c_void_p]),
     'tt_conv_out': (c_int, [c_void_p] * 4 + [c_int] * 5 + [c_void_p]),
-    'tt_conv_out_crossfade': (c_int, [c_void_p] * 4 + [c_int] * 5 + [c_void_p] * 3),
     'tt_cqt_inverse_clips': (c_int, [c_void_p] * 3 + [c_int] * 2 + [c_void_p] * 2 + [c_int, c_void_p]),
     'tt_scale_by_clip_peak': (c_int, [c_void_p] * 2 + [c_int] * 3 + [c_void_p] * 2),
     'tt_gather_chunks': (c_int, [c_void_p] * 2 + [c_int] * 4 + [c_void_p] * 2),

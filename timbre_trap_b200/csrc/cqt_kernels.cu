@@ -577,21 +577,17 @@ __global__ void decibels_kernel(const float* __restrict__ x, long long per_item,
 // frame t (after the M/2 trim) receives chunk i1 = (t + M/2) / (M/2) at position p1 = (t + M/2) mod (M/2) and chunk
 // i1 - 1 at position p1 + M/2, each scaled by the window.  Products are rounded separately and added in chunk order,
 // like the reference's `coefficients[...] += window * output_chunk`.
-// blockIdx.z is the item: batch items of n_chunks chunks each, or - clip_chunk0 non-null - clip z of the chunk prefix table
-// (find_clip), whose chunks and whose (F, (n - 1) M/2) output rows follow those of the clips before it.
-__global__ void crossfade_kernel(const float2* __restrict__ chunks, const float* __restrict__ window, int n_chunks, int F,
-                                 int M, float2* __restrict__ coeffs_out, float* __restrict__ act_out, const int* __restrict__ clip_chunk0) {
+// blockIdx.z is clip z of the chunk prefix table clip_chunk0 (find_clip), whose chunks and whose (F, (n - 1) M/2) output rows
+// follow those of the clips before it.
+__global__ void crossfade_kernel(const float2* __restrict__ chunks, const float* __restrict__ window, int F, int M,
+                                 float2* __restrict__ coeffs_out, float* __restrict__ act_out, const int* __restrict__ clip_chunk0) {
     const int half = M / 2;
     const int b = blockIdx.z, f = blockIdx.y;
-    size_t chunk0 = (size_t)b * n_chunks, out0 = (size_t)b * F * ((size_t)(n_chunks - 1) * half);
-    if (clip_chunk0) {
-        const int c0 = __ldg(clip_chunk0 + b) - __ldg(clip_chunk0);
-        n_chunks = __ldg(clip_chunk0 + b + 1) - __ldg(clip_chunk0 + b);
-        chunk0 = (size_t)c0;
-        out0 = (size_t)F * half * (size_t)(c0 - b);       // sum over earlier clips of F (n_c - 1) M/2
-    }
+    const size_t chunk0 = (size_t)(__ldg(clip_chunk0 + b) - __ldg(clip_chunk0));
+    const int n_chunks = __ldg(clip_chunk0 + b + 1) - __ldg(clip_chunk0 + b);
+    const size_t out0 = (size_t)F * half * (chunk0 - b);      // sum over earlier clips of F (n_c - 1) M/2
     const long long n_out = (long long)(n_chunks - 1) * half;
-    const float2* base = chunks + (chunk0 * F + f) * M;       // chunk i of the item: + i * F * M
+    const float2* base = chunks + (chunk0 * F + f) * M;       // chunk i of the clip: + i * F * M
     const size_t chunk_stride = (size_t)F * M;
     const size_t out_row = out0 + (size_t)f * n_out;
     for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < n_out; t += (long long)gridDim.x * blockDim.x) {
@@ -969,20 +965,6 @@ extern "C" int tt_to_decibels(const float* magnitude, int batch, int64_t per_ite
     return TT_OK;
 }
 
-extern "C" int tt_chunk_crossfade(const float* chunks, const float* window, int batch, int n_chunks, int n_bins, int frames_per_chunk,
-                                  float* coeffs_out, float* act_out, void* stream_) {
-    TT_REQUIRE(chunks && window && (coeffs_out || act_out), "null argument");
-    TT_REQUIRE(n_chunks >= 2 && frames_per_chunk % 2 == 0, "need at least two chunks and an even chunk length");
-    if (batch <= 0 || n_bins <= 0) return TT_OK;
-    const long long n_out = (long long)(n_chunks - 1) * (frames_per_chunk / 2);
-    dim3 grid((unsigned)std::min<long long>((n_out + 255) / 256, 64), n_bins, batch);
-    crossfade_kernel<<<grid, 256, 0, (cudaStream_t)stream_>>>((const float2*)chunks, window, n_chunks, n_bins, frames_per_chunk,
-                                                              (float2*)coeffs_out, act_out, nullptr);
-    tt_count_launches(1);
-    TT_CUDA_CHECK(cudaGetLastError());
-    return TT_OK;
-}
-
 extern "C" int tt_chunk_crossfade_clips(const float* chunks, const float* window, const int* clip_chunk0, int n_clips,
                                         int max_chunks, int n_bins, int frames_per_chunk, float* coeffs_out, float* act_out,
                                         void* stream_) {
@@ -992,7 +974,7 @@ extern "C" int tt_chunk_crossfade_clips(const float* chunks, const float* window
     if (n_clips <= 0 || n_bins <= 0) return TT_OK;
     const long long n_out = (long long)(max_chunks - 1) * (frames_per_chunk / 2);
     dim3 grid((unsigned)std::min<long long>((n_out + 255) / 256, 64), n_bins, n_clips);
-    crossfade_kernel<<<grid, 256, 0, (cudaStream_t)stream_>>>((const float2*)chunks, window, 0, n_bins, frames_per_chunk,
+    crossfade_kernel<<<grid, 256, 0, (cudaStream_t)stream_>>>((const float2*)chunks, window, n_bins, frames_per_chunk,
                                                               (float2*)coeffs_out, act_out, clip_chunk0);
     tt_count_launches(1);
     TT_CUDA_CHECK(cudaGetLastError());

@@ -478,7 +478,7 @@ class TimbreTrap(nn.Module):
 
     # chunks per kernel batch of the chunked paths (bounds activation memory: ~2.3 GB per live tensor at 256 chunks)
     MAX_CHUNKS_PER_BATCH = 256
-    # convout + Hann cross-fade + trim (+ tanh|.|) as one kernel over all chunks; False = per-chunk convout, then tt_chunk_crossfade
+    # convout + Hann cross-fade + trim (+ tanh|.|) as one kernel over all chunks; False = per-chunk convout, then tt_chunk_crossfade_clips
     # (same arithmetic in the same order: results are bit-identical, tests/test_model_gpu.py)
     FUSE_CONVOUT_CROSSFADE = True
 
@@ -619,102 +619,115 @@ class TimbreTrap(nn.Module):
         return chunks.reshape(audio.size(0) * n_chunks, 1, L), n_chunks
 
     def _fused_convout(self):
-        """Whether the chunked paths run convout + cross-fade as one kernel (tt_conv_out_crossfade) on the packed last stage."""
+        """Whether the chunked paths run convout + cross-fade as one kernel (tt_conv_out_crossfade_clips) on the packed last stage."""
         return self.FUSE_CONVOUT_CROSSFADE and self.decoder.packed4 and self.sliCQ.max_window_length % 8 == 0 and self.HEAD_MODE is None
+
+    def _pipeline(self, chunk_rows, chunk0, t_chunk0, want_transcription, want_reconstruction, activations=True, trn=None,
+                  on_activations=None):
+        """
+        Batched form of chunked_inference (modules.py:204-269) over the clips of a clip table, for one or both switch settings with a
+        shared encoder pass.  chunk0: the host prefix array of chunks per clip (clip i owns the chunk rows [chunk0[i], chunk0[i + 1])
+        counted from chunk0[0]), t_chunk0: its int32 device copy; chunk_rows(c0, m): the audio of chunk rows [c0, c0 + m) as
+        (m, 1, L).  Returns flat (transcription, reconstruction) buffers holding, clip after clip, each clip's (F, T, 2) interleaved
+        coefficients - for the transcription, when `activations` and the model has no output head, its (F, T) activations instead (a
+        variant's own to_activations is the caller's) - None where not requested.  `trn`: a flat buffer to write the transcription to.
+
+        The last decoder stage of every chunk goes into one (chunks, F, M, 4) bf16 buffer per output; `convout`, the Hann cross-fade,
+        the trim and (for activations) tanh|.| then run as ONE kernel over it (tt_conv_out_crossfade_clips): the per-chunk fp32
+        coefficients of the reference's loop never exist.
+
+        `on_activations(lo, hi, activations of the clips [lo, hi))` (fused path only): called as soon as the clips [lo, hi) have all
+        their chunks through the decoder - their activations are produced right then, while the remaining chunk batches still compute,
+        so a caller that streams results off the device (framework.HostPipeline) can start copying early.
+        """
+        device = t_chunk0.device
+        F, M = self.sliCQ.n_bins, self.sliCQ.max_window_length
+        rel = chunk0 - chunk0[0]
+        total = int(rel[-1])
+        out0 = F * (M // 2) * (rel - np.arange(len(rel)))            # first output value of each clip
+        fused = self._fused_convout()
+        wants = (want_transcription, want_reconstruction)
+        if fused:
+            stages = [torch.empty((total, F, M, 4), dtype=torch.bfloat16, device=device) if w else None for w in wants]
+        else:
+            stages = [torch.empty((total, F, M, 2), dtype=torch.float32, device=device) if w else None for w in wants]
+        step = self.MAX_CHUNKS_PER_BATCH
+        early = on_activations is not None and fused and want_transcription and activations
+        if early and trn is None:
+            trn = torch.empty((int(out0[-1]),), dtype=torch.float32, device=device)
+        emitted = 0
+        for c0 in range(0, total, step):
+            m = min(step, total - c0)
+            lat, skips = self._codes(chunk_rows(c0, m))
+            for stage, reconstruct in zip(stages, (False, True)):
+                if stage is None:
+                    continue
+                if fused:
+                    self.decoder.last_stage_c8(lat, reconstruct, skips, out=stage[c0:c0 + m])
+                else:
+                    y = self.decoder.forward_c8(lat, reconstruct, skips)
+                    if self.HEAD_MODE is not None:
+                        # the reference's loop adds the variant's ONE output channel into its hard-coded two-channel buffer
+                        # (modules.py:244, 259-263): broadcast, i.e. both channels carry the head's output
+                        y = ops.channel0(y, self.HEAD_MODE).unsqueeze(-1).expand(-1, -1, -1, 2)
+                    stage[c0:c0 + m] = y
+            if early:
+                done = int(np.searchsorted(rel[1:], c0 + step, side='right'))     # clips whose chunks have all been decoded
+                if done > emitted:
+                    self._crossfade(stages[0], rel, t_chunk0, emitted, done, trn, True)
+                    on_activations(emitted, done, trn[out0[emitted]:out0[done]])
+                    emitted = done
+        outs = [trn, None]
+        for k, stage in enumerate(stages):
+            if stage is None or (k == 0 and early):
+                continue
+            as_act = k == 0 and activations and self.HEAD_MODE is None     # the fused tanh|.| is the BASE model's to_activations
+            if outs[k] is None:
+                outs[k] = torch.empty((int(out0[-1]) * (1 if as_act else 2),), dtype=torch.float32, device=device)
+            self._crossfade(stage, rel, t_chunk0, 0, len(rel) - 1, outs[k], as_act)
+        return outs
+
+    def _crossfade(self, stage, rel, t_chunk0, lo, hi, out, as_act):
+        """The cross-fade + trim (+ tanh|.| when `as_act`) of the clips [lo, hi) of _pipeline's clip table (rel: the host prefix array
+        counted from its first entry) from a stage buffer into their place in the flat output `out`."""
+        F, M = self.sliCQ.n_bins, self.sliCQ.max_window_length
+        o = F * (M // 2) * int(rel[lo] - lo) * (1 if as_act else 2)
+        dst = (None, _ptr(out[o:])) if as_act else (_ptr(out[o:]), None)
+        x, window, table = _ptr(stage[int(rel[lo]):]), _ptr(self._window(stage.device)), _ptr(t_chunk0[lo:])
+        max_chunks = int(np.diff(rel[lo:hi + 1]).max())
+        stream = ctypes.c_void_p(torch.cuda.current_stream(stage.device).cuda_stream)
+        with torch.cuda.device(stage.device):
+            if self._fused_convout():
+                _, _, w_out, b_out = self.decoder._packed()
+                _lib.check(_lib.lib().tt_conv_out_crossfade_clips(x, window, _ptr(w_out), _ptr(b_out), table, hi - lo, int(rel[hi] - rel[lo]),
+                                                                  max_chunks, self.decoder.channels[4], F, M, *dst, stream))
+            else:
+                _lib.check(_lib.lib().tt_chunk_crossfade_clips(x, window, table, hi - lo, max_chunks, F, M, *dst, stream))
 
     def _chunked(self, audio, want_transcription, want_reconstruction, activations=True, prepadded=False, on_activations=None):
         """
-        Batched form of chunked_inference (modules.py:204-269) for one or both switch settings with a shared
-        encoder pass.  Returns (transcription, reconstruction) coefficient tensors (B, F, T, 2) interleaved - or the
-        activations (B, F, T) for the transcription when `activations` - None where not requested.
-
-        The last decoder stage of every chunk goes into one (B * n_chunks, F, M, 4) bf16 buffer per output; `convout`, the Hann
-        cross-fade, the trim and (for activations) tanh|.| then run as ONE kernel over it (tt_conv_out_crossfade): the
-        per-chunk fp32 coefficients of the reference's loop never exist.
-
-        `on_activations(lo, hi, activations[lo:hi])` (fused path only): called as soon as the clips [lo, hi) have all their chunks
-        through the decoder - their activations are produced right then, while the remaining chunk batches still compute, so a
-        caller that streams results off the device (framework.HostPipeline) can start copying early.
+        _pipeline over a batch (B, 1, N) of equal clips cut by _chunks.  Returns (transcription, reconstruction) coefficient tensors
+        (B, F, T, 2) interleaved - or the activations (B, F, T) for the transcription when `activations` - None where not requested.
+        `on_activations(lo, hi, activations[lo:hi])`: see _pipeline.
         """
         _lib.require_cuda(audio, 'audio')
         with torch.no_grad():
-            B, F, M = audio.size(0), self.sliCQ.n_bins, self.sliCQ.max_window_length
+            B, F = audio.size(0), self.sliCQ.n_bins
             chunks, n_chunks = self._chunks(audio.detach().float(), prepadded)
-            n_out = (n_chunks - 1) * (M // 2)
-            window = self._window(audio.device)
-            fused = self._fused_convout()
-            wants = (want_transcription, want_reconstruction)
-            if fused:
-                stages = [torch.empty((B * n_chunks, F, M, 4), dtype=torch.bfloat16, device=audio.device) if w else None for w in wants]
-            else:
-                stages = [torch.empty((B * n_chunks, F, M, 2), dtype=torch.float32, device=audio.device) if w else None for w in wants]
-            step = self.MAX_CHUNKS_PER_BATCH
-            early = on_activations is not None and fused and want_transcription and activations
-            if early:
-                act_early = torch.empty((B, F, n_out), dtype=torch.float32, device=audio.device)
-                emitted = 0
-            for c0 in range(0, B * n_chunks, step):
-                lat, skips = self._codes(chunks[c0:c0 + step])
-                for stage, reconstruct in zip(stages, (False, True)):
-                    if stage is None:
-                        continue
-                    if fused:
-                        self.decoder.last_stage_c8(lat, reconstruct, skips, out=stage[c0:c0 + step])
-                    else:
-                        y = self.decoder.forward_c8(lat, reconstruct, skips)
-                        if self.HEAD_MODE is not None:
-                            # the reference's loop adds the variant's ONE output channel into its hard-coded two-channel buffer
-                            # (modules.py:244, 259-263): broadcast, i.e. both channels carry the head's output
-                            y = ops.channel0(y, self.HEAD_MODE).unsqueeze(-1).expand(-1, -1, -1, 2)
-                        stage[c0:c0 + step] = y
-                if early:
-                    done = min(B, (c0 + step) // n_chunks)            # clips whose chunks have all been decoded
-                    if done > emitted:
-                        self._convout_crossfade(stages[0], emitted, done, n_chunks, window, None, act_early)
-                        on_activations(emitted, done, act_early[emitted:done])
-                        emitted = done
-            _, _, w_out, b_out = self.decoder._packed()
-            results = []
-            for stage, want_act in zip(stages, (activations, False)):
-                if stage is None:
-                    results.append(None)
-                    continue
-                if early and want_act:
-                    results.append(act_early)
-                    continue
-                as_act = want_act and self.HEAD_MODE is None         # the fused tanh|.| is the BASE model's to_activations
-                if as_act:
-                    res = torch.empty((B, F, n_out), dtype=torch.float32, device=audio.device)
-                    args = (None, ctypes.c_void_p(res.data_ptr()))
+            n_out = (n_chunks - 1) * (self.sliCQ.max_window_length // 2)
+            # the clip table [0, n, 2n, ..., Bn] made on the device: an upload from the host would wait for the stream
+            table = torch.arange(0, (B + 1) * n_chunks, n_chunks, dtype=torch.int32, device=audio.device)
+            hook = None if on_activations is None else lambda lo, hi, act: on_activations(lo, hi, act.view(hi - lo, F, n_out))
+            trn, rec = self._pipeline(lambda c0, m: chunks[c0:c0 + m], np.arange(0, (B + 1) * n_chunks, n_chunks), table,
+                                      want_transcription, want_reconstruction, activations, on_activations=hook)
+            if trn is not None:
+                if activations and self.HEAD_MODE is None:
+                    trn = trn.view(B, F, n_out)
                 else:
-                    res = torch.empty((B, F, n_out, 2), dtype=torch.float32, device=audio.device)
-                    args = (ctypes.c_void_p(res.data_ptr()), None)
-                stream = ctypes.c_void_p(torch.cuda.current_stream(audio.device).cuda_stream)
-                with torch.cuda.device(audio.device):
-                    if fused:
-                        _lib.check(_lib.lib().tt_conv_out_crossfade(ctypes.c_void_p(stage.data_ptr()), ctypes.c_void_p(window.data_ptr()),
-                                                                    ctypes.c_void_p(w_out.data_ptr()), ctypes.c_void_p(b_out.data_ptr()),
-                                                                    B, n_chunks, self.decoder.channels[4], F, M, args[0], args[1], stream))
-                    else:
-                        _lib.check(_lib.lib().tt_chunk_crossfade(ctypes.c_void_p(stage.data_ptr()), ctypes.c_void_p(window.data_ptr()),
-                                                                 B, n_chunks, F, M, args[0], args[1], stream))
-                if want_act and not as_act:
-                    res = self.to_activations(res.permute(0, 3, 1, 2))       # a variant's own activation function
-                results.append(res)
-            return results
-
-    def _convout_crossfade(self, stage, lo, hi, n_chunks, window, out_coeffs, out_act):
-        """tt_conv_out_crossfade over the clips [lo, hi) of a (B * n_chunks, F, M, 4) stage buffer."""
-        F, M = self.sliCQ.n_bins, self.sliCQ.max_window_length
-        _, _, w_out, b_out = self.decoder._packed()
-        sub = stage[lo * n_chunks: hi * n_chunks]
-        with torch.cuda.device(stage.device):
-            _lib.check(_lib.lib().tt_conv_out_crossfade(ctypes.c_void_p(sub.data_ptr()), ctypes.c_void_p(window.data_ptr()),
-                                                        ctypes.c_void_p(w_out.data_ptr()), ctypes.c_void_p(b_out.data_ptr()),
-                                                        hi - lo, n_chunks, self.decoder.channels[4], F, M,
-                                                        None if out_coeffs is None else ctypes.c_void_p(out_coeffs[lo:hi].data_ptr()),
-                                                        None if out_act is None else ctypes.c_void_p(out_act[lo:hi].data_ptr()),
-                                                        ctypes.c_void_p(torch.cuda.current_stream(stage.device).cuda_stream)))
+                    trn = trn.view(B, F, n_out, 2)
+                    if activations:
+                        trn = self.to_activations(trn.permute(0, 3, 1, 2))       # a variant's own activation function
+            return trn, None if rec is None else rec.view(B, F, n_out, 2)
 
     def chunked_inference(self, audio, transcribe=False):
         """modules.py:204-269: (B, 1, N) -> (B, 2, F, T) cross-faded coefficients."""
@@ -813,7 +826,7 @@ class TimbreTrap(nn.Module):
         return flat, samples, blocks, chunks
 
     def _many(self, clips, want_transcription, want_reconstruction):
-        """(activations list or None, audio list or None) of the *_many calls."""
+        """(activations list or None, audio list or None) of the *_many calls: _pipeline and the inverse CQT once per group."""
         clips = list(clips)
         if not clips:
             return [] if want_transcription else None, [] if want_reconstruction else None
@@ -838,62 +851,26 @@ class TimbreTrap(nn.Module):
             clip_tab = torch.from_numpy(np.stack((np.array([x.data_ptr() for x in flat], dtype=np.int64), samples), 1)).to(device)
             t_chunk0, t_block0 = tab[:n + 1], tab[n + 1:]
             stream = ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
-            window = self._window(device)
-            fused = self._fused_convout()
             as_act = self.HEAD_MODE is None                  # the BASE model's tanh|.| is fused into the cross-fade
-            _, _, w_out, b_out = self.decoder._packed()
-            step = self.MAX_CHUNKS_PER_BATCH
             f32 = dict(dtype=torch.float32, device=device)
-            batch = torch.empty((min(step, rows), L), **f32)
-            wants = (want_transcription, want_reconstruction)
-            if fused:
-                stages = [torch.empty((rows, F, M, 4), dtype=torch.bfloat16, device=device) if w else None for w in wants]
-            else:
-                stages = [torch.empty((rows, F, M, 2), **f32) if w else None for w in wants]
+            batch = torch.empty((min(self.MAX_CHUNKS_PER_BATCH, rows), L), **f32)
             total_out = int(out0[-1])
             trn = torch.empty((F * total_out * (1 if as_act else 2),), **f32) if want_transcription else None
             audio = torch.empty((int(block0[-1]) * L,), **f32) if want_reconstruction else None
             peaks = torch.empty((n,), **f32) if want_reconstruction else None
-            for g in range(len(groups) - 1):
-                lo, hi = groups[g], groups[g + 1]
-                c_lo, c_hi = int(chunk0[lo]), int(chunk0[hi])
-                for c0 in range(c_lo, c_hi, step):
-                    m = min(step, c_hi - c0)
-                    _lib.check(_lib.lib().tt_gather_chunks(_ptr(clip_tab), _ptr(t_chunk0), n, c0, m, L, _ptr(batch), stream))
-                    lat, skips = self._codes(batch[:m].view(m, 1, L))
-                    for stage, reconstruct in zip(stages, (False, True)):
-                        if stage is None:
-                            continue
-                        part = stage[c0 - c_lo:c0 - c_lo + m]
-                        if fused:
-                            self.decoder.last_stage_c8(lat, reconstruct, skips, out=part)
-                        else:
-                            y = self.decoder.forward_c8(lat, reconstruct, skips)
-                            if self.HEAD_MODE is not None:          # both channels carry the head's output, as in _chunked
-                                y = ops.channel0(y, self.HEAD_MODE).unsqueeze(-1).expand(-1, -1, -1, 2)
-                            part.copy_(y)
-                tab_g = ctypes.c_void_p(t_chunk0.data_ptr() + 4 * lo)
-                max_chunks = int(chunks[lo:hi].max())
-                for stage, reconstruct in zip(stages, (False, True)):
-                    if stage is None:
-                        continue
-                    o = F * int(out0[lo])
-                    if not reconstruct:
-                        dst = (None, _ptr(trn[o:])) if as_act else (_ptr(trn[2 * o:]), None)
-                    else:
-                        coeffs = torch.empty((F * int(out0[hi] - out0[lo]), 2), **f32)
-                        dst = (_ptr(coeffs), None)
-                    if fused:
-                        _lib.check(_lib.lib().tt_conv_out_crossfade_clips(_ptr(stage), _ptr(window), _ptr(w_out), _ptr(b_out), tab_g, hi - lo,
-                                                                          c_hi - c_lo, max_chunks, self.decoder.channels[4], F, M, *dst, stream))
-                    else:
-                        _lib.check(_lib.lib().tt_chunk_crossfade_clips(_ptr(stage), _ptr(window), tab_g, hi - lo, max_chunks, F, M, *dst,
-                                                                       stream))
-                    if reconstruct:
-                        _lib.check(_lib.lib().tt_cqt_inverse_clips(self.sliCQ._plan(device).handle, _ptr(coeffs),
-                                                                   ctypes.c_void_p(t_block0.data_ptr() + 4 * lo), hi - lo,
-                                                                   int(block0[hi] - block0[lo]), _ptr(audio[int(block0[lo]) * L:]),
-                                                                   _ptr(peaks[lo:]), 1, stream))
+            for lo, hi in zip(groups[:-1], groups[1:]):
+                c_lo = int(chunk0[lo])
+
+                def gather(c0, m):
+                    _lib.check(_lib.lib().tt_gather_chunks(_ptr(clip_tab), _ptr(t_chunk0), n, c_lo + c0, m, L, _ptr(batch), stream))
+                    return batch[:m].view(m, 1, L)
+                o = F * int(out0[lo]) * (1 if as_act else 2)
+                _, coeffs = self._pipeline(gather, chunk0[lo:hi + 1], t_chunk0[lo:hi + 1], want_transcription, want_reconstruction,
+                                           trn=None if trn is None else trn[o:])
+                if want_reconstruction:
+                    _lib.check(_lib.lib().tt_cqt_inverse_clips(self.sliCQ._plan(device).handle, _ptr(coeffs), _ptr(t_block0[lo:]), hi - lo,
+                                                               int(block0[hi] - block0[lo]), _ptr(audio[int(block0[lo]) * L:]),
+                                                               _ptr(peaks[lo:]), 1, stream))
             acts = wavs = None
             if want_transcription:
                 if not as_act:
@@ -918,48 +895,39 @@ class TimbreTrap(nn.Module):
     def transcribe_sharded(self, audio, group=None, rank=None, world=None, gather=True):
         """transcribe() of a clip every rank holds, each rank computing a contiguous range of blocks.  Returns the whole
         (B, F, T) activations on every rank (gather=True, via all_gather over `group`) or the rank's own frames."""
-        group, rank, world = _resolve_group(group, rank, world)
-        sub, b0, b1 = self.shard_audio(audio, rank, world)
-        M, F = self.sliCQ.max_window_length, self.sliCQ.n_bins
-        if b1 > b0:
-            local = self._chunked(sub, True, False, prepadded=True)[0]
-        else:
-            local = torch.empty((audio.size(0), F, 0), dtype=torch.float32, device=audio.device)
-        return _gather_frames(local, -1, M, audio, self.sliCQ.block_length, group, world) if gather else local
+        return self._sharded(audio, True, False, group, rank, world, gather)[0]
 
     def reconstruct_sharded(self, audio, group=None, rank=None, world=None, gather=True):
         """reconstruct() of a clip every rank holds, sharded like transcribe_sharded; the reference's global peak normalise
         (cqtwrapper.py:209-211) is one scalar MAX all-reduce over `group`."""
-        group, rank, world = _resolve_group(group, rank, world)
-        sub, b0, b1 = self.shard_audio(audio, rank, world)
-        L = self.sliCQ.block_length
-        if b1 > b0:
-            rec = self._chunked(sub, False, True, prepadded=True)[1].permute(0, 3, 1, 2)
-            local = self._decode_shared_peak(rec, group)
-        else:
-            local = torch.empty((audio.size(0), 1, 0), dtype=torch.float32, device=audio.device)
-            if group is not None:                      # still take part in the peak exchange
-                import torch.distributed as dist
-                dist.all_reduce(torch.zeros(1, device=audio.device), op=dist.ReduceOp.MAX, group=group)
-        return _gather_frames(local, -1, L, audio, L, group, world) if gather else local
+        return self._sharded(audio, False, True, group, rank, world, gather)[1]
 
     def transcribe_and_reconstruct_sharded(self, audio, group=None, rank=None, world=None, gather=True):
         """Both results for a clip every rank holds from ONE encoder pass per rank (transcribe_sharded + reconstruct_sharded run two)."""
+        return self._sharded(audio, True, True, group, rank, world, gather)
+
+    def _sharded(self, audio, want_transcription, want_reconstruction, group, rank, world, gather):
+        """(activations or None, audio or None) of the *_sharded calls."""
         group, rank, world = _resolve_group(group, rank, world)
         sub, b0, b1 = self.shard_audio(audio, rank, world)
         M, F, L = self.sliCQ.max_window_length, self.sliCQ.n_bins, self.sliCQ.block_length
+        act = wav = None
         if b1 > b0:
-            act, rec = self._chunked(sub, True, True, prepadded=True)
-            wav = self._decode_shared_peak(rec.permute(0, 3, 1, 2), group)
+            act, rec = self._chunked(sub, want_transcription, want_reconstruction, prepadded=True)
+            if want_reconstruction:
+                wav = self._decode_shared_peak(rec.permute(0, 3, 1, 2), group)
         else:
-            act = torch.empty((audio.size(0), F, 0), dtype=torch.float32, device=audio.device)
-            wav = torch.empty((audio.size(0), 1, 0), dtype=torch.float32, device=audio.device)
-            if group is not None:
-                import torch.distributed as dist
-                dist.all_reduce(torch.zeros(1, device=audio.device), op=dist.ReduceOp.MAX, group=group)
-        if not gather:
-            return act, wav
-        return _gather_frames(act, -1, M, audio, L, group, world), _gather_frames(wav, -1, L, audio, L, group, world)
+            if want_transcription:
+                act = torch.empty((audio.size(0), F, 0), dtype=torch.float32, device=audio.device)
+            if want_reconstruction:
+                wav = torch.empty((audio.size(0), 1, 0), dtype=torch.float32, device=audio.device)
+                if group is not None:                  # still take part in the peak exchange
+                    import torch.distributed as dist
+                    dist.all_reduce(torch.zeros(1, device=audio.device), op=dist.ReduceOp.MAX, group=group)
+        if gather:
+            act = None if act is None else _gather_frames(act, -1, M, audio, L, group, world)
+            wav = None if wav is None else _gather_frames(wav, -1, L, audio, L, group, world)
+        return act, wav
 
     def forward(self, audio, consistency=False):
         """modules.py:338-393: audio (B, 1, N) -> (reconstruction, latents, transcription, transcription_rec, transcription_scr, {}), the
