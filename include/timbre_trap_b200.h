@@ -172,11 +172,9 @@ int tt_res_block_rs(const void* x, void* y, const void* w1, const void* w2, cons
 int tt_res_block_rs_mid(const void* x, void* y, void* mid, const void* w1, const void* w2, const float* bias, int B, int C, int c_real,
                         int H, int T, int dilation, int layout, void* stream);
 /* One 3x3 dilated 'same' conv (k = 3, weights packing.pack_res3x3) or 1x1 conv (k = 1, packing.pack_res1x1), optional ELU, on C8
- * planar tensors: building block of the backward pass (recompute + data gradients as convs with transformed weights) */
-int tt_conv_same(const void* x, void* y, const void* w, const float* bias, int B, int C, int H, int T, int k, int dilation,
-                 int act_elu, void* stream);
-/* The same conv with one of the element-wise passes of the residual blocks' backward fused into its epilogue, on a tensor `e` of the
-   output's shape and layout: post = 1: y = conv(x) * ELU'(e), e the ACTIVATED value (e > 0 ? 1 : e + 1); post = 2: y = conv(x) + e. */
+ * planar tensors: building block of the backward pass (data gradients as convs with transformed weights).  post = 0: the plain conv;
+ * otherwise one of the element-wise passes of the residual blocks' backward fused into its epilogue, on a tensor `e` of the output's
+ * shape and layout: post = 1: y = conv(x) * ELU'(e), e the ACTIVATED value (e > 0 ? 1 : e + 1); post = 2: y = conv(x) + e. */
 int tt_conv_same_post(const void* x, void* y, const void* w, const float* bias, int B, int C, int H, int T, int k, int dilation,
                       int act_elu, int post, const void* e, void* stream);
 /* EncoderBlock.sconv + ELU (modules.py:626-629): Conv2d(Cin, Cout, (4,1), stride (2,1)); Hout = (Hin-4)/2 + 1, and

@@ -526,11 +526,10 @@ def test_pairs_to_c8_rounding():
 
 
 @pytest.mark.parametrize('n', [8, 3_000_000])
-def test_dot_bf16(n):
-    """tt_dot_bf16 (the skip weights' gradient) against an fp64 sum: 8 values, and more than one grid-stride span (1184 CTAs x 256
-    threads x 8 values); the fixed-order reduction is bit-reproducible."""
+def test_dot_bf16_abi(n):
+    """tt_dot_bf16 (the skip weights' gradient), called through the C ABI, against an fp64 sum: 8 values, and more than one
+    grid-stride span (1184 CTAs x 256 threads x 8 values); the fixed-order reduction is bit-reproducible."""
     from timbre_trap_b200 import _lib
-    from timbre_trap_b200.framework import layer_grads as LG
     a = (1 + 0.5 * _randn((n,), 8)).to(torch.bfloat16)
     b = (1 + 0.5 * _randn((n,), 9)).to(torch.bfloat16)
     lib = _lib.lib()
@@ -538,7 +537,8 @@ def test_dot_bf16(n):
     out = [torch.empty((), dtype=torch.float32, device='cuda') for _ in range(2)]
     ac, bc = a.cuda(), b.cuda()
     for o in out:
-        _lib.check(lib.tt_dot_bf16(LG._p(ac), LG._p(bc), n, LG._p(o), LG._p(scratch), LG._s(ac)))
+        _lib.check(lib.tt_dot_bf16(ac.data_ptr(), bc.data_ptr(), n, o.data_ptr(), scratch.data_ptr(),
+                                   torch.cuda.current_stream().cuda_stream))
     want = float((a.double() * b.double()).sum())
     assert abs(float(out[0]) - want) <= 1e-6 * abs(want), (float(out[0]), want)
     assert torch.equal(out[0], out[1])

@@ -9,6 +9,8 @@ exception is raised.  Build it with `python -c "import __graft_entry__ as g; g.b
 import ctypes
 import os
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('TT_LIB_PATH') or os.path.join(_HERE, 'libtimbretrap_b200.so')   # override: A/B builds while tuning
 
@@ -36,7 +38,6 @@ SIGNATURES = {
     'tt_set_strip_rows': (c_int, [c_int]),
     'tt_conv_down_strip': (c_int, [c_void_p] * 3 + [c_int] * 7 + [c_void_p]),
     'tt_conv_up_strip': (c_int, [c_void_p] * 3 + [c_int] * 8 + [c_void_p]),
-    'tt_conv_same': (c_int, [c_void_p] * 4 + [c_int] * 7 + [c_void_p]),
     'tt_conv_same_post': (c_int, [c_void_p] * 4 + [c_int] * 8 + [c_void_p] * 2),
     'tt_conv_lat': (c_int, [c_void_p] * 4 + [c_int] * 5 + [c_void_p]),
     'tt_deconv_in': (c_int, [c_void_p] * 4 + [c_int] * 6 + [c_void_p]),
@@ -113,3 +114,23 @@ def require_cuda(tensor, what):
     if not tensor.is_cuda:
         raise TimbreTrapB200Error(f'{what} must be a CUDA tensor: timbre_trap_b200 has no CPU path '
                                   '(the CPU oracle lives in oracle/ and is test-only).')
+
+
+def launch(name, *args):
+    """Call the entry point `name` with `args` and the current stream of their device, that device current, and check the status.
+    Tensors go in as their data pointers, None as NULL, anything else as it is.  Every tensor must be a CUDA tensor and all of them
+    on one device: the kernels would otherwise read memory of another device than the stream they run on."""
+    device, ptrs = None, []
+    for i, a in enumerate(args):
+        if isinstance(a, torch.Tensor):
+            d = a.get_device()                      # the CUDA device index; -1 for a CPU tensor
+            if d < 0:
+                require_cuda(a, f'argument {i} of {name}')
+            if device is None:
+                device = d
+            elif d != device:
+                raise ValueError(f'argument {i} of {name} is on cuda:{d}, an earlier one on cuda:{device}: all must be on one device')
+            a = a.data_ptr()
+        ptrs.append(a)
+    with torch.cuda.device(device):
+        check(getattr(lib(), name)(*ptrs, torch.cuda.current_stream(device).cuda_stream))

@@ -266,14 +266,9 @@ static int dispatch_n1(const ConvRowsParams& p, int n1, cudaStream_t s) {
     }
 }
 
-// A single 3x3 dilated 'same' conv (optionally + ELU) or 1x1 conv on C8 planar tensors through the generic tile kernel: used by
-// the backward pass (recompute of the residual block's inner activation; data gradients = convs with transformed weights).
+// A single 3x3 dilated 'same' conv (optionally + ELU) or 1x1 conv on C8 planar tensors through the generic tile kernel, with an
+// optional fused element-wise epilogue: used by the backward pass (data gradients = convs with transformed weights).
 //   k = 3: weights from packing.pack_res3x3 (K order tap-major);  k = 1: packing.pack_res1x1.  bias may be NULL (zeros).
-extern "C" int tt_conv_same(const void* x, void* y, const void* w, const float* bias, int B, int C, int H, int T, int k, int dilation,
-                            int act_elu, void* stream) {
-    return tt_conv_same_post(x, y, w, bias, B, C, H, T, k, dilation, act_elu, 0, nullptr, stream);
-}
-
 extern "C" int tt_conv_same_post(const void* x, void* y, const void* w, const float* bias, int B, int C, int H, int T, int k, int dilation,
                                  int act_elu, int post, const void* e, void* stream) {
     TT_REQUIRE(x && y && w, "null argument");

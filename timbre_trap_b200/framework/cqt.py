@@ -20,14 +20,6 @@ from ..nsgt_tables import FilterBank
 __all__ = ['CQT']
 
 
-def _ptr(t):
-    return ctypes.c_void_p(t.data_ptr())
-
-
-def _stream(device):
-    return ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
-
-
 def _i32(a):
     return a.ctypes.data_as(ctypes.POINTER(ctypes.c_int32))
 
@@ -144,9 +136,7 @@ class CQT(torch.nn.Module):
         B, n = audio.size(0), audio.size(-1) // self.block_length
         out = torch.empty((B, self.n_bins, n * self.max_window_length, 2), dtype=torch.float32, device=audio.device)
         if B * n:
-            with torch.cuda.device(audio.device):
-                _lib.check(_lib.lib().tt_cqt_forward(self._plan(audio.device).handle, _ptr(audio), B, n, _ptr(out),
-                                                     _stream(audio.device)))
+            _lib.launch('tt_cqt_forward', self._plan(audio.device).handle, audio, B, n, out)
         return out
 
     def encode(self, audio):
@@ -176,9 +166,7 @@ class CQT(torch.nn.Module):
             audio = torch.empty((B, 1, n * self.block_length), dtype=torch.float32, device=c.device)
             peak = torch.zeros((), dtype=torch.float32, device=c.device)
             if B * n:
-                with torch.cuda.device(c.device):
-                    _lib.check(_lib.lib().tt_cqt_inverse(self._plan(c.device).handle, _ptr(c), B, n, _ptr(audio),
-                                                         _ptr(peak), int(normalise), _stream(c.device)))
+                _lib.launch('tt_cqt_inverse', self._plan(c.device).handle, c, B, n, audio, peak, int(normalise))
         return audio, peak
 
     def decode(self, coefficients):
@@ -204,8 +192,7 @@ class CQT(torch.nn.Module):
         c = c if c.is_contiguous() else c.contiguous()
         out = torch.empty(c.shape[:-1], dtype=torch.float32, device=c.device)
         if out.numel():
-            with torch.cuda.device(c.device):
-                _lib.check(_lib.lib().tt_magnitude(_ptr(c), out.numel(), int(apply_tanh), _ptr(out), _stream(c.device)))
+            _lib.launch('tt_magnitude', c, out.numel(), int(apply_tanh), out)
         return out
 
     @staticmethod
@@ -222,9 +209,7 @@ class CQT(torch.nn.Module):
         B = m.size(0)
         if m.numel():
             scratch = torch.empty(B, dtype=torch.float32, device=m.device)
-            with torch.cuda.device(m.device):
-                _lib.check(_lib.lib().tt_to_decibels(_ptr(m), B, m.numel() // B, int(rescale), _ptr(out), _ptr(scratch),
-                                                     _stream(m.device)))
+            _lib.launch('tt_to_decibels', m, B, m.numel() // B, int(rescale), out, scratch)
         return out
 
     # ---- host-side frame-grid helpers -----------------------------------------------------

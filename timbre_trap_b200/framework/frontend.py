@@ -10,7 +10,6 @@ from decoded samples to model input - and from model output to the reported metr
 Kernels: csrc/frontend_kernels.cu through the C ABI.  No CPU fallback.
 """
 
-import ctypes
 import math
 
 import numpy as np
@@ -19,14 +18,6 @@ import torch
 from .. import _lib
 
 __all__ = ['prepare_audio', 'sinc_resample_kernel', 'multi_pitch_to_activations', 'signal_distortion_ratio']
-
-
-def _p(t):
-    return ctypes.c_void_p(t.data_ptr())
-
-
-def _s(device):
-    return ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
 def sinc_resample_kernel(orig_freq, new_freq, lowpass_filter_width=6, rolloff=0.99):
@@ -78,11 +69,9 @@ def prepare_audio(audio, fs, sample_rate, normalise=True):
     n_out = int(math.ceil(new * N / orig))
     out = torch.empty((1, n_out), dtype=torch.float32, device=audio.device)
     peak = torch.empty((), dtype=torch.float32, device=audio.device)
-    with torch.cuda.device(audio.device):
-        lib = _lib.lib()
-        _lib.check(lib.tt_resample_mono(_p(audio), C, N, _p(table), orig, new, width, _p(out), n_out, _p(peak), _s(audio.device)))
-        if normalise and n_out:
-            _lib.check(lib.tt_scale_by_peak(_p(out), n_out, _p(peak), _s(audio.device)))
+    _lib.launch('tt_resample_mono', audio, C, N, table, orig, new, width, out, n_out, peak)
+    if normalise and n_out:
+        _lib.launch('tt_scale_by_peak', out, n_out, peak)
     return out
 
 
@@ -128,8 +117,7 @@ def multi_pitch_to_activations(multi_pitch, midi_freqs, n_bins_blur_decay=2.5, d
     blur = torch.from_numpy(taps).to(device)
     act = torch.empty((F, T), dtype=torch.float32, device=device)
     scratch = torch.empty(1, dtype=torch.float32, device=device)
-    with torch.cuda.device(device):
-        _lib.check(_lib.lib().tt_rasterise_pitches(_p(dense), T, P, _p(freqs), F, _p(blur), radius, _p(act), _p(scratch), _s(device)))
+    _lib.launch('tt_rasterise_pitches', dense, T, P, freqs, F, blur, radius, act, scratch)
     return act
 
 
@@ -157,8 +145,7 @@ def signal_distortion_ratio(preds, target, filter_length=512, zero_mean=False, l
     r0 = torch.empty((B, filter_length), dtype=torch.float64, device=p.device)
     b = torch.empty_like(r0)
     norms = torch.empty((B, 2), dtype=torch.float64, device=p.device)
-    with torch.cuda.device(p.device):
-        _lib.check(_lib.lib().tt_sdr_correlations(_p(t), _p(p), B, n, filter_length, _p(r0), _p(b), _p(norms), _s(p.device)))
+    _lib.launch('tt_sdr_correlations', t, p, B, n, filter_length, r0, b, norms)
     nt = norms[:, 0].sqrt().clamp(min=1e-6)
     npred = norms[:, 1].sqrt().clamp(min=1e-6)
     r0 = r0 / (nt * nt).unsqueeze(-1)

@@ -10,8 +10,6 @@ re-layouts are one-pass bf16 kernels.  A layer computes its weight and bias grad
 walks the graph and accumulates `.grad`; there is no cuDNN / ATen compute on the path.
 """
 
-import ctypes
-
 import torch
 from torch.utils.weak import WeakIdKeyDictionary
 
@@ -22,19 +20,11 @@ from .cqt import CQT
 from .packing import _PackedCache
 
 
-def _p(t):
-    return ctypes.c_void_p(t.data_ptr()) if t is not None else None
-
-
-def _s(t):
-    return ctypes.c_void_p(torch.cuda.current_stream(t.device).cuda_stream)
-
-
 # ---- residual blocks: the whole backward in the inference layouts (bf16), convolutions AND weight gradients on the tensor cores ----
 def _ew(fn_name, *tensors):
     """element-wise bf16 kernel over tensors of one common layout -> new tensor like the first"""
     out = torch.empty_like(tensors[0])
-    _lib.check(getattr(_lib.lib(), fn_name)(*[_p(t) for t in tensors], _p(out), out.numel(), _s(out)))
+    _lib.launch(fn_name, *tensors, out, out.numel())
     return out
 
 
@@ -44,7 +34,7 @@ def _as_c8(t):
         return t
     B, H, T, _ = t.shape
     out = torch.empty((B, 1, H, T, 8), dtype=torch.bfloat16, device=t.device)
-    _lib.check(_lib.lib().tt_p4_to_c8(_p(t), _p(out), B * H * T, _s(t)))
+    _lib.launch('tt_p4_to_c8', t, out, B * H * T)
     return out
 
 
@@ -53,7 +43,7 @@ def _to_layout_of(c8, ref):
     if ref.dim() == 5:
         return c8
     out = torch.empty_like(ref)
-    _lib.check(_lib.lib().tt_c8_to_p4(_p(c8), _p(out), out.numel() // 4, _s(out)))
+    _lib.launch('tt_c8_to_p4', c8, out, out.numel() // 4)
     return out
 
 
@@ -95,19 +85,17 @@ def _bw_pack_entries():
 def _wgrad_same(x8, dz8, cin, cout, k, d):
     """(dW (cout, cin, k, k), db (cout)) fp32 of a 'same' conv from C8 planar bf16 x and dz (tt_conv_wgrad_same, tensor cores)."""
     B, CGi, H, T, _ = x8.shape
-    lib = _lib.lib()
-    scratch = _scratch(_WGRAD_SCRATCH, x8.device, int(lib.tt_wgrad_scratch_floats(B, H, T)))
+    scratch = _scratch(_WGRAD_SCRATCH, x8.device, int(_lib.lib().tt_wgrad_scratch_floats(B, H, T)))
     dw = torch.zeros((cout, cin, k, k), dtype=torch.float32, device=x8.device)
     db = torch.zeros(cout, dtype=torch.float32, device=x8.device)
-    _lib.check(lib.tt_conv_wgrad_same(_p(x8), _p(dz8), _p(dw), _p(db), B, CGi * 8, dz8.size(1) * 8, cin, cout, H, T, k, d,
-                                      _p(scratch), _s(x8)))
+    _lib.launch('tt_conv_wgrad_same', x8, dz8, dw, db, B, CGi * 8, dz8.size(1) * 8, cin, cout, H, T, k, d, scratch)
     return dw, db
 
 
 class _ResFn(torch.autograd.Function):
     """ResidualConv2dBlock: fused forward kernel, which also writes the inner activation ELU(W1 * x + b1) it stages in shared memory
     (tt_res_block_rs_mid) - the backward needs it and a recompute costs a whole 3x3 conv launch per block; the backward stays in bf16
-    C8 planar end to end - both data-gradient convolutions through the tile kernel (tt_conv_same), both weight gradients through the
+    C8 planar end to end - both data-gradient convolutions through the tile kernel (tt_conv_same_post), both weight gradients through the
     MN-major tcgen05 kernels (tt_conv_wgrad_same), the ELU derivatives / residual add as one-pass element-wise kernels."""
 
     @staticmethod
@@ -141,8 +129,7 @@ class _ResFn(torch.autograd.Function):
                 gx = ops.conv_same(dz1, w1_t, None, 3, d, plus=gy)               # gx = gy + W1^T (*) dz1: the residual add in the epilogue
             else:
                 gx = _to_layout_of(ops.conv_same(dz1, w1_t, None, 3, d), x)      # packed 4-channel stage: re-layout, then add
-                one = torch.ones((), dtype=torch.float32, device=gx.device)
-                _lib.check(_lib.lib().tt_add_scaled_bf16(_p(gy), _p(gx), _p(one.reshape(1)), _p(gx), gx.numel(), _s(gx)))
+                gx = ops.add_scaled(gy, gx, torch.ones((), dtype=torch.float32, device=gx.device), out=gx)
         return gx, _needed(dw1, need[1]), _needed(db1, need[2]), _needed(dw2, need[3]), _needed(db2, need[4]), None, None, None
 
 
@@ -157,12 +144,11 @@ def _wgrad_updown(fine8, coarse8, cfine, ccoarse, transposed):
     input) -> dW (ccoarse, cfine, 4, 1) in the ConvTranspose2d layout, db (cfine)."""
     B, CGf, Hf, T, _ = fine8.shape
     Hc = coarse8.size(2)
-    lib = _lib.lib()
-    scratch = _scratch(_WGRAD_SCRATCH, fine8.device, int(lib.tt_wgrad_scratch_floats(B, Hc, T)))
+    scratch = _scratch(_WGRAD_SCRATCH, fine8.device, int(_lib.lib().tt_wgrad_scratch_floats(B, Hc, T)))
     dw = torch.zeros((ccoarse, cfine, 4, 1), dtype=torch.float32, device=fine8.device)
     db = torch.zeros(cfine if transposed else ccoarse, dtype=torch.float32, device=fine8.device)
-    _lib.check(lib.tt_conv_wgrad_updown(_p(fine8), _p(coarse8), _p(dw), _p(db), B, CGf * 8, coarse8.size(1) * 8, cfine, ccoarse, Hf, Hc, T,
-                                        int(transposed), _p(scratch), _s(fine8)))
+    _lib.launch('tt_conv_wgrad_updown', fine8, coarse8, dw, db, B, CGf * 8, coarse8.size(1) * 8, cfine, ccoarse, Hf, Hc, T, int(transposed),
+                scratch)
     return dw, db
 
 
@@ -230,13 +216,12 @@ def _wgrad_lat(tall8, flat8, ctall, cflat, dw, db, row_sums):
     """tt_conv_wgrad_lat: accumulates into dw (cflat.., ctall, H, 1) [first cflat rows], db (cflat) and row_sums (ctall, H) (either may be None).
     The kernel takes up to 128 flat-side channels; wider latents go through it in slices of 128 (a slice of the 1-row latents is a tiny copy)."""
     B, CGt, H, T, _ = tall8.shape
-    lib = _lib.lib()
-    scratch = _scratch(_LAT_SCRATCH, tall8.device, int(lib.tt_wgrad_lat_scratch_floats(B, H, T)))
+    scratch = _scratch(_LAT_SCRATCH, tall8.device, int(_lib.lib().tt_wgrad_lat_scratch_floats(B, H, T)))
     for c0 in range(0, cflat, 128):
         c1 = min(cflat, c0 + 128)
         flat = flat8[:, c0 // 8:c0 // 8 + 16].contiguous()
-        _lib.check(lib.tt_conv_wgrad_lat(_p(tall8), _p(flat), _p(dw[c0:c1]), _p(None if db is None else db[c0:c1]), _p(row_sums if c0 == 0 else None),
-                                         B, CGt * 8, flat.size(1) * 8, ctall, c1 - c0, H, T, _p(scratch), _s(tall8)))
+        _lib.launch('tt_conv_wgrad_lat', tall8, flat, dw[c0:c1], None if db is None else db[c0:c1], row_sums if c0 == 0 else None,
+                    B, CGt * 8, flat.size(1) * 8, ctall, c1 - c0, H, T, scratch)
 
 
 class _LatFn(torch.autograd.Function):
@@ -274,7 +259,7 @@ def _pairs_to_c8(pairs):
     pairs = pairs.contiguous()
     B, F_, T, _ = pairs.shape
     out = torch.empty((B, 1, F_, T, 8), dtype=torch.bfloat16, device=pairs.device)
-    _lib.check(_lib.lib().tt_pairs_to_c8(_p(pairs), B * F_ * T, _p(out), _s(pairs)))
+    _lib.launch('tt_pairs_to_c8', pairs, B * F_ * T, out)
     return out
 
 
@@ -345,9 +330,7 @@ class _OutFn(torch.autograd.Function):
         if need[0]:
             wt, zb = _bw_pack(weight, 'outT', lambda: (_two_channels(weight.detach().float(), 0).transpose(0, 1).flip(2, 3).contiguous(),  # (c, 2, 3, 3)
                                                        torch.zeros(c, device=gy.device)))
-            B, F_, T, _ = gy.shape
-            gx = torch.empty((B, F_, T, 4), dtype=torch.bfloat16, device=gy.device)
-            _lib.check(_lib.lib().tt_conv_in(_p(gy), _p(gx), _p(wt), _p(zb), B, c, F_, T, 2, _s(gy)))
+            gx = ops.conv_in(gy, wt, zb, c, packed4=True, act=False)
         return gx, _needed(dw, need[1]), _needed(db, need[2]), None, None
 
 
@@ -358,24 +341,20 @@ class _SkipAddFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, e, w):
         scale = w.detach().float().reshape(1)
-        out = torch.empty_like(x)
-        _lib.check(_lib.lib().tt_add_scaled_bf16(_p(x), _p(e), _p(scale), _p(out), x.numel(), _s(x)))
         ctx.save_for_backward(e, scale)
-        return out
+        return ops.add_scaled(x, e, scale)
 
     @staticmethod
     def backward(ctx, g):
         e, scale = ctx.saved_tensors
         g = g.contiguous()
-        lib = _lib.lib()
         ge = gw = None
         if ctx.needs_input_grad[1]:
-            ge = torch.empty_like(g)
-            _lib.check(lib.tt_add_scaled_bf16(_p(g), _p(g), _p(scale - 1.0), _p(ge), g.numel(), _s(g)))    # g + (w - 1) g = w g
+            ge = ops.add_scaled(g, g, scale - 1.0)                                   # g + (w - 1) g = w g
         if ctx.needs_input_grad[2]:
             gw = torch.empty((), dtype=torch.float32, device=g.device)
-            scratch = torch.empty(int(lib.tt_dot_scratch_floats()), dtype=torch.float32, device=g.device)
-            _lib.check(lib.tt_dot_bf16(_p(g), _p(e), g.numel(), _p(gw), _p(scratch), _s(g)))
+            scratch = torch.empty(int(_lib.lib().tt_dot_scratch_floats()), dtype=torch.float32, device=g.device)
+            _lib.launch('tt_dot_bf16', g, e, g.numel(), gw, scratch)
         return g, ge, gw
 
 
@@ -391,7 +370,7 @@ class _ActivationsFn(torch.autograd.Function):
     def backward(ctx, gact):
         (coeffs,) = ctx.saved_tensors
         g = torch.empty_like(coeffs)
-        _lib.check(_lib.lib().tt_activations_bwd(_p(coeffs), _p(gact.contiguous()), _p(g), gact.numel(), _s(coeffs)))
+        _lib.launch('tt_activations_bwd', coeffs, gact.contiguous(), g, gact.numel())
         return g
 
 
@@ -399,7 +378,7 @@ def _channel0_bwd(pairs, gpairs, mode):
     """(g * f'(v0), 0) for the pre-activation pairs v and the output-pair gradient g (tt_channel0_activation_bwd)."""
     gpairs = gpairs.contiguous()
     g = torch.empty_like(pairs)
-    _lib.check(_lib.lib().tt_channel0_activation_bwd(_p(pairs), _p(gpairs), pairs.numel() // 2, mode, _p(g), _s(pairs)))
+    _lib.launch('tt_channel0_activation_bwd', pairs, gpairs, pairs.numel() // 2, mode, g)
     return g
 
 
@@ -513,8 +492,7 @@ def _film_convin_grads(dz, lat, weight, gamma_w, gamma_b, beta_w, beta_b, hot, d
         db = torch.empty(c0, dtype=torch.float32, device=dev)
         dgw, dbw = torch.empty_like(gamma_w), torch.empty_like(beta_w)
         dgb, dbb = torch.empty_like(gamma_b), torch.empty_like(beta_b)
-        _lib.check(_lib.lib().tt_film_convin_grad(_p(G), _p(rows), _p(weight), _p(gamma_w), _p(gamma_b), _p(beta_w), _p(beta_b), d, c0, h0, hot,
-                                                  _p(dw), _p(db), _p(dgw), _p(dgb), _p(dbw), _p(dbb), _s(G)))
+        _lib.launch('tt_film_convin_grad', G, rows, weight, gamma_w, gamma_b, beta_w, beta_b, d, c0, h0, hot, dw, db, dgw, dgb, dbw, dbb)
     if latents:
         d_pad = lat.size(1) * 8
 

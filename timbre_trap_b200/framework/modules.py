@@ -10,8 +10,6 @@ names, shapes and default initialisation as the reference); their forward is nev
 Activations between layers live in the C8 planar bf16 layout (B, ceil(C/8), H, T, 8).
 """
 
-import ctypes
-
 import numpy as np
 import torch
 import torch.nn as nn
@@ -26,10 +24,6 @@ from .packing import _PackedCache       # also the name under which pickled modu
 
 __all__ = ['TimbreTrap', 'TimbreTrapFiLM', 'FiLM', 'TimbreTrapMag', 'TimbreTrapMagDB', 'Encoder', 'Decoder', 'EncoderBlock', 'DecoderBlock',
            'ResidualConv2dBlock', 'shard_block_range', 'shard_audio']
-
-
-def _ptr(t):
-    return ctypes.c_void_p(t.data_ptr())
 
 
 def _n16(c):
@@ -692,17 +686,15 @@ class TimbreTrap(nn.Module):
         counted from its first entry) from a stage buffer into their place in the flat output `out`."""
         F, M = self.sliCQ.n_bins, self.sliCQ.max_window_length
         o = F * (M // 2) * int(rel[lo] - lo) * (1 if as_act else 2)
-        dst = (None, _ptr(out[o:])) if as_act else (_ptr(out[o:]), None)
-        x, window, table = _ptr(stage[int(rel[lo]):]), _ptr(self._window(stage.device)), _ptr(t_chunk0[lo:])
+        dst = (None, out[o:]) if as_act else (out[o:], None)
+        x, window, table = stage[int(rel[lo]):], self._window(stage.device), t_chunk0[lo:]
         max_chunks = int(np.diff(rel[lo:hi + 1]).max())
-        stream = ctypes.c_void_p(torch.cuda.current_stream(stage.device).cuda_stream)
-        with torch.cuda.device(stage.device):
-            if self._fused_convout():
-                _, _, w_out, b_out = self.decoder._packed()
-                _lib.check(_lib.lib().tt_conv_out_crossfade_clips(x, window, _ptr(w_out), _ptr(b_out), table, hi - lo, int(rel[hi] - rel[lo]),
-                                                                  max_chunks, self.decoder.channels[4], F, M, *dst, stream))
-            else:
-                _lib.check(_lib.lib().tt_chunk_crossfade_clips(x, window, table, hi - lo, max_chunks, F, M, *dst, stream))
+        if self._fused_convout():
+            _, _, w_out, b_out = self.decoder._packed()
+            _lib.launch('tt_conv_out_crossfade_clips', x, window, w_out, b_out, table, hi - lo, int(rel[hi] - rel[lo]), max_chunks,
+                        self.decoder.channels[4], F, M, *dst)
+        else:
+            _lib.launch('tt_chunk_crossfade_clips', x, window, table, hi - lo, max_chunks, F, M, *dst)
 
     def _chunked(self, audio, want_transcription, want_reconstruction, activations=True, prepadded=False, on_activations=None):
         """
@@ -767,9 +759,7 @@ class TimbreTrap(nn.Module):
         import torch.distributed as dist
         audio, peak = self.sliCQ.decode_raw(coefficients, normalise=False)
         dist.all_reduce(peak, op=dist.ReduceOp.MAX, group=group)
-        with torch.cuda.device(audio.device):
-            _lib.check(_lib.lib().tt_scale_by_peak(ctypes.c_void_p(audio.data_ptr()), audio.numel(), ctypes.c_void_p(peak.data_ptr()),
-                                                   ctypes.c_void_p(torch.cuda.current_stream(audio.device).cuda_stream)))
+        _lib.launch('tt_scale_by_peak', audio, audio.numel(), peak)
         return audio
 
     def reconstruct(self, audio_in, group=None):
@@ -850,7 +840,6 @@ class TimbreTrap(nn.Module):
             tab = torch.from_numpy(np.concatenate((chunk0, block0)).astype(np.int32)).to(device)
             clip_tab = torch.from_numpy(np.stack((np.array([x.data_ptr() for x in flat], dtype=np.int64), samples), 1)).to(device)
             t_chunk0, t_block0 = tab[:n + 1], tab[n + 1:]
-            stream = ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
             as_act = self.HEAD_MODE is None                  # the BASE model's tanh|.| is fused into the cross-fade
             f32 = dict(dtype=torch.float32, device=device)
             batch = torch.empty((min(self.MAX_CHUNKS_PER_BATCH, rows), L), **f32)
@@ -862,15 +851,14 @@ class TimbreTrap(nn.Module):
                 c_lo = int(chunk0[lo])
 
                 def gather(c0, m):
-                    _lib.check(_lib.lib().tt_gather_chunks(_ptr(clip_tab), _ptr(t_chunk0), n, c_lo + c0, m, L, _ptr(batch), stream))
+                    _lib.launch('tt_gather_chunks', clip_tab, t_chunk0, n, c_lo + c0, m, L, batch)
                     return batch[:m].view(m, 1, L)
                 o = F * int(out0[lo]) * (1 if as_act else 2)
                 _, coeffs = self._pipeline(gather, chunk0[lo:hi + 1], t_chunk0[lo:hi + 1], want_transcription, want_reconstruction,
                                            trn=None if trn is None else trn[o:])
                 if want_reconstruction:
-                    _lib.check(_lib.lib().tt_cqt_inverse_clips(self.sliCQ._plan(device).handle, _ptr(coeffs), _ptr(t_block0[lo:]), hi - lo,
-                                                               int(block0[hi] - block0[lo]), _ptr(audio[int(block0[lo]) * L:]),
-                                                               _ptr(peaks[lo:]), 1, stream))
+                    _lib.launch('tt_cqt_inverse_clips', self.sliCQ._plan(device).handle, coeffs, t_block0[lo:], hi - lo, int(block0[hi] - block0[lo]),
+                                audio[int(block0[lo]) * L:], peaks[lo:], 1)
             acts = wavs = None
             if want_transcription:
                 if not as_act:

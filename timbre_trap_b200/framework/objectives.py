@@ -6,21 +6,11 @@ through the gradient kernels of csrc/train_kernels.cu (tt_sum_sq_diff_bwd, tt_tr
 (framework/train.py) uses the same Functions.
 """
 
-import ctypes
-
 import torch
 
 from .. import _lib
 
 __all__ = ['compute_reconstruction_loss', 'compute_transcription_loss', 'compute_consistency_loss']
-
-
-def _p(t):
-    return ctypes.c_void_p(t.data_ptr()) if t is not None else None
-
-
-def _s(t):
-    return ctypes.c_void_p(torch.cuda.current_stream(t.device).cuda_stream)
 
 
 def _same_order(a, b):
@@ -45,8 +35,7 @@ class _SqDiffFn(torch.autograd.Function):
     def forward(ctx, a, b, scale):
         x, y, channels_last = _same_order(a, b)
         out = torch.empty((), dtype=torch.float32, device=x.device)
-        with torch.cuda.device(x.device):
-            _lib.check(_lib.lib().tt_sum_sq_diff(_p(x), _p(y), x.numel(), scale, _p(out), _p(_scratch(x.device)), _s(x)))
+        _lib.launch('tt_sum_sq_diff', x, y, x.numel(), scale, out, _scratch(x.device))
         ctx.save_for_backward(x, y)
         ctx.meta = (scale, channels_last)
         return out
@@ -59,8 +48,7 @@ class _SqDiffFn(torch.autograd.Function):
         gb = torch.empty_like(y) if ctx.needs_input_grad[1] else None
         if ga is None and gb is None:
             return None, None, None
-        with torch.cuda.device(x.device):
-            _lib.check(_lib.lib().tt_sum_sq_diff_bwd(_p(x), _p(y), _p(gout.float().contiguous()), scale, _p(ga), _p(gb), x.numel(), _s(x)))
+        _lib.launch('tt_sum_sq_diff_bwd', x, y, gout.float().contiguous(), scale, ga, gb, x.numel())
         if channels_last:
             ga, gb = [None if g is None else g.permute(0, 3, 1, 2) for g in (ga, gb)]
         return ga, gb, None
@@ -82,9 +70,7 @@ class _TrnLossFn(torch.autograd.Function):
         g = target.detach().float().contiguous()
         B, F, T = e.shape
         out = torch.empty((), dtype=torch.float32, device=e.device)
-        with torch.cuda.device(e.device):
-            _lib.check(_lib.lib().tt_transcription_loss(_p(e), _p(g), B, F, T, int(bool(weight_positive_class)), _p(out),
-                                                        _p(_scratch(e.device)), _s(e)))
+        _lib.launch('tt_transcription_loss', e, g, B, F, T, int(bool(weight_positive_class)), out, _scratch(e.device))
         ctx.save_for_backward(e, g)
         ctx.weighted = int(bool(weight_positive_class))
         return out
@@ -97,9 +83,7 @@ class _TrnLossFn(torch.autograd.Function):
         if ge is None and gg is None:
             return None, None, None
         B, F, T = e.shape
-        with torch.cuda.device(e.device):
-            _lib.check(_lib.lib().tt_transcription_loss_bwd(_p(e), _p(g), _p(gout.float().contiguous()), B, F, T, ctx.weighted, _p(ge),
-                                                            _p(gg), _s(e)))
+        _lib.launch('tt_transcription_loss_bwd', e, g, gout.float().contiguous(), B, F, T, ctx.weighted, ge, gg)
         return ge, gg, None
 
 

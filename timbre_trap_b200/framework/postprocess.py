@@ -11,7 +11,6 @@ but on CUDA tensors (CPU tensors raise: there is no fallback):
                                                       estimates and references on a common frame grid
 """
 
-import ctypes
 import sys
 
 import torch
@@ -19,14 +18,6 @@ import torch
 from .. import _lib
 
 __all__ = ['filter_non_peaks', 'threshold', 'activations_to_binary', 'multipitch_counts', 'multipitch_scores']
-
-
-def _p(t):
-    return ctypes.c_void_p(t.data_ptr())
-
-
-def _s(t):
-    return ctypes.c_void_p(torch.cuda.current_stream(t.device).cuda_stream)
 
 
 def _as_bft(x, name):
@@ -43,8 +34,7 @@ def filter_non_peaks(activations):
     B, F, T = a.shape
     if a.numel() == 0:
         return out.reshape(activations.shape)
-    with torch.cuda.device(a.device):
-        _lib.check(_lib.lib().tt_filter_non_peaks(_p(a), _p(out), B, F, T, _s(a)))
+    _lib.launch('tt_filter_non_peaks', a, out, B, F, T)
     return out.reshape(activations.shape)
 
 
@@ -55,9 +45,7 @@ def activations_to_binary(activations, t=0.5, peaks_only=False, bin_lo=0, bin_hi
     out = torch.empty((B, F, T), dtype=torch.uint8, device=a.device)
     if a.numel() == 0:
         return out.reshape(activations.shape)
-    with torch.cuda.device(a.device):
-        _lib.check(_lib.lib().tt_peak_threshold(_p(a), _p(out), B, F, T, float(t), int(peaks_only), int(bin_lo), int(F if bin_hi is None else bin_hi),
-                                                _s(a)))
+    _lib.launch('tt_peak_threshold', a, out, B, F, T, float(t), int(peaks_only), int(bin_lo), int(F if bin_hi is None else bin_hi))
     return out.reshape(activations.shape)
 
 
@@ -76,8 +64,7 @@ def multipitch_counts(est, ref, tolerance_bins):
     counts = torch.zeros((B, 3), dtype=torch.int64, device=e.device)
     if e.numel() == 0:
         return counts
-    with torch.cuda.device(e.device):
-        _lib.check(_lib.lib().tt_multipitch_counts(_p(e), _p(r), B, F, T, int(tolerance_bins), _p(counts), _s(e)))
+    _lib.launch('tt_multipitch_counts', e, r, B, F, T, int(tolerance_bins), counts)
     return counts
 
 

@@ -20,11 +20,8 @@ layers (the reference runs the forward under fp16 autocast).
 import torch
 
 from .. import _lib
-from . import packing as P  # noqa: F401
-from .layer_grads import _ActivationsFn, _Channel0ActivationsFn, _p, _s
+from .layer_grads import _ActivationsFn, _Channel0ActivationsFn
 from .objectives import _sum_sq_diff, _TrnLossFn
-# the weight-gradient and edge-kernel wrappers, where code written against the earlier layout of this module reaches them
-from .layer_grads import _channel0_bwd, _film_convin_grads, _wgrad_lat, _wgrad_same, _wgrad_updown  # noqa: F401
 from .packing import _PackedCache
 
 __all__ = ['compute_step_losses', 'TrainStep', 'allreduce_mean_gradients']
@@ -156,11 +153,10 @@ class TrainStep:
         self.t += 1
         self._sync_grad_views()
         acc = torch.zeros((), dtype=torch.float64, device=self.flat_p.device)
-        lib = _lib.lib()
         n = self.flat_p.numel()
-        _lib.check(lib.tt_grad_sumsq(_p(self.flat_g), n, _p(acc), _s(self.flat_g)))
-        _lib.check(lib.tt_adamw_step(_p(self.flat_p), _p(self.flat_g), _p(self.flat_m), _p(self.flat_v), n, _p(acc), self.max_norm, self.lr,
-                                     self.betas[0], self.betas[1], self.eps, self.wd, self.t, _s(self.flat_p)))
+        _lib.launch('tt_grad_sumsq', self.flat_g, n, acc)
+        _lib.launch('tt_adamw_step', self.flat_p, self.flat_g, self.flat_m, self.flat_v, n, acc, self.max_norm, self.lr,
+                    self.betas[0], self.betas[1], self.eps, self.wd, self.t)
         _PackedCache.epoch += 1                                                  # weights changed behind torch's back: repack lazily
         return acc.sqrt()
 
